@@ -388,6 +388,40 @@ def run_configs(wfagpu):
     return out
 
 
+DUMP_CIGAR_PAIRS = 256
+
+
+def dump_outputs(path, lib, wfagpu, a, out, ops):
+    """What the last timed step returned to its caller, as .npy files for comparing two builds output for output:
+    distance.npy   every pair's score (float64),
+    n_ops.npy      every pair's number of backtrace operations (float64),
+    cigar_index.npy / cigar.npy   a fixed sample of DUMP_CIGAR_PAIRS pairs (seeded) and their CIGAR text as
+                   character codes (float32, one row per pair, zero-padded)."""
+    import ctypes as C
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    n = a.num_pairs
+    np.save(os.path.join(path, "distance.npy"), np.array([out[i].distance for i in range(n)], dtype=np.float64))
+    np.save(os.path.join(path, "n_ops.npy"), np.array([out[i].n_ops for i in range(n)], dtype=np.float64))
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_CIGAR_PAIRS, n), replace=False))
+    free = C.CDLL(None).free
+    free.argtypes = [C.c_void_p]
+    base = C.addressof(ops.contents)
+    texts = []
+    for i in idx:
+        p, t = (s.encode() for s in a.pair(int(i)))
+        cg = wfagpu.Cigar()
+        words = C.cast(base + 4 * out[i].ops_off, C.POINTER(C.c_uint32))
+        assert lib.wfagpu_ops_to_cigar(p, len(p), t, len(t), out[i].distance, words, out[i].n_ops, C.byref(cg))
+        texts.append(C.string_at(cg.buffer) if cg.buffer else b"")
+        free(cg.buffer)
+    codes = np.zeros((len(idx), max(map(len, texts), default=0)), dtype=np.float32)
+    for r, s in enumerate(texts):
+        codes[r, :len(s)] = np.frombuffer(s, dtype=np.uint8)
+    np.save(os.path.join(path, "cigar_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "cigar.npy"), codes)
+
+
 def envelope_block(wfagpu, a, local):
     """Operating envelope around the steady-state numbers: cold first call, un-hinted provisioning, stale hint."""
     out = {}
@@ -502,6 +536,8 @@ def run_ours(args):
     scores = [out[i].distance for i in range(rb.n)]
     n_ops_total = sum(out[i].n_ops for i in range(rb.n))
     assert all(out[i].status & 1 for i in range(rb.n)), "unfinished pairs in the benchmark batch"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lib, wfagpu, a, out, ops)
     rb.release()
 
     t_max, wall_max = reduce_max([dev_ms / 1e3, wall], device="cuda")
@@ -751,6 +787,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE configs 1-5 block (N = 1 only)")
     ap.add_argument("--quick", action="store_true", help="headline numbers only (no reference GPU, envelope, configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (rank 0's batch) to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -1,24 +1,15 @@
 """BASELINE configurations 1-3 at their STATED sizes through wfagpu_align (VERDICT r1: parity was tested at the right
-shapes but at 24-4000 pairs): every score equals the unmodified reference CPU WFA (oracle/_ref/libref_cpu.so, all host
-threads), every CIGAR is an alignment of exactly that cost (host validator), a sample equals the oracle's CIGAR text.
+shapes but at 24-4000 pairs): every score equals the stored exact score of the CPU WFA (tests/golden/cpu_wfa_scores.json),
+every CIGAR is an alignment of exactly that cost (host validator), a sample equals the oracle's CIGAR text.
 Config 4 at 8192 pairs is tests/test_gpu_parity.py::test_headline_batch_at_full_size, config 5 on 64 pairs
 tests/test_gpu_large_tier.py; bench.py's `configs` block runs all five at full size with parity samples."""
-import os
-
 import pytest
 
 import wfagpu
-from util import synth_aligner
+from util import assert_cpu_wfa_scores, synth_aligner
 
 pytestmark = pytest.mark.gpu
 PEN = (2, 3, 1)
-
-
-def cpu_scores(refcpu, a, lo, hi):
-    pairs = [a.pair(i) for i in range(lo, hi)]
-    errs, _ = refcpu.align_batch([p for p, _ in pairs], [t for _, t in pairs], *PEN, cigar=False,
-                                 threads=len(os.sched_getaffinity(0)))
-    return list(errs)
 
 
 def check_cigars(a, idx):
@@ -30,12 +21,12 @@ def check_cigars(a, idx):
     return bad
 
 
-def test_config1_10k_pairs_150bp_cigar(oracle, refcpu):
+def test_config1_10k_pairs_150bp_cigar(oracle):
     a = synth_aligner([(10000, 150, 0.02, 0.02)], 0xB2000001)
     assert a.initialize_parameters(*PEN)
     a.options.compute_cigar = True
     a.align()
-    assert a.errors() == cpu_scores(refcpu, a, 0, a.num_pairs)
+    assert_cpu_wfa_scores("config1", a.errors())
     assert check_cigars(a, range(a.num_pairs)) == 0
     for i in range(0, a.num_pairs, 250):
         p, t = a.pair(i)
@@ -43,19 +34,17 @@ def test_config1_10k_pairs_150bp_cigar(oracle, refcpu):
         assert (a.error(i), a.cigar(i)) == (r["distance"], r["cigar"])
 
 
-def test_config2_1M_pairs_150bp_score_only(refcpu):
+def test_config2_1M_pairs_150bp_score_only():
     a = synth_aligner([(1000000, 150, 0.05, 0.05)], 0xB2000002)
     assert a.initialize_parameters(*PEN)
     a.options.compute_cigar = False
     a.align()
     st = a.run_stats()
     assert st["failed_pairs"] == 0
-    got = a.errors()
-    for lo in range(0, a.num_pairs, 250000):                 # the CPU reference in four slices (memory of the pair lists)
-        assert got[lo:lo + 250000] == cpu_scores(refcpu, a, lo, min(lo + 250000, a.num_pairs))
+    assert_cpu_wfa_scores("config2", a.errors())
 
 
-def test_config3_100k_pairs_1kbp_cigar_with_redispatch(oracle, refcpu, monkeypatch):
+def test_config3_100k_pairs_1kbp_cigar_with_redispatch(oracle, monkeypatch):
     # -e 300: ~4 % of the pairs score above it.  First with the budget lift off (every chunk re-dispatches them on the GPU),
     # then with the default policy (a fresh process-wide hint: the first chunks re-dispatch, later chunks and the second call
     # run their first pass with the budget the last batch needed) -- same results either way
@@ -69,8 +58,8 @@ def test_config3_100k_pairs_1kbp_cigar_with_redispatch(oracle, refcpu, monkeypat
         a.align()
         st = a.run_stats()
         assert st["redispatched"] > 1000 and st["failed_pairs"] == 0
-        want = cpu_scores(refcpu, a, 0, a.num_pairs)
-        assert a.errors() == want
+        want = a.errors()
+        assert_cpu_wfa_scores("config3", want)
         assert check_cigars(a, range(0, a.num_pairs, 7)) == 0
         for i in range(0, a.num_pairs, 5003):
             p, t = a.pair(i)

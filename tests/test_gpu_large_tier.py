@@ -7,7 +7,7 @@ import sys
 
 import pytest
 
-from util import synth_aligner
+from util import cpu_wfa_scores, synth_aligner
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -34,7 +34,7 @@ def test_wide_wavefront_falls_into_large_tier(oracle):
         assert (a.error(i), a.cigar(i)) == (r["distance"], r["cigar"])
 
 
-def test_sequences_longer_than_32767(oracle, refcpu):
+def test_sequences_longer_than_32767(oracle):
     # config 5 shape (50 kbp Nanopore-like, 15 % error), initial budget deliberately too small so
     # that every pair is re-dispatched on the GPU; parity = CPU WFA score + valid CIGAR of that score
     a = synth_aligner([(4, 50000, 0.15, 0.15), (4, 40000, 0.03, 0.03)], 0xB2004000)
@@ -43,16 +43,17 @@ def test_sequences_longer_than_32767(oracle, refcpu):
     a.options.max_error = 2000
     a.align()
     pairs = [a.pair(i) for i in range(a.num_pairs)]
-    errs, _ = refcpu.align_batch([p for p, _ in pairs], [t for _, t in pairs], 2, 3, 1, cigar=False)
+    errs = cpu_wfa_scores("longer_than_32767")["scores"]
+    assert len(errs) == len(pairs)
     for i, (p, t) in enumerate(pairs):
         assert a.error(i) == errs[i]
         assert oracle.cigar_score(p, t, a.cigar(i), 2, 3, 1) == errs[i]
     assert a.run_stats()["redispatched"] >= a.num_pairs
 
 
-def test_config5_shape_on_64_pairs_matches_cpu_wfa(oracle, refcpu):
+def test_config5_shape_on_64_pairs_matches_cpu_wfa(oracle):
     # BASELINE config 5 (50 kbp, 15 %, CIGAR, first budget 8000 below every score: every pair is re-dispatched on the GPU
-    # with a bound-guided budget) on 64 pairs: every score == the unmodified reference CPU WFA, every CIGAR an alignment of
+    # with a bound-guided budget) on 64 pairs: every score == the stored exact score of the CPU WFA, every CIGAR an alignment of
     # exactly that cost; the re-dispatched pass runs wfa_quadg_kernel (int32 rings in L2)
     a = synth_aligner([(64, 50000, 0.15, 0.15)], 0xB2000005)
     assert a.initialize_parameters(2, 3, 1)
@@ -62,8 +63,7 @@ def test_config5_shape_on_64_pairs_matches_cpu_wfa(oracle, refcpu):
     st = a.run_stats()
     assert st["redispatched"] == 64 and st["failed_pairs"] == 0
     pairs = [a.pair(i) for i in range(a.num_pairs)]
-    errs, _ = refcpu.align_batch([p for p, _ in pairs], [t for _, t in pairs], 2, 3, 1, cigar=False,
-                                 threads=len(os.sched_getaffinity(0)))
-    assert a.errors() == list(errs)
+    errs = cpu_wfa_scores("config5_64")["scores"]
+    assert a.errors() == errs
     for i, (p, t) in enumerate(pairs):
         assert oracle.cigar_score(p, t, a.cigar(i), 2, 3, 1) == errs[i]

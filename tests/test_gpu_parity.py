@@ -5,7 +5,7 @@ import os
 import pytest
 
 import wfagpu
-from util import synth_aligner, check_against_oracle
+from util import assert_cpu_wfa_scores, check_against_oracle, cpu_wfa_scores, non_acgt_pairs, synth_aligner
 
 pytestmark = pytest.mark.gpu
 
@@ -185,10 +185,10 @@ def test_penalties_whose_rings_do_not_fit_the_bound_kernel(oracle, pen, length, 
         assert (a.error(i), a.cigar(i)) == (r["distance"], r["cigar"])
 
 
-def test_headline_batch_at_full_size(oracle, refcpu):
+def test_headline_batch_at_full_size(oracle):
     # BASELINE's headline configuration at bench.py's full size (8192 x 10 kbp, 5 %, -e 3000, CIGAR),
     # checked through properties that do not need the oracle on every pair:
-    #   * every score equals the unmodified reference CPU WFA (all pairs),
+    #   * every score equals the stored exact score of the CPU WFA (all pairs),
     #   * every CIGAR is an alignment of its two sequences whose gap-affine cost is that score,
     #   * a second call (provisioned from the first one's scores: per-pair bounds, tighter rings,
     #     another CTA per SM) returns byte-identical results,
@@ -196,8 +196,7 @@ def test_headline_batch_at_full_size(oracle, refcpu):
     a = run([(8192, 10000, 0.05, 0.05)], (2, 3, 1), True, max_error=3000, batch=4096, seed=0xB2000004)
     errs, cigs = a.errors(), a.cigars()
     pairs = [a.pair(i) for i in range(a.num_pairs)]
-    ref, _ = refcpu.align_batch([p for p, _ in pairs], [t for _, t in pairs], 2, 3, 1, cigar=False)
-    assert errs == ref
+    assert_cpu_wfa_scores("headline", errs)
     for (p, t), s, c in zip(pairs, errs, cigs):
         assert oracle.cigar_score(p, t, c, 2, 3, 1) == s
     a.reset_results()
@@ -209,16 +208,15 @@ def test_headline_batch_at_full_size(oracle, refcpu):
 
 
 @pytest.mark.parametrize("pen", [(4, 6, 2), (3, 1, 4), (2, 10, 5), (5, 3, 2)])
-def test_long_reads_with_gap_extension_above_one(oracle, refcpu, pen):
+def test_long_reads_with_gap_extension_above_one(oracle, pen):
     # e > 1 exercises the quotient of the score-bound pruning ((Dmax - d) / e), the reachability bound
     # and the snapshot geometry at sizes where bounds, hints and re-provisioning are all active:
-    # scores vs the unmodified reference CPU WFA, CIGARs must be alignments of exactly that cost,
+    # scores vs the stored exact scores of the CPU WFA, CIGARs must be alignments of exactly that cost,
     # and a sample must equal the oracle's CIGAR text.
     a = run([(1536, 5000, 0.02, 0.08)], pen, True, max_error=6000, batch=512, seed=0xB2000040 + pen[2])
     errs, cigs = a.errors(), a.cigars()
     pairs = [a.pair(i) for i in range(a.num_pairs)]
-    ref, _ = refcpu.align_batch([p for p, _ in pairs], [t for _, t in pairs], *pen, cigar=False)
-    assert errs == ref
+    assert_cpu_wfa_scores("long_reads_%d_%d_%d" % pen, errs)
     for (p, t), s, c in zip(pairs, errs, cigs):
         assert oracle.cigar_score(p, t, c, *pen) == s
     for i in range(0, a.num_pairs, 191):
@@ -245,33 +243,23 @@ def test_banded_pairs_over_budget_are_finished_by_the_exact_kernels(oracle):
     assert a.run_stats()["redispatched"] == n_exact
 
 
-def test_non_acgt_pairs_match_cpu_wfa_scores(oracle, refcpu):
+def test_non_acgt_pairs_match_cpu_wfa_scores(oracle):
     # Pairs the packer flags (an 'N' in either sequence, sequence_packing_kernel.cu:54-76) go through the
     # byte-compare kernels, as the reference sends them to its CPU WFA: same byte-equality semantics, so
     # the same optimal score; the CIGAR must be an alignment of that cost.  (Other non-ACGT bytes are not
     # flagged by the reference and are 2-bit encoded as (c & 6) >> 1 on its GPU path -- and here.)
     # Mixed with clean pairs in one batch, small budget so that some flagged pairs are also re-dispatched.
-    import random
-    rng = random.Random(77)
-    a = synth_aligner([(300, 800, 0.02, 0.10), (40, 3000, 0.05, 0.05)], 0xB2000077)
-    pairs = [a.pair(i) for i in range(a.num_pairs)]
+    pairs, dirty = non_acgt_pairs()
     b = wfagpu.Aligner()
-    dirty = []
-    for i, (p, t) in enumerate(pairs):
-        if i % 3 == 0:
-            p, t = list(p), list(t)
-            for s in (p, t):
-                for _ in range(rng.randint(1, 6)):
-                    s[rng.randrange(len(s))] = "N"
-            p, t = "".join(p), "".join(t)
-            dirty.append(i)
+    for p, t in pairs:
         assert b.add_sequences(p, t)
     assert b.initialize_parameters(2, 3, 1)
     b.options.compute_cigar = True
     b.options.max_error = 150
     b.align()
     bp = [b.pair(i) for i in range(b.num_pairs)]
-    ref, _ = refcpu.align_batch([p for p, _ in bp], [t for _, t in bp], 2, 3, 1, cigar=False)
+    assert bp == pairs
+    ref = cpu_wfa_scores("non_acgt")["scores"]
     assert b.errors() == ref
     for i, (p, t) in enumerate(bp):
         assert oracle.cigar_score(p, t, b.cigar(i), 2, 3, 1) == ref[i]

@@ -48,6 +48,21 @@ typedef struct {
 int wfagpu_build_step_table(int x, int o, int e, int max_steps, int max_dist, int banded_win,
                             wfagpu_step_t *tab, uint64_t *arena_units);
 
+/* Ends-free alignments (exact kernels only): every score's range is widened by `start_half_width` diagonals on both
+ * sides, the half width of the start row [-pattern_begin_free, text_begin_free].  -1 if it does not fit the table. */
+int wfagpu_build_step_table_span(int x, int o, int e, int max_steps, int max_dist, int start_half_width,
+                                 wfagpu_step_t *tab, uint64_t *arena_units);
+
+/* ---------------------------------------------------------- ends-free --- */
+/* Ends-free (semi-global) span of a call, WFA2-lib's `ends-free` order.  All zero = global alignment.  Per pair each
+ * value is clamped to the sequence it applies to.  The score is the gap-affine cost of the aligned part: leading and
+ * trailing pattern / text bases up to these counts are free.  The CIGAR still covers both full sequences: the free
+ * parts print as leading / trailing I (text) or D (pattern) runs, joined with a gap run of the same letter next to
+ * them. */
+typedef struct {
+    int pattern_begin_free, pattern_end_free, text_begin_free, text_end_free;
+} wfagpu_span_t;
+
 /* ------------------------------------------------------- device batches --- */
 /* One pair as the device sees it (built by the host from sequence_pair_t). */
 typedef struct {
@@ -138,6 +153,15 @@ int wfagpu_device_align(wfagpu_device_t *d, int slot, size_t n, const wfagpu_pla
                         int resident);
 int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wfagpu_pair_out_t *out,
                            uint32_t **ops, size_t *ops_used, uint32_t *pair_flags);
+/* wfagpu_device_align with an ends-free span (NULL or all zero: exactly wfagpu_device_align).  A non-zero span runs
+ * the one-diagonal-per-thread kernels with decision-byte traceback on every tier and neither reads nor updates the
+ * provisioning hint of global batches.  -3 for negative values or band > 0 with a non-zero span. */
+int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident,
+                             const wfagpu_span_t *span);
+/* After wfagpu_device_download of an ends-free batch: per pair {k_begin, k_end} (2 n ints), the diagonals of the
+ * alignment's first and last cell: it starts at (max(0, -k_begin), max(0, k_begin)) and ends at offset
+ * min(tlen, plen + k_end).  Pairs that did not finish hold no record.  -1 for a global batch. */
+int wfagpu_device_download_ends(wfagpu_device_t *d, int slot, size_t n, int32_t *ends);
 /* Waits for the slot's stream; event-timed durations (milliseconds) of the pack kernel and of the
  * first pass of the alignment: score bounds + wavefronts + traceback + CIGAR text. */
 int wfagpu_device_wait(wfagpu_device_t *d, int slot, float *ms_pack, float *ms_align);
@@ -180,6 +204,12 @@ int wfagpu_device_pack_only(wfagpu_device_t *d, const char *ascii, size_t ascii_
  * from the reference's backtrace chain.  Appends to `cigar`. */
 bool wfagpu_ops_to_cigar(const char *pattern, size_t plen, const char *text, size_t tlen,
                          int distance, const uint32_t *ops, uint32_t n_ops, wfa_cigar_t *cigar);
+
+/* The same for an ends-free alignment that starts on diagonal `k_begin` (wfagpu_device_download_ends): a leading
+ * I (k_begin > 0) or D run of |k_begin|, the path from (max(0, -k_begin), max(0, k_begin)), and a trailing I / D run
+ * to the end of both sequences; a free run joins the gap run of the same letter next to it. */
+bool wfagpu_ops_to_cigar_span(const char *pattern, size_t plen, const char *text, size_t tlen, int k_begin,
+                              const uint32_t *ops, uint32_t n_ops, wfa_cigar_t *cigar);
 
 /* Appends formatted CIGAR text to a result buffer (growing it like insert_ops does). */
 bool wfagpu_cigar_append(wfa_cigar_t *cigar, const char *text, size_t len);
@@ -227,6 +257,9 @@ int wfagpu_parse_devices(const char *spec, int visible, int *devs, int max_devs)
  * one-diagonal-per-thread kernels, launch bound only -- no per-pair bounds, packed-SIMD kernel, snapshots or
  * provisioning hints.  scores[i] = -1 for a pair it could not finish. */
 int wfagpu_device_rescore(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int32_t *scores);
+/* The same for an ends-free span (NULL = global). */
+int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
+                               const wfagpu_span_t *span, int32_t *scores);
 
 /* Makes room for `bytes` more sequence bytes and `pairs` more pairs in one step (readers, generators). */
 bool wfagpu_reserve(wfagpu_aligner_t *aligner, size_t bytes, size_t pairs);
@@ -257,6 +290,21 @@ void wfagpu_clear_sequences(wfagpu_aligner_t *aligner);
  * `error` (replaces check_cigar_edit + check_affine_distance, utils/verification.c:27-146). */
 bool wfagpu_check_result(const char *pattern, size_t plen, const char *text, size_t tlen,
                          affine_penalties_t pen, unsigned int error, const char *cigar);
+/* The same under an ends-free span: a leading I run of length L costs 0 if L <= text_begin_free, else
+ * o + e (L - text_begin_free); likewise a leading D run (pattern_begin_free), a trailing I run (text_end_free) and a
+ * trailing D run (pattern_end_free).  A run that is both leading and trailing may use both allowances. */
+bool wfagpu_check_result_span(const char *pattern, size_t plen, const char *text, size_t tlen,
+                              affine_penalties_t pen, const wfagpu_span_t *span, unsigned int error, const char *cigar);
+
+/* wfagpu_align with an ends-free span (honours compute_cigar).  False, with a message, for negative values, or for
+ * band > 0 together with a non-zero span.  NULL or all zero: exactly wfagpu_align. */
+bool wfagpu_align_span(wfagpu_aligner_t *aligner, const wfagpu_span_t *span);
+/* launch_alignments / launch_alignments_distance (cigar = false) with an ends-free span; check_correctness validates
+ * every CIGAR under the span and re-computes every score with the same span. */
+void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buffer_size,
+                                   sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                   wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                   const wfagpu_span_t *span);
 
 /* The reference library's generic validators, same names, argument order (text first) and input format
  * (utils/verification.h:37-58): the op string may be UNROLLED ("MMXMMI", what the reference's recover_cigar

@@ -15,6 +15,8 @@
  *   -b/--batch-size B, -w/--workers W
  *   -B/--band L                      adaptive band, re-centred every L scores; "auto"/0 = 25
  *   -c/--check                       validate every result: CIGAR on the host, score against an independent GPU pass
+ *   -F/--ends-free P0,Pf,T0,Tf       ends-free alignment (WFA2-lib's order): that many leading / trailing pattern and
+ *                                    text bases are free; not with -B
  *   -o/--output-file FILE, -p/--print-output, -O/--output-verbose
  * Output lines: "-score\tCIGAR" (or "-score\tCIGAR\tpattern\ttext" with -O).
  * Pairs whose score exceeds -e are NOT sent to a CPU: they are re-dispatched on the GPU.
@@ -31,7 +33,7 @@
 #include "wfagpu_b200.h"
 
 typedef struct {
-    const char *seq, *fq, *ft, *out, *pen, *devices;
+    const char *seq, *fq, *ft, *out, *pen, *devices, *ends_free;
     long n, e, t, b, w, band, stream;
     int have_e, have_t, have_b, have_w, have_band, have_stream, cigar, check, print, verbose;
 } args_t;
@@ -54,6 +56,7 @@ static void usage(void)
             "\t-b, --batch-size B              alignments per batch\n"
             "\t-B, --band L                    banded heuristic, re-centre every L scores (auto = 25)\n"
             "\t-c, --check                     check the alignments\n"
+            "\t-F, --ends-free P0,Pf,T0,Tf     ends-free: free leading/trailing pattern (P) and text (T) bases\n"
             "[System]\n"
             "\t-t, --threads-per-block T       threads per alignment (band width with -B)\n"
             "\t-w, --workers W                 GPU workers (hint)\n"
@@ -70,7 +73,7 @@ static const struct { char s; const char *l; int has_val; } OPTS[] = {
     {'g', "affine-penalties", 1}, {'x', "compute-cigar", 0}, {'c', "check", 0}, {'e', "max-distance", 1},
     {'t', "threads-per-block", 1}, {'b', "batch-size", 1}, {'w', "workers", 1}, {'B', "band", 1},
     {'o', "output-file", 1}, {'p', "print-output", 0}, {'O', "output-verbose", 0}, {'D', "devices", 1},
-    {'S', "stream", 1},
+    {'S', "stream", 1}, {'F', "ends-free", 1},
 };
 
 static int parse(int argc, char **argv, args_t *a)
@@ -97,6 +100,7 @@ static int parse(int argc, char **argv, args_t *a)
         case 'o': a->out = val; break;
         case 'g': a->pen = val; break;
         case 'D': a->devices = val; break;
+        case 'F': a->ends_free = val; break;
         case 'S': a->stream = atol(val); a->have_stream = 1; break;
         case 'n': a->n = atoll(val); break;
         case 'e': a->e = atoll(val); a->have_e = 1; break;
@@ -203,6 +207,18 @@ int main(int argc, char **argv)
     int tpb = a.have_t ? (int)a.t : wfa_get_threads_per_alignment((size_t)max_distance);
     if (a.have_b && a.b <= 0) { fprintf(stderr, "[!] ERROR: Incorrect batch size (%ld).\n", a.b); return -1; }
     int workers = a.have_w ? (int)a.w : get_num_workers(tpb);
+    wfagpu_span_t span = {0, 0, 0, 0};
+    if (a.ends_free) {
+        if (sscanf(a.ends_free, "%d,%d,%d,%d", &span.pattern_begin_free, &span.pattern_end_free, &span.text_begin_free,
+                   &span.text_end_free) != 4 || span.pattern_begin_free < 0 || span.pattern_end_free < 0 ||
+            span.text_begin_free < 0 || span.text_end_free < 0) {
+            fprintf(stderr, "[!] ERROR: --ends-free takes four values >= 0: P0,Pf,T0,Tf (got %s).\n", a.ends_free);
+            return -1;
+        }
+        if (a.have_band) { fprintf(stderr, "[!] ERROR: --ends-free cannot be combined with the band (-B).\n"); return -1; }
+        fprintf(stderr, "INFO: Ends-free alignment: pattern %d,%d text %d,%d free bases at begin,end.\n",
+                span.pattern_begin_free, span.pattern_end_free, span.text_begin_free, span.text_end_free);
+    }
     int band = -1;
     if (a.have_band) {
         if (a.band < 0) { fprintf(stderr, "[!] ERROR: Band must positive (band=%ld).\n", a.band); return -1; }
@@ -253,7 +269,10 @@ int main(int argc, char **argv)
         opt.compute_cigar = a.cigar;
 
         t0 = now_s();
-        if (a.cigar) launch_alignments(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt, a.check);
+        if (a.ends_free)
+            wfagpu_launch_alignments_span(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt,
+                                          a.cigar, a.check, &span);
+        else if (a.cigar) launch_alignments(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt, a.check);
         else launch_alignments_distance(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt, a.check);
         t_align += now_s() - t0;
         ok_run = ok_run && wfagpu_last_launch_ok();

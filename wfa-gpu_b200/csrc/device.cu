@@ -168,7 +168,7 @@ struct Slot {
     PinBuf<uint32_t> h_counters;
     PinBuf<unsigned long long> h_cells;
     PinBuf<wfagpu_step_t> h_steps;
-    int tab_key[5] = {-1, -1, -1, -1, -1};
+    int tab_key[6] = {-1, -1, -1, -1, -1, -1};
     int tab_d_end = 0;
     uint64_t tab_arena_units = 0;
     size_t n = 0;
@@ -177,6 +177,13 @@ struct Slot {
     uint32_t max_len = 0;
     uint32_t kt_max = 0;               /* largest |tlen - plen| of the batch */
     uint32_t minlen_max = 0;           /* largest min(plen, tlen) of the batch */
+    /* ends-free batch (wfagpu_device_align_span with a non-zero span) */
+    bool ef = false;
+    wfagpu_span_t span{};
+    int ef_w = 0;                      /* half width of the start row: max(pb, tb), at most the longest sequence */
+    int ef_ext = 0;                    /* widest end of the target range: max(pe, te), likewise */
+    DevBuf<int2> ends;                 /* per pair {k_begin, k_end} */
+    PinBuf<int2> h_ends;
     size_t budget_cache = 0;           /* arena budget from the last cudaMemGetInfo (0 = ask again) */
     wfagpu_plan_t plan{};
     wfagpu_batch_stats_t stats{};
@@ -354,7 +361,7 @@ extern "C" void wfagpu_device_close_all(void)
             s.scratch.release(); s.steps.release(); s.band_lo.release(); s.gring.release(); s.slots.release(); s.text.release(); s.refs.release(); s.heads.release();
             s.h_text.release(); s.h_refs.release(); s.h_heads.release(); s.h_ascii.release();
             s.h_pairs.release(); s.h_order.release(); s.h_seed.release(); s.h_out.release(); s.h_pool.release();
-            s.h_counters.release(); s.h_cells.release(); s.h_steps.release();
+            s.h_counters.release(); s.h_cells.release(); s.h_steps.release(); s.ends.release(); s.h_ends.release();
             for (auto &ev : s.ev) if (ev) cudaEventDestroy(ev);
             if (s.ev_tab) cudaEventDestroy(s.ev_tab);
             if (s.stream) cudaStreamDestroy(s.stream);
@@ -439,7 +446,7 @@ extern "C" int wfagpu_device_upload(wfagpu_device_t *d, int slot, const char *as
  * 2 x 512 95 k, 3 x 384 109 k -- more, smaller CTAs hide the per-score barrier.
  * `n_want` is the half width the launch should be able to hold. */
 static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_min, uint32_t max_len, size_t n_items,
-                      bool ascii, bool bt, LaunchCfg *c)
+                      bool ascii, bool bt, bool ef, LaunchCfg *c)
 {
     const int A = std::max(o + e, x) + 1, E1 = e + 1, G = A;
     const size_t smem_max = d->prop.sharedMemPerBlockOptin;        /* 227 KB on B200 */
@@ -469,7 +476,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
         c->stages = 1;
         c->n_cap = n_want;
         /* packed pairs: four diagonals per thread with 128-bit loads (wfa_quadg_kernel): rows 16-byte aligned */
-        c->quad = !ascii && !d->no_quad;
+        c->quad = !ascii && !d->no_quad && !ef;       /* ends-free: one diagonal per thread */
         ck = c->quad;
         c->row_stride = rs(n_want);
         c->center = c->quad ? ctr(n_want) : n_want + 2 * G + 1;
@@ -490,7 +497,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
             /* wide wavefronts (50 kbp / 15 %: ~10 k diagonals per score) keep 1024 threads busy: 581 vs 416
              * pairs/s against 512 threads on B200 */
             c->group_threads = d->force_threads ? d->force_threads : (n_want >= 2048 ? 1024 : 512);
-            occ = large_max_ctas_per_sm(c->group_threads, c->smem, ascii, bt);
+            occ = large_max_ctas_per_sm(c->group_threads, c->smem, ascii, bt, ef);
             if (occ < 1) return -1;
             occ = std::min(occ, d->force_ctas_per_sm ? d->force_ctas_per_sm : 2);
         }
@@ -516,11 +523,11 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
     }
     if (!warp) {
         c->groups_per_cta = 1;
-        c->ckpt = bt && !d->no_ckpt;
+        c->ckpt = bt && !d->no_ckpt && !ef;            /* ends-free: decision bytes */
         /* packed pairs on shared-memory rings run four diagonals per thread (with backtrace: snapshots only) */
         /* (measured on B200: 1 kbp / 10 %, ring half width 196: 9.5 ms per 50 k pairs with one diagonal per thread and 16 CTAs per
          * SM against 11.0 ms; from a half width of ~300 on the four-diagonal kernel wins) */
-        c->quad = !ascii && !d->no_quad && (!bt || c->ckpt) && n_want >= d->quad_min;
+        c->quad = !ascii && !d->no_quad && !ef && (!bt || c->ckpt) && n_want >= d->quad_min;
         /* two scores per barrier: score d + 1 must not read the extended M of score d (x >= 2, o + e >= 2) and takes
          * its extend sources from registers (e == 1); costs one more row per ring */
         c->quad_pairs = c->quad && !d->no_quad_pairs && x >= 2 && o + e >= 2 && e == 1;
@@ -542,7 +549,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
          * the arithmetic allowed cost rank 3 of an 8-GPU run its fifth CTA per SM, 33.4 instead of 29.2 ms per step) */
         auto fits = [&](int k, size_t bytes, size_t budget) {
             if (bytes > budget) return false;
-            const int occ_k = c->quad ? quad_max_ctas_per_sm(64, bytes, bt) : exact_max_ctas_per_sm(64, 1, bytes, ascii, bt, c->ckpt);
+            const int occ_k = c->quad ? quad_max_ctas_per_sm(64, bytes, bt) : exact_max_ctas_per_sm(64, 1, bytes, ascii, bt, c->ckpt, ef);
             return occ_k >= k;
         };
         for (int k = kmax; k >= 1 && !best_k; --k) {
@@ -595,7 +602,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
     }
     const int threads = warp ? 32 * c->groups_per_cta : c->group_threads;
     int occ = c->quad ? quad_max_ctas_per_sm(c->group_threads, c->smem, bt)
-                      : exact_max_ctas_per_sm(c->group_threads, c->groups_per_cta, c->smem, ascii, bt, c->ckpt);
+                      : exact_max_ctas_per_sm(c->group_threads, c->groups_per_cta, c->smem, ascii, bt, c->ckpt, ef);
     if (occ < 1) {
         fprintf(stderr, "[wfagpu] kernel configuration does not fit (threads=%d smem=%zu)\n", threads, c->smem);
         return -1;
@@ -679,18 +686,21 @@ static int ensure_step_table(Slot &s, const wfagpu_plan_t &plan, int max_steps)
 {
     const int max_dist = std::min<long long>((long long)max_steps * (std::max(plan.x, plan.o + plan.e) + 1) + 16, 1 << 30);
     const int tab_win = plan.band > 0 ? (plan.band_width > 0 ? plan.band_width : 512) : 0;
+    const int extra = s.ef ? s.ef_w : 0;   /* ends-free: the start row widens every score's range */
     if (s.tab_key[0] == plan.x && s.tab_key[1] == plan.o && s.tab_key[2] == plan.e && s.tab_key[3] == max_steps &&
-        s.tab_key[4] == tab_win)
+        s.tab_key[4] == tab_win && s.tab_key[5] == extra)
         return 0;
     if (s.h_steps.ensure((size_t)max_dist + 1)) return -1;
     if (tables_idle(s)) return -1;        /* a previous pass may still be reading the pinned table */
     uint64_t units = 0;
-    const int de = wfagpu_build_step_table(plan.x, plan.o, plan.e, max_steps, max_dist, tab_win, s.h_steps.p, &units);
+    const int de = extra ? wfagpu_build_step_table_span(plan.x, plan.o, plan.e, max_steps, max_dist, extra, s.h_steps.p, &units)
+                         : wfagpu_build_step_table(plan.x, plan.o, plan.e, max_steps, max_dist, tab_win, s.h_steps.p, &units);
     if (de < 1) return -1;
     if (s.steps.ensure((size_t)de + 1)) return -1;
     CK(cudaMemcpyAsync(s.steps.p, s.h_steps.p, (size_t)de * sizeof(wfagpu_step_t), cudaMemcpyHostToDevice, s.stream));
     if (tables_sent(s)) return -1;
     s.tab_key[0] = plan.x; s.tab_key[1] = plan.o; s.tab_key[2] = plan.e; s.tab_key[3] = max_steps; s.tab_key[4] = tab_win;
+    s.tab_key[5] = extra;
     s.tab_d_end = de;
     s.tab_arena_units = units;
     s.ck_key[0] = -1;     /* snapshot offsets follow the table */
@@ -738,6 +748,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
 {
     HostTrace tr;
     if (first_pass) pull_hint(d);            /* what the last batch on this GPU needed (any context) */
+    if (first_pass && s.ef) { d->hint_dist = 0; d->hint_mean = 0; }     /* ends-free: hints of global batches do not apply */
     if (ensure_step_table(s, plan, max_steps)) return -1;
     const wfagpu_step_t *tab = s.h_steps.p;
     const int d_full = s.tab_d_end;
@@ -851,9 +862,11 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
     const int pen_e = plan.e;
     const long long kt_max = s.kt_max;
     auto n_need = [&](int d_end) -> int {
-        /* n_d grows, kt + (Dmax - d) / e shrinks: the largest min sits where they cross */
+        /* n_d grows, kt + (Dmax - d) / e shrinks: the largest min sits where they cross.  A global pair with |kt| > Dmax / e
+         * cannot finish; an ends-free one can (the start row and the target range may meet at no cost), and its window
+         * reaches max(pe, te) beyond kt: no clamp, n_d bounds it */
         const long long Dmax = d_end - 1;
-        const long long ktm = std::min<long long>(kt_max, Dmax / pen_e);
+        const long long ktm = s.ef ? kt_max + s.ef_ext : std::min<long long>(kt_max, Dmax / pen_e);
         int lo = 0, hi = d_end;                      /* first d with n_d >= ktm + (Dmax - d) / e */
         while (lo < hi) {
             const int mid = (lo + hi) / 2;
@@ -909,7 +922,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         if (occ < 1) return -1;
         c.ctas = (int)std::max<size_t>(1, std::min<size_t>((size_t)occ * d->prop.multiProcessorCount, n_items));
     } else {
-        rc = choose_cfg(d, plan.x, plan.o, plan.e, n_want, n_min, s.max_len, n_items, ascii, plan.with_cigar != 0, &c);
+        rc = choose_cfg(d, plan.x, plan.o, plan.e, n_want, n_min, s.max_len, n_items, ascii, plan.with_cigar != 0, s.ef, &c);
     }
     if (rc) return rc;
     tr.mark("cfg");
@@ -1078,6 +1091,11 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
     kp.ascii_list = s.ascii_list.p;
     kp.ascii_count = s.counters.p + CTR_ASCII;
     kp.cells = d->count_cells ? s.cells.p : nullptr;
+    if (s.ef) {
+        kp.ef_pb = s.span.pattern_begin_free; kp.ef_pe = s.span.pattern_end_free;
+        kp.ef_tb = s.span.text_begin_free; kp.ef_te = s.span.text_end_free;
+        kp.ends = s.ends.p;
+    }
     if (env_int("WFAGPU_VERBOSE", 0))
         fprintf(stderr, "[wfagpu] pass: items=%zu max_steps=%d n_cap=%d d_end=%d group=%d x%d ctas=%d stages=%d smem=%zu ascii=%d band=%d tier=%s period=%d arena=%.1f MB\n",
                 n_items, max_steps, c.n_cap, d_end, c.group_threads, c.groups_per_cta, c.ctas, c.stages, c.smem,
@@ -1181,6 +1199,7 @@ static int enqueue_text(wfagpu_device *d, Slot &s, size_t n, int d_end_bound)
     cp.text_head = s.heads.p + 1;
     cp.refs = s.refs.p;
     cp.overflow = reinterpret_cast<uint32_t *>(s.heads.p + 2);
+    cp.ends = s.ef ? s.ends.p : nullptr;
     launch_cigar_text(cp, s.stream);
     CK(cudaGetLastError());
     s.stats.launches += 2;
@@ -1192,8 +1211,25 @@ static int enqueue_text(wfagpu_device *d, Slot &s, size_t n, int d_end_bound)
 
 extern "C" int wfagpu_device_align(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident)
 {
+    return wfagpu_device_align_span(d, slot, n, plan, resident, nullptr);
+}
+
+extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident,
+                                        const wfagpu_span_t *span)
+{
     (void)resident;
     if (!d || slot < 0 || slot > 1 || !plan) return -1;
+    const wfagpu_span_t sp = span ? *span : wfagpu_span_t{0, 0, 0, 0};
+    if (sp.pattern_begin_free < 0 || sp.pattern_end_free < 0 || sp.text_begin_free < 0 || sp.text_end_free < 0) {
+        fprintf(stderr, "[wfagpu] ends-free span values must be >= 0 (got %d,%d,%d,%d)\n", sp.pattern_begin_free,
+                sp.pattern_end_free, sp.text_begin_free, sp.text_end_free);
+        return -3;
+    }
+    const bool ef = sp.pattern_begin_free || sp.pattern_end_free || sp.text_begin_free || sp.text_end_free;
+    if (ef && plan->band > 0) {
+        fprintf(stderr, "[wfagpu] ends-free alignment is exact only: it cannot be combined with the adaptive band\n");
+        return -3;
+    }
     if (plan->x < 1 || plan->e < 1 || plan->o < 0) {
         /* x = 0 or e = 0 make a wavefront its own source (and divide by zero in the pruning quotient) */
         fprintf(stderr, "[wfagpu] penalties must satisfy x >= 1, e >= 1, o >= 0 (got %d,%d,%d)\n", plan->x, plan->o, plan->e);
@@ -1203,7 +1239,21 @@ extern "C" int wfagpu_device_align(wfagpu_device_t *d, int slot, size_t n, const
     Slot &s = d->slots[slot];
     if (n != s.n) return -1;
     s.plan = *plan;
+    s.ef = ef;
+    s.span = sp;
+    /* the span clamped to every pair, then the widest of the batch: the start row's half width and the reach of the
+     * target range beyond kt (the step table and the rings are shared by the pairs of a batch) */
+    s.ef_w = 0;
+    s.ef_ext = 0;
+    if (ef) {
+        for (size_t i = 0; i < n; ++i) {
+            const int pl = (int)s.h_pairs.p[i].plen, tl = (int)s.h_pairs.p[i].tlen;
+            s.ef_w = std::max(s.ef_w, std::max(std::min(sp.pattern_begin_free, pl), std::min(sp.text_begin_free, tl)));
+            s.ef_ext = std::max(s.ef_ext, std::max(std::min(sp.pattern_end_free, pl), std::min(sp.text_end_free, tl)));
+        }
+    }
     if (n == 0) return 0;
+    if (ef && (s.ends.ensure(n) || s.h_ends.ensure(n))) return -1;
     /* the batch may be re-aligned while it stays resident: start from clean counters */
     s.stats.launches = 0;
     s.stats.redispatched = 0;
@@ -1224,7 +1274,7 @@ extern "C" int wfagpu_device_align(wfagpu_device_t *d, int slot, size_t n, const
      * given that budget straight away: 100 k x 1 kbp / 10 % with -e 300 re-dispatched 4.4 % of its pairs in every chunk. */
     int first_steps = plan->max_steps;
     pull_hint(d);
-    if (plan->band <= 0 && d->hint_dist > 0 && d->hint_lift_pm > 0 && d->hint_key[0] == plan->x && d->hint_key[1] == plan->o &&
+    if (!ef && plan->band <= 0 && d->hint_dist > 0 && d->hint_lift_pm > 0 && d->hint_key[0] == plan->x && d->hint_key[1] == plan->o &&
         d->hint_key[2] == plan->e && d->hint_key[3] == length_class(s.max_len)) {
         const long long want = (long long)d->hint_dist + (long long)d->hint_dist * d->hint_margin_pm / 1000 + 12;
         const long long most = (long long)plan->max_steps + (long long)plan->max_steps * d->hint_lift_pm / 1000;
@@ -1376,7 +1426,7 @@ extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wf
     }
     s.stats.failed_pairs = (uint32_t)failed.size();
     memcpy(out, s.h_out.p, n * sizeof(wfagpu_pair_out_t));
-    if (!d->independent) learn_hint(d, s, n);
+    if (!d->independent && !s.ef) learn_hint(d, s, n);
     if (pair_flags)
         for (size_t i = 0; i < n; ++i) pair_flags[i] = s.h_pairs.p[i].flags;
     if (ops) *ops = s.h_pool.p;
@@ -1394,6 +1444,12 @@ extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wf
 
 extern "C" int wfagpu_device_rescore(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int32_t *scores)
 {
+    return wfagpu_device_rescore_span(d, slot, n, plan, nullptr, scores);
+}
+
+extern "C" int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
+                                          const wfagpu_span_t *span, int32_t *scores)
+{
     if (!d || !plan || !scores || slot < 0 || slot > 1) return -1;
     if (n != d->slots[slot].n) return -1;
     /* a different code path on purpose: what it shares with the production path is the packing, the step table
@@ -1404,11 +1460,24 @@ extern "C" int wfagpu_device_rescore(wfagpu_device_t *d, int slot, size_t n, con
     wfagpu_plan_t p2 = *plan;
     p2.with_cigar = 0;
     std::vector<wfagpu_pair_out_t> out(n);
-    int rc = wfagpu_device_align(d, slot, n, &p2, 1);
+    int rc = wfagpu_device_align_span(d, slot, n, &p2, 1, span);
     if (!rc) rc = wfagpu_device_download(d, slot, n, out.data(), nullptr, nullptr, nullptr);
     d->no_bound = nb; d->no_quad = nq; d->use_hint = uh; d->force_warp = fw; d->independent = false;
     if (rc) return rc;
     for (size_t i = 0; i < n; ++i) scores[i] = (out[i].status & WFAGPU_ST_FINISHED) ? out[i].distance : -1;
+    return 0;
+}
+
+extern "C" int wfagpu_device_download_ends(wfagpu_device_t *d, int slot, size_t n, int32_t *ends)
+{
+    if (!d || slot < 0 || slot > 1 || (!ends && n)) return -1;
+    CK(cudaSetDevice(d->dev));
+    Slot &s = d->slots[slot];
+    if (n != s.n || !s.ef) return -1;
+    if (n == 0) return 0;
+    CK(cudaMemcpyAsync(s.h_ends.p, s.ends.p, n * sizeof(int2), cudaMemcpyDeviceToHost, s.stream));
+    CK(cudaStreamSynchronize(s.stream));
+    memcpy(ends, s.h_ends.p, n * sizeof(int2));
     return 0;
 }
 
@@ -1428,7 +1497,7 @@ extern "C" int wfagpu_device_wait(wfagpu_device_t *d, int slot, float *ms_pack, 
         CK(cudaStreamSynchronize(s.stream));
         s.stats.pending_pairs = s.h_counters.p[CTR_RETRY] + s.h_counters.p[CTR_ASCII];
     }
-    if (s.n && d->use_hint) {
+    if (s.n && d->use_hint && !s.ef) {
         /* read the result records back (16 B per pair) so that a re-run of the resident
          * batch is provisioned like the next batch of a stream would be */
         if (s.h_out.ensure(s.n)) return -1;

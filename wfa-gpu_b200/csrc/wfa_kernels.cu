@@ -4,6 +4,7 @@
  */
 #include "wfa_kernels.cuh"
 
+#include <climits>
 #include <mutex>
 #include <unordered_map>
 #include <unordered_set>
@@ -431,13 +432,24 @@ __device__ __forceinline__ bool prune_window(int n, int kt, int q, int n_cap, in
     return live;
 }
 
+/* The same for an ends-free alignment: the diagonals within q of the target range [tlo, thi]. */
+__device__ __forceinline__ bool prune_window_range(int n, int tlo, int thi, int q, int n_cap, int &lo, int &hi)
+{
+    lo = max(-n, tlo - q);
+    hi = min(n, thi + q);
+    const bool live = lo <= hi;
+    if (!live) { hi = min(n, n_cap); lo = -hi; }
+    return live;
+}
+
 struct GroupCtl {
     uint64_t bar[2];     /* TMA completion barriers, one per sequence stage */
     uint32_t idx[2];     /* pair index staged in each buffer                */
     uint32_t n_ops;
     uint32_t ops_off;
     uint32_t pos[2];     /* queue position of that pair (its snapshot arena) */
-    uint32_t pad[2];
+    int32_t k_end;       /* ends-free CTA kernels: lowest finishing diagonal of the current score */
+    uint32_t pad;
 };
 
 /* Per-score schedule record (CTA-per-pair kernels with shared-memory rings).  Everything a thread
@@ -460,11 +472,17 @@ constexpr uint32_t kSchedBytes = 2u * kSchedBlock * (uint32_t)sizeof(StepRec);
 /* CKPT (CTA per pair, shared-memory rings, with backtrace): instead of a decision byte per
  * cell the forward pass snapshots the ring rows every p.ck_period scores, and the traceback
  * recomputes the offsets it needs on the dependency cone below the cell it stands on
- * (model + proof of equivalence: oracle/kernel_model.c, km_align_pair_ckpt). */
-template <bool WARP, bool ASCII, bool BT, typename R, bool CKPT>
+ * (model + proof of equivalence: oracle/kernel_model.c, km_align_pair_ckpt).
+ *
+ * EF (ends-free, DESIGN.md §9): score 0 holds the extend of (max(0, -k), max(0, k)) on every diagonal of
+ * [-pb, tb]; the pruning measures the distance to the target range [kt - te, kt + pe] instead of kt; an M cell on
+ * a target diagonal finishes when its offset reaches min(tlen, plen + k), the lowest such k of the first finishing
+ * score wins; the traceback starts there and stops at score 0.  k_begin / k_end go to p.ends[idx]. */
+template <bool WARP, bool ASCII, bool BT, typename R, bool CKPT, bool EF = false>
 __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_kernel(const __grid_constant__ KernelParams p)
 {
     static_assert(!CKPT || (BT && !WARP && R::kElem == 2), "checkpointed traceback: CTA groups with shared-memory rings");
+    static_assert(!(EF && CKPT), "ends-free: decision-byte traceback only");
     using G = Group<WARP>;
     using RA = typename R::addr_t;
     constexpr bool GR = (R::kElem == 4);          /* rings in global memory */
@@ -551,6 +569,9 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
         const wfagpu_pair_t pr = p.pairs[idx];
         const int plen = (int)pr.plen, tlen = (int)pr.tlen;
         const int kt = tlen - plen;
+        /* ends-free: the span clamped to this pair, and its target diagonals */
+        const int ef_pb = EF ? min(p.ef_pb, plen) : 0, ef_tb = EF ? min(p.ef_tb, tlen) : 0;
+        const int klo_t = EF ? kt - min(p.ef_te, tlen) : kt, khi_t = EF ? kt + min(p.ef_pe, plen) : kt;
 
         const uint32_t Pa = seq_sa + (uint32_t)(2 * stage) * seq_bytes;
         const uint32_t Ta = Pa + seq_bytes;
@@ -565,7 +586,18 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
         const bool skip = !ASCII && (pr.flags & WFAGPU_PAIR_HAS_N);
 
         /* ---- ring prologue: NULL over [-2G, 2G] on every row (no full re-init) ---- */
-        {
+        if constexpr (EF) {
+            /* ... widened by the start row's half width (steps[0].n): the windows of the first A scores reach W + G */
+            const int wz = min((int)p.steps[0].n, p.n_cap);
+            const int span = 4 * GW + 2 * wz + 1;
+            const int total = rows * span;
+            for (int i = tid; i < total; i += gsz) {
+                const int r = i / span;
+                const int k = i - r * span - 2 * GW - wz;
+                R::st(R::add(M0, (uint32_t)r * row_bytes), k, NULLV);
+            }
+            if (tid == 0) ctl->k_end = INT_MAX;
+        } else {
             const int span = 4 * GW + 1;
             const int total = rows * span;
             for (int i = tid; i < total; i += gsz) {
@@ -580,6 +612,18 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
 
         int dist = 0;
         bool finished = false;
+        int k_end = kt;                              /* ends-free: diagonal of the finishing cell */
+        /* ends-free end test: the lowest finishing diagonal of the group (kb = INT_MAX: none on this thread); also the
+         * barrier after the score's cells */
+        auto ef_lowest = [&](int kb) -> int {
+            if constexpr (WARP) {
+                __syncwarp();
+                return __reduce_min_sync(0xffffffffu, kb);
+            } else {
+                if (kb != INT_MAX) atomicMin(&ctl->k_end, kb);
+                return __syncthreads_or(kb != INT_MAX) ? ctl->k_end : INT_MAX;
+            }
+        };
 
         if (!skip) {
             /* Score-bound pruning: this launch only reports pairs that finish with a score <= Dmax
@@ -587,7 +631,8 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
              * and the target diagonal kt costs at least one gap extension, so a cell (d, k) with
              * d + e * |k - kt| > Dmax cannot be on such an alignment.  Those cells are not computed and
              * read as NULL; the cells of the optimal path keep their offsets and win the same
-             * tie-breaks (proof and poisoned-cell model: oracle/kernel_model.c, km_prune_range). */
+             * tie-breaks (proof and poisoned-cell model: oracle/kernel_model.c, km_prune_range).
+             * Ends-free: the same with the distance to the target range. */
             const int Dmax = p.bound ? min(p.d_end - 1, p.bound[idx]) : p.d_end - 1;
             /* schedule records of scores dbase .. dbase + kSchedBlock - 1 (warp 0, one score per lane) */
             auto fill_sched = [&](int dbase, int buf) {
@@ -599,12 +644,13 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                     if (d <= Dmax) {
                         const wfagpu_step_t st = p.steps[d];
                         int lo, hi;
-                        const bool live = prune_window((int)st.n, kt, (Dmax - d) / e, p.n_cap, lo, hi);
+                        const bool live = EF ? prune_window_range((int)st.n, klo_t, khi_t, (Dmax - d) / e, p.n_cap, lo, hi)
+                                             : prune_window((int)st.n, kt, (Dmax - d) / e, p.n_cap, lo, hi);
                         const bool stop = live && (lo < -p.n_cap || hi > p.n_cap);     /* wider than the rings */
                         const bool work = live && st.kind != WFAGPU_STEP_NULL;
                         r.lo = lo; r.hi = hi; r.n = (int)st.n;
                         r.flags = (uint32_t)st.kind | (live ? kRecLive : 0u) | (stop ? kRecStop : 0u) |
-                                  ((work && kt >= lo && kt <= hi) ? kRecTarget : 0u) |
+                                  ((work && (EF ? (khi_t >= lo && klo_t <= hi) : (kt >= lo && kt <= hi))) ? kRecTarget : 0u) |
                                   ((CKPT && d % p.ck_period == 0) ? kRecSnap : 0u);
                         r.ck_j = CKPT ? (uint32_t)(d / p.ck_period) : st.row_off;    /* snapshot index, or decision row */
                         const int dm = d % A, de1 = d % E1;
@@ -625,11 +671,32 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                     sts_v4(a + 32u, make_uint4(r.aIe, r.aDc, r.aDe, r.ck_j));
                 }
             };
-            if (tid == 0) R::st(M0, 0, extend(0, 0));
-            if (SCHED && tid < kSchedBlock) fill_sched(1, 0);
-            G::sync();
-            if (kt == 0 && R::ld(M0, 0) == tlen) {
-                finished = true;
+            bool stop0 = false;                      /* ends-free: finished (or too wide for the rings) at score 0 */
+            if constexpr (EF) {
+                /* score 0: the start row [-pb, tb], within the pruning window of score 0 */
+                int lo0, hi0;
+                const bool live0 = prune_window_range((int)p.steps[0].n, klo_t, khi_t, Dmax / e, p.n_cap, lo0, hi0);
+                const int slo = live0 ? max(-ef_pb, lo0) : 1, shi = live0 ? min(ef_tb, hi0) : 0;
+                int kb = INT_MAX;
+                if (slo >= -p.n_cap && shi <= p.n_cap) {
+                    for (int k = slo + tid; k <= shi; k += gsz) {
+                        const int m = extend(k, max(0, k));
+                        R::st(M0, k, m);
+                        if (k >= klo_t && k <= khi_t && m == min(tlen, plen + k)) kb = min(kb, k);
+                    }
+                } else {
+                    stop0 = true;                    /* re-dispatched with wider rings */
+                }
+                if (SCHED && tid < kSchedBlock) fill_sched(1, 0);
+                kb = ef_lowest(kb);
+                if (kb != INT_MAX) { finished = true; k_end = kb; stop0 = true; }
+            } else {
+                if (tid == 0) R::st(M0, 0, extend(0, 0));
+                if (SCHED && tid < kSchedBlock) fill_sched(1, 0);
+                G::sync();
+            }
+            if (EF ? stop0 : (kt == 0 && R::ld(M0, 0) == tlen)) {
+                finished = EF ? finished : true;
             } else {
                 wfagpu_step_t st_next = p.steps[1 < p.d_end ? 1 : 0];
                 /* Row addresses of the current score and of its sources are carried from
@@ -701,7 +768,8 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                         kind = st.kind;
                         row_off = st.row_off;
                         if (pr_r == 0) { pr_r = e - 1; --pr_q; } else --pr_r;
-                        live = prune_window(n, kt, pr_q, p.n_cap, lo, hi);
+                        live = EF ? prune_window_range(n, klo_t, khi_t, pr_q, p.n_cap, lo, hi)
+                                  : prune_window(n, kt, pr_q, p.n_cap, lo, hi);
                         if (live && (lo < -p.n_cap || hi > p.n_cap)) break;     /* wider than the rings of this launch */
                         if (live && kind != WFAGPU_STEP_NULL) n_cells += (unsigned)(hi - lo + 1);
                         target_in = live && kind != WFAGPU_STEP_NULL && kt >= lo && kt <= hi;
@@ -726,6 +794,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                         if (CKPT && snap_now) checkpoint(n, lo, hi);
                         continue;
                     }
+                    int kb = INT_MAX;                            /* ends-free: lowest finishing diagonal of this thread */
                     if (kind == WFAGPU_STEP_M) {
                         for (int k = lo - GW + tid; k <= hi + GW; k += gsz) {
                             R::st(aIc, k, NULLV);
@@ -734,6 +803,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                             if (k >= lo && k <= hi) {
                                 m = R::ld(aMx, k) + 1;
                                 if (m >= 0) m = extend(k, m);
+                                if (EF && k >= klo_t && k <= khi_t && m == min(tlen, plen + k)) kb = min(kb, k);
                             }
                             R::st(aMc, k, m);
                         }
@@ -768,13 +838,24 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                             R::st(aDc, k, D);
                             R::st(aMc, k, M);
                             if (BT && !CKPT) rowb[k] = (uint8_t)((bI ? 1u : 0u) | (bD ? 2u : 0u) | (bM0 ? 4u : 0u) | (bM1 ? 8u : 0u));
+                            if (EF && k >= klo_t && k <= khi_t && M == min(tlen, plen + k)) kb = min(kb, k);
                         }
                     }
-                    G::sync();
-                    if (target_in && R::ld(aMc, kt) == tlen) {
-                        finished = true;
-                        dist = d;
-                        break;
+                    if constexpr (EF) {
+                        kb = ef_lowest(kb);
+                        if (kb != INT_MAX) {
+                            finished = true;
+                            dist = d;
+                            k_end = kb;
+                            break;
+                        }
+                    } else {
+                        G::sync();
+                        if (target_in && R::ld(aMc, kt) == tlen) {
+                            finished = true;
+                            dist = d;
+                            break;
+                        }
                     }
                     if (CKPT && snap_now) checkpoint(n, lo, hi);
                 }
@@ -786,9 +867,10 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
         uint32_t n_ops = 0;
         if (tid == 0) {
             uint32_t ops_off = 0;
+            int k_begin = k_end;                     /* ends-free: diagonal of the path's score-0 cell */
             if (BT && finished && dist > 0) {
               if constexpr (!CKPT) {
-                int cd = dist, ck = kt, comp = 0;
+                int cd = dist, ck = EF ? k_end : kt, comp = 0;
                 uint32_t word = 0;
                 while (!(comp == 0 && cd == 0)) {
                     const wfagpu_step_t st = p.steps[cd];
@@ -832,8 +914,10 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                 const uint32_t nw = (n_ops + 15u) >> 4;
                 ops_off = atomicAdd(p.ops_pool_head, nw);
                 if (ops_off + nw > p.ops_pool_words) { n_ops = 0; finished = false; }
+                if (EF) k_begin = ck;
               }
             }
+            if (EF && finished) p.ends[idx] = make_int2(k_begin, k_end);
             ctl->n_ops = n_ops;
             ctl->ops_off = ops_off;
             wfagpu_pair_out_t r;
@@ -2935,7 +3019,11 @@ __device__ __forceinline__ uint32_t match_run_warp(const char *__restrict__ P, c
 }
 
 /* One warp per pair.  The op walk is sequential; the warp shares the match-run scans
- * (coalesced 32-byte reads of both sequences) and lane 0 prints. */
+ * (coalesced 32-byte reads of both sequences) and lane 0 prints.
+ * EF (ends-free, p.ends): the walk starts at (max(0, -k0), max(0, k0)) behind a leading I / D run of |k0| and ends
+ * with the trailing I / D run to the end of both sequences; a free run joins the gap run of the same letter next to
+ * it (wfagpu_ops_to_cigar_span prints the same text on the host). */
+template <bool EF>
 __global__ void __launch_bounds__(256) cigar_text_kernel(CigarParams p)
 {
     const uint32_t i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -2947,6 +3035,70 @@ __global__ void __launch_bounds__(256) cigar_text_kernel(CigarParams p)
     const wfagpu_pair_t pr = p.pairs[i];
     const char *P = p.ascii + pr.p_ascii, *T = p.ascii + pr.t_ascii;
     const int plen = (int)pr.plen, tlen = (int)pr.tlen;
+    if constexpr (EF) {
+        /* every op prints at most 10 characters; plus the leading, last match and trailing runs (11 each) */
+        const uint32_t cap = (10u * o.n_ops + 40u + 7u) & ~7u;
+        unsigned long long slot = 0;
+        if (lane == 0) slot = atomicAdd(p.slot_head, (unsigned long long)cap);
+        slot = __shfl_sync(0xffffffffu, slot, 0);
+        if (slot + cap > p.slot_bytes) {
+            if (lane == 0) { p.refs[i] = ref; atomicOr(p.overflow, 1u); }
+            return;
+        }
+        char *dst = p.slots + slot;
+        uint32_t pos = 0;
+        const int k0 = p.ends[i].x;
+        const uint32_t *ops = p.ops_pool + o.ops_off;
+        int k = k0, off = max(0, k0);
+        bool in_gap = false;
+        uint32_t run_op = k0 > 0 ? OP_INS : (k0 < 0 ? OP_DEL : OP_NOOP), run_len = (uint32_t)abs(k0);
+        uint32_t word = 0;
+        for (uint32_t j = o.n_ops; j-- > 0;) {
+            if ((j & 15u) == 15u || j == o.n_ops - 1) word = ops[j >> 4];
+            uint32_t op = (word >> (2u * (j & 15u))) & 3u;
+            /* the newest op closing a gap: hold the gap run, the trailing run may join it */
+            const bool hold = j == 0 && in_gap && op == OP_SUB;
+            if (op != run_op && run_len && !hold) { if (lane == 0) pos = put_run(dst, pos, run_len, "?IXD"[run_op]); run_len = 0; }
+            if (!in_gap) {
+                const uint32_t m = match_run_warp(P, T, plen, tlen, off - k, off, lane);
+                if (m) {
+                    if (run_len) { if (lane == 0) pos = put_run(dst, pos, run_len, "?IXD"[run_op]); run_len = 0; }
+                    if (lane == 0) pos = put_run(dst, pos, m, 'M');
+                    off += (int)m;
+                }
+            }
+            if (op == OP_DEL) { in_gap = true; --k; ++run_len; }
+            else if (op == OP_INS) { in_gap = true; ++k; ++off; ++run_len; }
+            else if (op == OP_SUB) {
+                if (in_gap) { in_gap = false; op = hold ? run_op : OP_NOOP; }
+                else { ++off; ++run_len; }
+            }
+            run_op = op;
+        }
+        const uint32_t m = in_gap ? 0u : match_run_warp(P, T, plen, tlen, off - k, off, lane);
+        if (m) {
+            if (run_len && lane == 0) pos = put_run(dst, pos, run_len, "?IXD"[run_op]);
+            run_len = 0;
+            if (lane == 0) pos = put_run(dst, pos, m, 'M');
+            off += (int)m;
+        }
+        const uint32_t tail_i = (uint32_t)(tlen - off), tail_d = (uint32_t)(plen - (off - k));
+        const uint32_t tail = tail_i ? tail_i : tail_d, tail_op = tail_i ? OP_INS : OP_DEL;
+        if (tail) {
+            if (run_len && run_op == tail_op) run_len += tail;
+            else {
+                if (run_len && lane == 0) pos = put_run(dst, pos, run_len, "?IXD"[run_op]);
+                run_op = tail_op; run_len = tail;
+            }
+        }
+        if (run_len && lane == 0) pos = put_run(dst, pos, run_len, "?IXD"[run_op]);
+        if (lane == 0) {
+            ref.off = (uint32_t)(slot >> 3);
+            ref.len = pos;
+            p.refs[i] = ref;
+        }
+        return;
+    }
     /* every op prints at most "1X" + "NNNNNNNM": 10 characters; plus the leading/trailing run */
     const uint32_t cap = (10u * o.n_ops + 24u + 7u) & ~7u;
     unsigned long long slot = 0;
@@ -3018,26 +3170,27 @@ __global__ void __launch_bounds__(256) cigar_compact_kernel(CigarParams p)
 void launch_cigar_text(const CigarParams &p, cudaStream_t s)
 {
     if (p.n_pairs == 0) return;
-    cigar_text_kernel<<<(p.n_pairs + 7) / 8, 256, 0, s>>>(p);
+    if (p.ends) cigar_text_kernel<true><<<(p.n_pairs + 7) / 8, 256, 0, s>>>(p);
+    else cigar_text_kernel<false><<<(p.n_pairs + 7) / 8, 256, 0, s>>>(p);
     cigar_compact_kernel<<<(p.n_pairs + 7) / 8, 256, 0, s>>>(p);
 }
 
 /* ---- host-side launch helpers ---------------------------------------------- */
 
-template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false>
+template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false>
 static cudaError_t launch_one(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
 {
-    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT>;
+    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF>;
     cudaError_t err = allow_max_smem(kfn);
     if (err != cudaSuccess) return err;
     kfn<<<ctas, threads, smem, s>>>(p);
     return cudaGetLastError();
 }
 
-template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false>
+template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false>
 static int occupancy_one(int threads, size_t smem)
 {
-    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT>;
+    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF>;
     int n = 0;
     if (allow_max_smem(kfn) != cudaSuccess) return 0;
     if (occupancy_of(&n, kfn, threads, smem) != cudaSuccess) return 0;
@@ -3119,6 +3272,18 @@ int traceback_max_ctas_per_sm(int A, int period, int warps, bool ascii)
           : (ascii ? (bt ? FN<false, true, true>(__VA_ARGS__) : FN<false, true, false>(__VA_ARGS__))     \
                    : (bt ? FN<false, false, true>(__VA_ARGS__) : FN<false, false, false>(__VA_ARGS__))))
 
+/* ends-free instantiations: FN<WARP, ASCII, BT, RingS16, false, true> */
+template <bool WARP, bool ASCII, bool BT>
+static cudaError_t launch_one_ef(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
+{
+    return launch_one<WARP, ASCII, BT, RingS16, false, true>(p, threads, ctas, smem, s);
+}
+template <bool WARP, bool ASCII, bool BT>
+static int occupancy_one_ef(int threads, size_t smem)
+{
+    return occupancy_one<WARP, ASCII, BT, RingS16, false, true>(threads, smem);
+}
+
 template <bool BT, bool COUNT>
 static cudaError_t launch_quad_one(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
 {
@@ -3193,6 +3358,17 @@ cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_pe
     const bool warp = (group_threads == 32);
     const bool bt = p.with_bt != 0;
     const int threads = warp ? 32 * groups_per_cta : group_threads;
+    if (p.ends) {
+        /* ends-free: decision-byte traceback on every tier */
+        if (p.ck_off) return cudaErrorInvalidValue;
+        if (p.gring) {
+            if (ascii) return bt ? launch_one<false, true, true, RingG32, false, true>(p, threads, ctas, smem_bytes, s)
+                                 : launch_one<false, true, false, RingG32, false, true>(p, threads, ctas, smem_bytes, s);
+            return bt ? launch_one<false, false, true, RingG32, false, true>(p, threads, ctas, smem_bytes, s)
+                      : launch_one<false, false, false, RingG32, false, true>(p, threads, ctas, smem_bytes, s);
+        }
+        return WFAGPU_DISPATCH(launch_one_ef, p, threads, ctas, smem_bytes, s);
+    }
     if (p.gring) {
         /* large tier: CTA per pair, rings in global memory, int32 offsets */
         if (ascii) return bt ? launch_one<false, true, true, RingG32>(p, threads, ctas, smem_bytes, s)
@@ -3209,18 +3385,26 @@ cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_pe
     return WFAGPU_DISPATCH(launch_one, p, threads, ctas, smem_bytes, s);
 }
 
-int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii, bool bt)
+int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii, bool bt, bool ef)
 {
+    if (ef) {
+        if (ascii) return bt ? occupancy_one<false, true, true, RingG32, false, true>(threads, smem_bytes)
+                             : occupancy_one<false, true, false, RingG32, false, true>(threads, smem_bytes);
+        return bt ? occupancy_one<false, false, true, RingG32, false, true>(threads, smem_bytes)
+                  : occupancy_one<false, false, false, RingG32, false, true>(threads, smem_bytes);
+    }
     if (ascii) return bt ? occupancy_one<false, true, true, RingG32>(threads, smem_bytes)
                          : occupancy_one<false, true, false, RingG32>(threads, smem_bytes);
     return bt ? occupancy_one<false, false, true, RingG32>(threads, smem_bytes)
               : occupancy_one<false, false, false, RingG32>(threads, smem_bytes);
 }
 
-int exact_max_ctas_per_sm(int group_threads, int groups_per_cta, size_t smem_bytes, bool ascii, bool bt, bool ckpt)
+int exact_max_ctas_per_sm(int group_threads, int groups_per_cta, size_t smem_bytes, bool ascii, bool bt, bool ckpt,
+                          bool ef)
 {
     const bool warp = (group_threads == 32);
     const int threads = warp ? 32 * groups_per_cta : group_threads;
+    if (ef) return WFAGPU_DISPATCH(occupancy_one_ef, threads, smem_bytes);
     if (ckpt) return ascii ? occupancy_one<false, true, true, RingS16, true>(threads, smem_bytes)
                            : occupancy_one<false, false, true, RingS16, true>(threads, smem_bytes);
     return WFAGPU_DISPATCH(occupancy_one, threads, smem_bytes);

@@ -87,6 +87,10 @@ struct KernelParams {
     uint32_t *ascii_list;         /* pairs the packer flagged (byte-compare launch)          */
     uint32_t *ascii_count;
     unsigned long long *cells;    /* optional work counter (may be null)                     */
+    /* ends-free alignment (wfa_exact_kernel<..., EF = true>): free leading / trailing bases of the pattern and the
+     * text, clamped per pair; the step table's half widths include the start row's max(pb, tb) */
+    int ef_pb, ef_pe, ef_tb, ef_te;
+    int2 *ends;                   /* ends-free: per pair {k_begin, k_end}; null in global mode */
 };
 
 struct PackParams {
@@ -109,11 +113,13 @@ struct CigarParams {
     unsigned long long *text_head;
     wfagpu_cigar_ref_t *refs;         /* per pair: offset (bytes) + length of its text          */
     uint32_t *overflow;
+    const int2 *ends;                 /* ends-free: per pair {k_begin, k_end} (leading / trailing runs); null = global */
 };
 
 void launch_pack(const PackParams &p, cudaStream_t s);
 void launch_cigar_text(const CigarParams &p, cudaStream_t s);
-/* group_threads == 32 -> warp-per-pair variant; otherwise CTA-per-pair */
+/* group_threads == 32 -> warp-per-pair variant; otherwise CTA-per-pair.  p.ends != null runs the ends-free
+ * variant (decision-byte traceback only: p.ck_off must be null) */
 cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_per_cta, int ctas,
                          size_t smem_bytes, bool ascii_extend, cudaStream_t s);
 /* CTA per pair, four diagonals per thread (packed sequences, shared-memory rings whose diagonal 0 is 16-byte
@@ -144,8 +150,8 @@ size_t bandq_smem_bytes(int A, int win, int seq_words, int stages);
 int bandq_max_ctas_per_sm(int threads, size_t smem_bytes, bool with_bt);
 /* decision bytes of wfa_bandq_kernel -> 2-bit ops, one thread per pair of the launch */
 cudaError_t launch_band_traceback(const KernelParams &p, cudaStream_t s);
-int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii_extend, bool with_bt);
+int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii_extend, bool with_bt, bool ef = false);
 int exact_max_ctas_per_sm(int group_threads, int groups_per_cta, size_t smem_bytes, bool ascii_extend, bool with_bt,
-                          bool ckpt = false);
+                          bool ckpt = false, bool ef = false);
 
 } // namespace wfagpu

@@ -243,6 +243,27 @@ bool wfagpu_align(wfagpu_aligner_t *aligner)
     return wfagpu_last_launch_ok();
 }
 
+bool wfagpu_align_span(wfagpu_aligner_t *aligner, const wfagpu_span_t *span)
+{
+    if (!aligner) { ERR("Invalid aligner."); return false; }
+    if (!aligner->results || !aligner->sequences_metadata) { ERR("Aligner parameters are not initialized."); return false; }
+    if (span && (span->pattern_begin_free < 0 || span->pattern_end_free < 0 || span->text_begin_free < 0 ||
+                 span->text_end_free < 0)) {
+        ERR("Ends-free span values must be >= 0.");
+        return false;
+    }
+    const bool ef = span && (span->pattern_begin_free || span->pattern_end_free || span->text_begin_free ||
+                             span->text_end_free);
+    if (ef && aligner->alignment_options.band > 0) {
+        ERR("Ends-free alignment cannot be combined with the adaptive band.");
+        return false;
+    }
+    wfagpu_launch_alignments_span(aligner->sequences_buffer, aligner->sequences_buffer_len, aligner->sequences_metadata,
+                                  aligner->results, aligner->alignment_options,
+                                  aligner->alignment_options.compute_cigar, false, ef ? span : NULL);
+    return wfagpu_last_launch_ok();
+}
+
 /* Extension: forget the pairs, keep the buffers (streaming: the next window is read into the same pinned memory). */
 void wfagpu_clear_sequences(wfagpu_aligner_t *aligner)
 {

@@ -111,6 +111,8 @@ typedef struct {
     bool failed;
     bool verbose;
     bool host_cigar;        /* WFAGPU_HOST_CIGAR=1: print the CIGAR text on the host instead of the GPU */
+    bool ef;                /* ends-free call: `span` is not all zero */
+    wfagpu_span_t span;
     int decode_threads;
     /* accumulated */
     wfagpu_run_stats_t stats;
@@ -133,6 +135,7 @@ typedef struct {
     size_t pairs_cap;
     wfagpu_pair_out_t *out;
     size_t out_cap;
+    int32_t *ends;          /* ends-free, CIGAR text on the host: {k_begin, k_end} per pair */
 } inflight_t;
 
 static double now_s(void)
@@ -306,7 +309,7 @@ static int submit(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
         src = stage;
     }
     if (wfagpu_device_upload(d, slot, src, bytes, f->pairs, f->n)) return -1;
-    if (wfagpu_device_align(d, slot, f->n, &plan, 0)) return -1;
+    if (wfagpu_device_align_span(d, slot, f->n, &plan, 0, j->ef ? &j->span : NULL)) return -1;
     f->active = true;
     return 0;
 }
@@ -325,15 +328,16 @@ static void check_chunk(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
     wfagpu_plan_t plan;
     fill_plan(j, false, &plan);
     plan.band = 0;                                            /* the exact optimum, also for banded runs */
-    const bool have_ref = ref && wfagpu_device_rescore(d, slot, f->n, &plan, ref) == 0;
+    const bool have_ref = ref && wfagpu_device_rescore_span(d, slot, f->n, &plan, j->ef ? &j->span : NULL, ref) == 0;
     long bad = 0, sum = 0;
     #pragma omp parallel for schedule(dynamic, 64) num_threads(j->decode_threads) reduction(+:bad,sum) if (f->n > 256)
     for (long i = 0; i < (long)f->n; ++i) {
         if (!(f->out[i].status & WFAGPU_ST_FINISHED)) continue;
         bool ok = true;
         if (j->cigar)
-            ok = wfagpu_check_result(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
-                                     m[i].text_len, j->opt.penalties, res[i].error, res[i].cigar.buffer);
+            ok = wfagpu_check_result_span(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
+                                          m[i].text_len, j->opt.penalties, j->ef ? &j->span : NULL, res[i].error,
+                                          res[i].cigar.buffer);
         /* a banded score may legitimately exceed the optimum; an exact one must equal it */
         if (have_ref && ref[i] >= 0 && (j->opt.band > 0 ? (long)res[i].error < ref[i] : (long)res[i].error != ref[i])) {
             fprintf(stderr, "[!] ERROR: Incorrect distance (%zu). GPU=%u, independent GPU check=%d\n", f->from + (size_t)i,
@@ -374,6 +378,11 @@ static int collect(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f, wfagpu
     if (j->cigar && !j->host_cigar) {
         if (wfagpu_device_download_text(d, slot, f->n, &text, &text_bytes, &refs)) return -1;
         wfagpu_device_last_stats(d, slot, &bs);
+    } else if (j->cigar && j->ef) {
+        /* the host decoder needs the diagonal every alignment starts on */
+        free(f->ends);
+        f->ends = (int32_t *)malloc(2 * f->n * sizeof(int32_t));
+        if (!f->ends || wfagpu_device_download_ends(d, slot, f->n, f->ends)) return -1;
     }
     acc->launches += bs.launches;
     acc->d2h_bytes += bs.d2h_bytes;
@@ -397,6 +406,10 @@ static int collect(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f, wfagpu
         if (j->cigar && refs) {
             /* text was printed on the GPU: append it to the caller's buffer */
             if (!wfagpu_cigar_append(&res[i].cigar, text + refs[i].off, refs[i].len)) bad++;
+        } else if (j->cigar && j->ef) {
+            if (!wfagpu_ops_to_cigar_span(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
+                                          m[i].text_len, f->ends[2 * i], ops + o->ops_off, o->n_ops, &res[i].cigar))
+                bad++;
         } else if (j->cigar) {
             if (!wfagpu_ops_to_cigar(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
                                      m[i].text_len, o->distance, ops + o->ops_off, o->n_ops, &res[i].cigar))
@@ -450,7 +463,7 @@ static void *worker_main(void *arg)
         slot = other;
     }
     if (!ok) fail_job(j);
-    for (int s = 0; s < 2; ++s) { free(fl[s].pairs); free(fl[s].out); }
+    for (int s = 0; s < 2; ++s) { free(fl[s].pairs); free(fl[s].out); free(fl[s].ends); }
     wfagpu_device_release(d);
     pthread_mutex_lock(&j->mu);
     j->stats.gpu_align_ms += acc.gpu_align_ms;
@@ -489,7 +502,7 @@ void wfagpu_plan_chunks(size_t n, size_t batch_size, int n_devices, size_t ascii
 }
 
 static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_alignment_result_t *res,
-                    wfa_alignment_options_t opt, bool cigar, bool check)
+                    wfa_alignment_options_t opt, bool cigar, bool check, const wfagpu_span_t *ends_free)
 {
     const double t0 = now_s();
     memset(&t_last_stats, 0, sizeof(t_last_stats));
@@ -502,6 +515,16 @@ static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_align
         fprintf(stderr, "[!] ERROR: penalties must satisfy x >= 1, e >= 1, o >= 0.\n");
         return;
     }
+    const wfagpu_span_t *sp = ends_free;
+    const bool ef = sp && (sp->pattern_begin_free || sp->pattern_end_free || sp->text_begin_free || sp->text_end_free);
+    if (sp && (sp->pattern_begin_free < 0 || sp->pattern_end_free < 0 || sp->text_begin_free < 0 || sp->text_end_free < 0)) {
+        fprintf(stderr, "[!] ERROR: ends-free span values must be >= 0.\n");
+        return;
+    }
+    if (ef && opt.band > 0) {
+        fprintf(stderr, "[!] ERROR: ends-free alignment cannot be combined with the adaptive band (-B).\n");
+        return;
+    }
     int devs[MAX_DEVICES];
     const int ndev = select_devices(devs);
     if (ndev < 1) return;
@@ -510,6 +533,8 @@ static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_align
     memset(&job, 0, sizeof(job));
     job.buf = buf; job.buf_size = buf_size; job.meta = meta; job.res = res; job.opt = opt; job.cigar = cigar;
     job.check = check;
+    job.ef = ef;
+    if (ef) job.span = *sp;
     job.n = opt.num_alignments;
     job.pageable = !wfagpu_host_is_pinned(buf);
     const size_t span = meta[job.n - 1].text_offset + meta[job.n - 1].text_len + 1 - meta[0].pattern_offset;
@@ -602,7 +627,7 @@ void launch_alignments(char *sequences_buffer, const size_t sequences_buffer_siz
                        wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, true,
-            check_correctness);
+            check_correctness, NULL);
 }
 
 void launch_alignments_distance(char *sequences_buffer, const size_t sequences_buffer_size,
@@ -611,5 +636,14 @@ void launch_alignments_distance(char *sequences_buffer, const size_t sequences_b
                                 wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, false,
-            check_correctness);
+            check_correctness, NULL);
+}
+
+void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buffer_size,
+                                   sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                   wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                   const wfagpu_span_t *span)
+{
+    run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
+            check_correctness, span);
 }

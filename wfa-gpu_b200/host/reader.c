@@ -203,6 +203,45 @@ bool wfagpu_check_result(const char *pattern, size_t plen, const char *text, siz
     return v == plen && h == tlen && score == error;
 }
 
+/* The same under an ends-free span: the first and the last run of the CIGAR, when they are I or D runs, are free up
+ * to the span's allowance for that end (wfagpu_b200.h). */
+bool wfagpu_check_result_span(const char *pattern, size_t plen, const char *text, size_t tlen,
+                              affine_penalties_t pen, const wfagpu_span_t *span, unsigned int error, const char *cigar)
+{
+    if (!span) return wfagpu_check_result(pattern, plen, text, tlen, pen, error, cigar);
+    if (span->pattern_begin_free < 0 || span->pattern_end_free < 0 || span->text_begin_free < 0 || span->text_end_free < 0)
+        return false;
+    size_t v = 0, h = 0;
+    unsigned long score = 0;
+    const char *c = cigar;
+    bool first = true;
+    if (!c) return false;
+    while (*c) {
+        unsigned long rep = 0;
+        if (*c < '0' || *c > '9') return false;
+        while (*c >= '0' && *c <= '9') rep = rep * 10 + (unsigned long)(*c++ - '0');
+        const char op = *c++;
+        const bool last = (*c == 0);
+        if (op == 'M' || op == 'X') {
+            if (v + rep > plen || h + rep > tlen) return false;
+            for (unsigned long i = 0; i < rep; ++i)
+                if ((pattern[v + i] == text[h + i]) != (op == 'M')) return false;
+            v += rep; h += rep;
+            if (op == 'X') score += rep * (unsigned long)pen.x;
+        } else if (op == 'I' || op == 'D') {
+            unsigned long free_bases = 0;
+            if (first) free_bases += (unsigned long)(op == 'I' ? span->text_begin_free : span->pattern_begin_free);
+            if (last) free_bases += (unsigned long)(op == 'I' ? span->text_end_free : span->pattern_end_free);
+            if (rep > free_bases) score += (unsigned long)pen.o + (rep - free_bases) * (unsigned long)pen.e;
+            if (op == 'I') h += rep; else v += rep;
+        } else {
+            return false;
+        }
+        if (v > plen || h > tlen) return false;
+        first = false;
+    }
+    return v == plen && h == tlen && score == error;
+}
 
 /* ---------------------------------------------------------------------------------------------
  * The reference library's validators under their own names, argument order (text first) and input format

@@ -11,7 +11,8 @@
 #include <stdlib.h>
 #include "wfagpu_b200.h"
 
-int wfagpu_build_step_table(int x, int o, int e, int max_steps, int max_dist, int banded_win,
+/* `extra`: diagonals added on both sides of every score's range (the start row of an ends-free alignment) */
+static int build_step_table(int x, int o, int e, int max_steps, int max_dist, int banded_win, int extra,
                             wfagpu_step_t *tab, uint64_t *arena_units)
 {
     if (max_dist < 1) max_dist = 1;
@@ -27,10 +28,10 @@ int wfagpu_build_step_table(int x, int o, int e, int max_steps, int max_dist, in
     const uint64_t band_units = banded_win > 0 ? (uint64_t)((banded_win + 8 + 15) / 16) : 0;
     int d;
     has_m[0] = 1;
-    if (tab) { tab[0].row_off = 0; tab[0].n = 0; tab[0].kind = WFAGPU_STEP_M; }
+    if (tab) { tab[0].row_off = 0; tab[0].n = (uint16_t)extra; tab[0].kind = WFAGPU_STEP_M; }
     for (d = 1; d < max_dist; ++d) {
         if (steps >= max_steps - 1) break;          /* while (steps < max_steps - 1) */
-        if (n >= 65535 || mdi >= 65535) break;
+        if (n + extra >= 65535 || mdi >= 65535) break;
         int gap = 0, m = 0;
         if (d - o - e >= 0) gap = has_m[d - o - e] || has_gap[d - e];
         if (gap) m = 1;
@@ -50,11 +51,24 @@ int wfagpu_build_step_table(int x, int o, int e, int max_steps, int max_dist, in
             }
         } else if (m) { kind = WFAGPU_STEP_M; has_m[d] = 1; }
         if (units > 0xffffffffull) break;           /* row offsets are 32-bit */
-        if (tab) { tab[d].row_off = (uint32_t)units; tab[d].n = (uint16_t)n; tab[d].kind = (uint16_t)kind; }
-        if (kind == WFAGPU_STEP_MDI) units += banded_win > 0 ? band_units : (uint64_t)((2 * n + 1 + 15) / 16);
+        if (tab) { tab[d].row_off = (uint32_t)units; tab[d].n = (uint16_t)(n + extra); tab[d].kind = (uint16_t)kind; }
+        if (kind == WFAGPU_STEP_MDI) units += banded_win > 0 ? band_units : (uint64_t)((2 * (n + extra) + 1 + 15) / 16);
     }
     free(has_m);
     free(has_gap);
     if (arena_units) *arena_units = units;
     return d;
+}
+
+int wfagpu_build_step_table(int x, int o, int e, int max_steps, int max_dist, int banded_win,
+                            wfagpu_step_t *tab, uint64_t *arena_units)
+{
+    return build_step_table(x, o, e, max_steps, max_dist, banded_win, 0, tab, arena_units);
+}
+
+int wfagpu_build_step_table_span(int x, int o, int e, int max_steps, int max_dist, int start_half_width,
+                                 wfagpu_step_t *tab, uint64_t *arena_units)
+{
+    if (start_half_width < 0 || start_half_width >= 65535) return -1;
+    return build_step_table(x, o, e, max_steps, max_dist, 0, start_half_width, tab, arena_units);
 }

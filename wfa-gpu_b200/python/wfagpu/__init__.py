@@ -76,6 +76,12 @@ class BatchStats(C.Structure):
                 ("reserved1", C.c_uint32)]
 
 
+class Span(C.Structure):
+    """wfagpu_span_t: ends-free span in WFA2-lib's order (pattern begin / end, text begin / end)."""
+    _fields_ = [("pattern_begin_free", C.c_int), ("pattern_end_free", C.c_int), ("text_begin_free", C.c_int),
+                ("text_end_free", C.c_int)]
+
+
 class DevPair(C.Structure):
     _fields_ = [("p_ascii", C.c_uint32), ("t_ascii", C.c_uint32), ("p_word", C.c_uint32), ("t_word", C.c_uint32),
                 ("plen", C.c_uint32), ("tlen", C.c_uint32), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
@@ -96,7 +102,9 @@ EXPORTS = [
     "check_cigar_edit", "check_affine_distance", "wfagpu_cigar_append", "wfagpu_device_download_text",
     "recover_cigar", "wfagpu_unroll_cigar", "wfagpu_device_release", "wfagpu_device_rescore", "wfagpu_device_staging",
     "wfagpu_host_is_pinned", "wfagpu_host_alloc", "wfagpu_host_free", "wfagpu_reserve", "wfagpu_parse_devices",
-    "wfagpu_set_host_threads",
+    "wfagpu_set_host_threads", "wfagpu_align_span", "wfagpu_launch_alignments_span", "wfagpu_device_align_span",
+    "wfagpu_device_download_ends", "wfagpu_device_rescore_span", "wfagpu_ops_to_cigar_span",
+    "wfagpu_check_result_span", "wfagpu_build_step_table_span",
 ]
 
 _lib = None
@@ -185,8 +193,33 @@ def load():
     L.wfagpu_host_unregister.argtypes = [C.c_void_p]
     L.wfagpu_pairs_from_metadata.argtypes = [P(SequencePair), C.c_size_t, C.c_size_t, C.c_size_t, P(DevPair),
                                              P(C.c_size_t), P(C.c_size_t)]
+    L.wfagpu_align_span.argtypes = [P(AlignerStruct), P(Span)]
+    L.wfagpu_align_span.restype = C.c_bool
+    L.wfagpu_launch_alignments_span.argtypes = [C.c_void_p, C.c_size_t, P(SequencePair), P(AlignmentResult),
+                                                AlignmentOptions, C.c_bool, C.c_bool, P(Span)]
+    L.wfagpu_launch_alignments_span.restype = None
+    L.wfagpu_device_align_span.argtypes = [C.c_void_p, C.c_int, C.c_size_t, P(Plan), C.c_int, P(Span)]
+    L.wfagpu_device_download_ends.argtypes = [C.c_void_p, C.c_int, C.c_size_t, P(C.c_int32)]
+    L.wfagpu_device_rescore_span.argtypes = [C.c_void_p, C.c_int, C.c_size_t, P(Plan), P(Span), P(C.c_int32)]
+    L.wfagpu_ops_to_cigar_span.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_size_t, C.c_int,
+                                           P(C.c_uint32), C.c_uint32, P(Cigar)]
+    L.wfagpu_ops_to_cigar_span.restype = C.c_bool
+    L.wfagpu_check_result_span.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_size_t, AffinePenalties, P(Span),
+                                           C.c_uint, C.c_char_p]
+    L.wfagpu_check_result_span.restype = C.c_bool
+    L.wfagpu_build_step_table_span.argtypes = [C.c_int] * 6 + [P(Step), P(C.c_uint64)]
     _lib = L
     return L
+
+
+def span_of(ends_free):
+    """A 4-tuple (pattern_begin_free, pattern_end_free, text_begin_free, text_end_free) -> Span (None -> None)."""
+    if ends_free is None:
+        return None
+    vals = tuple(int(v) for v in ends_free)
+    if len(vals) != 4:
+        raise ValueError("ends_free takes four values: pattern_begin_free, pattern_end_free, text_begin_free, text_end_free")
+    return Span(*vals)
 
 
 def _b(s):
@@ -217,9 +250,16 @@ class Aligner:
     def options(self):
         return self.s.alignment_options
 
-    def align(self):
-        if not self.L.wfagpu_align(C.byref(self.s)):
-            raise RuntimeError("wfagpu_align failed (see stderr); there is no CPU fallback")
+    def align(self, ends_free=None):
+        """ends_free: None (global) or (pattern_begin_free, pattern_end_free, text_begin_free, text_end_free),
+        WFA2-lib's order: that many leading / trailing bases of either sequence are free (wfagpu_align_span)."""
+        sp = span_of(ends_free)
+        if sp is None:
+            if not self.L.wfagpu_align(C.byref(self.s)):
+                raise RuntimeError("wfagpu_align failed (see stderr); there is no CPU fallback")
+            return True
+        if not self.L.wfagpu_align_span(C.byref(self.s), C.byref(sp)):
+            raise RuntimeError("wfagpu_align_span failed (see stderr); there is no CPU fallback")
         return True
 
     def destroy(self):

@@ -53,6 +53,22 @@ int wfagpu_build_step_table(int x, int o, int e, int max_steps, int max_dist, in
 int wfagpu_build_step_table_span(int x, int o, int e, int max_steps, int max_dist, int start_half_width,
                                  wfagpu_step_t *tab, uint64_t *arena_units);
 
+/* Gap-affine 2-piece penalties (exact kernels, global alignment only): a second gap component (o2, e2).  A score is
+ * an M/I/D step when a gap of either piece exists (gap_i[d] = M[d - o_i - e_i] || gap_i[d - e_i]), and its half width
+ * is min(#M/I/D steps, max((d - o1) / e1, (d - o2) / e2)).  With o2 = o1, e2 = e1 the table equals
+ * wfagpu_build_step_table(x, o1, e1, ...).  -1 for x < 1, e1 < 1, e2 < 1 or a negative opening. */
+int wfagpu_build_step_table_affine2p(int x, int o1, int e1, int o2, int e2, int max_steps, int max_dist,
+                                     wfagpu_step_t *tab, uint64_t *arena_units);
+
+/* --------------------------------------------------- gap-affine 2-piece --- */
+/* WFA2-lib's `affine2p` model: a gap of L bases costs min(o1 + e1 L, o2 + e2 L), a mismatch x.  Valid: x >= 1,
+ * e1, e2 >= 1, o1, o2 >= 0, the pieces in either order.  Scores do not depend on the order; on equal offsets the
+ * traceback prefers piece 1 (M: D1 > D2 > X > I1 > I2; I / D: extend beats open).  Identical pieces give the
+ * single-piece scores and CIGAR text byte for byte.  Global alignment only: no band, no ends-free span. */
+typedef struct {
+    int x, o1, e1, o2, e2;
+} wfagpu_affine2p_t;
+
 /* ---------------------------------------------------------- ends-free --- */
 /* Ends-free (semi-global) span of a call, WFA2-lib's `ends-free` order.  All zero = global alignment.  Per pair each
  * value is clamped to the sequence it applies to.  The score is the gap-affine cost of the aligned part: leading and
@@ -106,6 +122,7 @@ typedef struct {
     int with_cigar;
     int threads_hint;
     int workers_hint;
+    int o2, e2;      /* gap-affine 2-piece: second gap piece; e2 == 0 = one piece (o, e) */
 } wfagpu_plan_t;
 
 /* Statistics of the last batch (kernel times from CUDA events on the launch
@@ -162,6 +179,10 @@ int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, const wfagp
  * alignment's first and last cell: it starts at (max(0, -k_begin), max(0, k_begin)) and ends at offset
  * min(tlen, plen + k_end).  Pairs that did not finish hold no record.  -1 for a global batch. */
 int wfagpu_device_download_ends(wfagpu_device_t *d, int slot, size_t n, int32_t *ends);
+/* A plan with e2 > 0 (gap-affine 2-piece, through wfagpu_device_align / _align_span / _rescore) runs the
+ * one-diagonal-per-thread kernels with decision-byte traceback, no score-bound kernel (pruning uses the launch bound)
+ * and neither reads nor updates the provisioning hint.  Those calls return -3 for a 2-piece plan with band > 0, a
+ * non-zero span, or a negative value. */
 /* Waits for the slot's stream; event-timed durations (milliseconds) of the pack kernel and of the
  * first pass of the alignment: score bounds + wavefronts + traceback + CIGAR text. */
 int wfagpu_device_wait(wfagpu_device_t *d, int slot, float *ms_pack, float *ms_align);
@@ -295,6 +316,22 @@ bool wfagpu_check_result(const char *pattern, size_t plen, const char *text, siz
  * trailing D run (pattern_end_free).  A run that is both leading and trailing may use both allowances. */
 bool wfagpu_check_result_span(const char *pattern, size_t plen, const char *text, size_t tlen,
                               affine_penalties_t pen, const wfagpu_span_t *span, unsigned int error, const char *cigar);
+
+/* The same under gap-affine 2-piece penalties: every gap run of length L costs min(o1 + e1 L, o2 + e2 L). */
+bool wfagpu_check_result_affine2p(const char *pattern, size_t plen, const char *text, size_t tlen,
+                                  const wfagpu_affine2p_t *pen, unsigned int error, const char *cigar);
+
+/* wfagpu_align under gap-affine 2-piece penalties: the five values replace the aligner's penalties for this call
+ * (honours compute_cigar).  False, with a message and the results untouched, for an invalid set (see
+ * wfagpu_affine2p_t), band > 0.  NULL: exactly wfagpu_align. */
+bool wfagpu_align_affine2p(wfagpu_aligner_t *aligner, const wfagpu_affine2p_t *pen);
+/* launch_alignments / launch_alignments_distance (cigar = false) under 2-piece penalties (options.penalties is not
+ * used); check_correctness validates every CIGAR under them and re-computes every score.  NULL: the single-piece
+ * function. */
+void wfagpu_launch_alignments_affine2p(char *sequences_buffer, size_t sequences_buffer_size,
+                                       sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                       wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                       const wfagpu_affine2p_t *pen);
 
 /* wfagpu_align with an ends-free span (honours compute_cigar).  False, with a message, for negative values, or for
  * band > 0 together with a non-zero span.  NULL or all zero: exactly wfagpu_align. */

@@ -10,13 +10,17 @@
  *   -g/--affine-penalties x,o,e      default 2,3,1 (signs are stripped)
  *   -x/--compute-cigar               CIGAR (otherwise score only)
  *   -e/--max-distance E              wavefront budget of the first GPU pass
- *                                    (default 0.1 * maxlen(pair 0) * max(x,o,e), at least 20)
+ *                                    (default 0.1 * maxlen(pair 0) * max(x,o,e), at least 20; with -G the maximum
+ *                                    of the five values)
  *   -t/--threads-per-block T         hint; the band width when -B is given
  *   -b/--batch-size B, -w/--workers W
  *   -B/--band L                      adaptive band, re-centred every L scores; "auto"/0 = 25
  *   -c/--check                       validate every result: CIGAR on the host, score against an independent GPU pass
  *   -F/--ends-free P0,Pf,T0,Tf       ends-free alignment (WFA2-lib's order): that many leading / trailing pattern and
  *                                    text bases are free; not with -B
+ *   -G/--affine2p-penalties x,o1,e1,o2,e2
+ *                                    gap-affine 2-piece penalties (WFA2-lib's affine2p): a gap of L bases costs
+ *                                    min(o1 + e1 L, o2 + e2 L); signs are stripped, e1, e2 >= 1; not with -g, -B or -F
  *   -o/--output-file FILE, -p/--print-output, -O/--output-verbose
  * Output lines: "-score\tCIGAR" (or "-score\tCIGAR\tpattern\ttext" with -O).
  * Pairs whose score exceeds -e are NOT sent to a CPU: they are re-dispatched on the GPU.
@@ -33,7 +37,7 @@
 #include "wfagpu_b200.h"
 
 typedef struct {
-    const char *seq, *fq, *ft, *out, *pen, *devices, *ends_free;
+    const char *seq, *fq, *ft, *out, *pen, *devices, *ends_free, *pen2;
     long n, e, t, b, w, band, stream;
     int have_e, have_t, have_b, have_w, have_band, have_stream, cigar, check, print, verbose;
 } args_t;
@@ -57,6 +61,7 @@ static void usage(void)
             "\t-B, --band L                    banded heuristic, re-centre every L scores (auto = 25)\n"
             "\t-c, --check                     check the alignments\n"
             "\t-F, --ends-free P0,Pf,T0,Tf     ends-free: free leading/trailing pattern (P) and text (T) bases\n"
+            "\t-G, --affine2p-penalties x,o1,e1,o2,e2  gap-affine 2-piece: a gap of L costs min(o1+e1*L, o2+e2*L)\n"
             "[System]\n"
             "\t-t, --threads-per-block T       threads per alignment (band width with -B)\n"
             "\t-w, --workers W                 GPU workers (hint)\n"
@@ -73,7 +78,7 @@ static const struct { char s; const char *l; int has_val; } OPTS[] = {
     {'g', "affine-penalties", 1}, {'x', "compute-cigar", 0}, {'c', "check", 0}, {'e', "max-distance", 1},
     {'t', "threads-per-block", 1}, {'b', "batch-size", 1}, {'w', "workers", 1}, {'B', "band", 1},
     {'o', "output-file", 1}, {'p', "print-output", 0}, {'O', "output-verbose", 0}, {'D', "devices", 1},
-    {'S', "stream", 1}, {'F', "ends-free", 1},
+    {'S', "stream", 1}, {'F', "ends-free", 1}, {'G', "affine2p-penalties", 1},
 };
 
 static int parse(int argc, char **argv, args_t *a)
@@ -101,6 +106,7 @@ static int parse(int argc, char **argv, args_t *a)
         case 'g': a->pen = val; break;
         case 'D': a->devices = val; break;
         case 'F': a->ends_free = val; break;
+        case 'G': a->pen2 = val; break;
         case 'S': a->stream = atol(val); a->have_stream = 1; break;
         case 'n': a->n = atoll(val); break;
         case 'e': a->e = atoll(val); a->have_e = 1; break;
@@ -156,6 +162,26 @@ int main(int argc, char **argv)
     if (!parse(argc, argv, &a)) { usage(); return 1; }
     if (!a.seq && !(a.fq && a.ft)) { fprintf(stderr, "[!] ERROR: No input file provided.\n"); return 1; }
 
+    /* -G: gap-affine 2-piece penalties instead of -g */
+    wfagpu_affine2p_t pen2 = {0, 0, 0, 0, 0};
+    if (a.pen2) {
+        if (a.pen) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --affine-penalties (-g).\n"); return 1; }
+        if (a.have_band) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with the band (-B).\n"); return 1; }
+        if (a.ends_free) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --ends-free (-F).\n"); return 1; }
+        if (sscanf(a.pen2, "%d,%d,%d,%d,%d", &pen2.x, &pen2.o1, &pen2.e1, &pen2.o2, &pen2.e2) != 5) {
+            fprintf(stderr, "[!] ERROR: --affine2p-penalties takes five values: x,o1,e1,o2,e2 (got %s).\n", a.pen2);
+            return 1;
+        }
+        if (pen2.x < 0) pen2.x = -pen2.x;
+        if (pen2.o1 < 0) pen2.o1 = -pen2.o1;
+        if (pen2.e1 < 0) pen2.e1 = -pen2.e1;
+        if (pen2.o2 < 0) pen2.o2 = -pen2.o2;
+        if (pen2.e2 < 0) pen2.e2 = -pen2.e2;
+        if (pen2.x < 1 || pen2.e1 < 1 || pen2.e2 < 1) {
+            fprintf(stderr, "[!] ERROR: --affine2p-penalties needs x, e1, e2 >= 1 (got %s).\n", a.pen2);
+            return 1;
+        }
+    }
     int x = 2, o = 3, e = 1;
     if (a.pen && sscanf(a.pen, "%d,%d,%d", &x, &o, &e) != 3) {
         fprintf(stderr, "WARNING: Invalid penalties format provided. Using default penalties (0,2,3,1).\n");
@@ -164,7 +190,13 @@ int main(int argc, char **argv)
     if (x < 0) x = -x;
     if (o < 0) o = -o;
     if (e < 0) e = -e;
-    fprintf(stderr, "INFO: Penalties: M=0, X=%d, O=%d, E=%d.\n", x, o, e);
+    if (a.pen2) {
+        x = pen2.x; o = pen2.o1; e = pen2.e1;
+        fprintf(stderr, "INFO: Gap-affine 2-piece penalties: M=0, X=%d, O1=%d, E1=%d, O2=%d, E2=%d.\n", pen2.x, pen2.o1, pen2.e1,
+                pen2.o2, pen2.e2);
+    } else {
+        fprintf(stderr, "INFO: Penalties: M=0, X=%d, O=%d, E=%d.\n", x, o, e);
+    }
     if (a.devices) wfagpu_set_devices(a.devices);
 
     wfagpu_reader_t *reader = a.seq ? wfagpu_reader_open_seq(a.seq) : wfagpu_reader_open_fasta(a.fq, a.ft);
@@ -200,6 +232,8 @@ int main(int argc, char **argv)
         max_distance = (int)((m0->text_len > m0->pattern_len ? m0->text_len : m0->pattern_len) * 0.1);
         int pm = x > o ? x : o;
         if (e > pm) pm = e;
+        if (a.pen2 && pen2.o2 > pm) pm = pen2.o2;
+        if (a.pen2 && pen2.e2 > pm) pm = pen2.e2;
         max_distance *= pm;
         if (max_distance <= 20) max_distance = 20;
         fprintf(stderr, "INFO: No maximum error provided by the user, using %d\n", max_distance);
@@ -269,7 +303,10 @@ int main(int argc, char **argv)
         opt.compute_cigar = a.cigar;
 
         t0 = now_s();
-        if (a.ends_free)
+        if (a.pen2)
+            wfagpu_launch_alignments_affine2p(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results,
+                                              opt, a.cigar, a.check, &pen2);
+        else if (a.ends_free)
             wfagpu_launch_alignments_span(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt,
                                           a.cigar, a.check, &span);
         else if (a.cigar) launch_alignments(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt, a.check);

@@ -117,6 +117,7 @@ struct LaunchCfg {
     int seq_words;
     size_t smem;
     int A, E1, G;
+    int E2;               /* gap-affine 2-piece: depth of the I2 / D2 rings (0: one piece) */
     bool global_ring;     /* large tier: rings in global memory, int32 offsets */
     bool ckpt;            /* checkpointed traceback (ring snapshots) instead of decision bytes */
     bool quad;            /* wfa_quad_kernel: four diagonals per thread, packed int16 SIMD */
@@ -168,7 +169,7 @@ struct Slot {
     PinBuf<uint32_t> h_counters;
     PinBuf<unsigned long long> h_cells;
     PinBuf<wfagpu_step_t> h_steps;
-    int tab_key[6] = {-1, -1, -1, -1, -1, -1};
+    int tab_key[8] = {-1, -1, -1, -1, -1, -1, -1, -1};
     int tab_d_end = 0;
     uint64_t tab_arena_units = 0;
     size_t n = 0;
@@ -446,13 +447,16 @@ extern "C" int wfagpu_device_upload(wfagpu_device_t *d, int slot, const char *as
  * 2 x 512 95 k, 3 x 384 109 k -- more, smaller CTAs hide the per-score barrier.
  * `n_want` is the half width the launch should be able to hold. */
 static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_min, uint32_t max_len, size_t n_items,
-                      bool ascii, bool bt, bool ef, LaunchCfg *c)
+                      bool ascii, bool bt, bool ef, int o2, int e2, LaunchCfg *c)
 {
-    const int A = std::max(o + e, x) + 1, E1 = e + 1, G = A;
+    /* 2-piece (e2 > 0): one diagonal per thread, decision bytes, no schedule records; two more rings of e2 + 1 rows */
+    const bool p2 = e2 > 0;
+    const int A = std::max(std::max(o + e, x), p2 ? o2 + e2 : 0) + 1, E1 = e + 1, G = A, E2 = p2 ? e2 + 1 : 0;
+    const bool sched = !p2;
     const size_t smem_max = d->prop.sharedMemPerBlockOptin;        /* 227 KB on B200 */
     const size_t smem_sm = d->prop.sharedMemPerMultiprocessor;     /* 228 KB */
     const int seq_words = (int)packed_words_for(max_len);
-    c->A = A; c->E1 = E1; c->G = G; c->seq_words = seq_words;
+    c->A = A; c->E1 = E1; c->G = G; c->E2 = E2; c->seq_words = seq_words;
     n_want = std::max(1, n_want);
     /* ring row geometry.  Checkpointed traceback copies rows in 16-byte units: diagonal 0 sits on
      * an 8-element boundary and a row has 8 spare cells on both sides. */
@@ -468,7 +472,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
     bool large = d->force_large || max_len >= (1u << 15);
     if (!large) {
         /* rings that do not fit one CTA's shared memory even single-buffered go to the large tier */
-        if (exact_smem_bytes(A, E1, rs(n_want), seq_words, 1, 1, true) > smem_max) large = true;
+        if (exact_smem_bytes(A, E1, rs(n_want), seq_words, 1, 1, sched, E2) > smem_max) large = true;
     }
     if (large) {
         c->global_ring = true;
@@ -476,7 +480,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
         c->stages = 1;
         c->n_cap = n_want;
         /* packed pairs: four diagonals per thread with 128-bit loads (wfa_quadg_kernel): rows 16-byte aligned */
-        c->quad = !ascii && !d->no_quad && !ef;       /* ends-free: one diagonal per thread */
+        c->quad = !ascii && !d->no_quad && !ef && !p2;       /* ends-free, 2-piece: one diagonal per thread */
         ck = c->quad;
         c->row_stride = rs(n_want);
         c->center = c->quad ? ctr(n_want) : n_want + 2 * G + 1;
@@ -497,7 +501,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
             /* wide wavefronts (50 kbp / 15 %: ~10 k diagonals per score) keep 1024 threads busy: 581 vs 416
              * pairs/s against 512 threads on B200 */
             c->group_threads = d->force_threads ? d->force_threads : (n_want >= 2048 ? 1024 : 512);
-            occ = large_max_ctas_per_sm(c->group_threads, c->smem, ascii, bt, ef);
+            occ = large_max_ctas_per_sm(c->group_threads, c->smem, ascii, bt, ef, p2);
             if (occ < 1) return -1;
             occ = std::min(occ, d->force_ctas_per_sm ? d->force_ctas_per_sm : 2);
         }
@@ -514,20 +518,20 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
         c->n_cap = n_want;
         c->row_stride = rs(c->n_cap);
         c->center = c->n_cap + 2 * G + 1;
-        c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages);
+        c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages, false, E2);
         while (c->smem > smem_max && c->groups_per_cta > 1) {
             c->groups_per_cta >>= 1;
-            c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages);
+            c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages, false, E2);
         }
         if (c->smem > smem_max) warp = false;
     }
     if (!warp) {
         c->groups_per_cta = 1;
-        c->ckpt = bt && !d->no_ckpt && !ef;            /* ends-free: decision bytes */
+        c->ckpt = bt && !d->no_ckpt && !ef && !p2;     /* ends-free, 2-piece: decision bytes */
         /* packed pairs on shared-memory rings run four diagonals per thread (with backtrace: snapshots only) */
         /* (measured on B200: 1 kbp / 10 %, ring half width 196: 9.5 ms per 50 k pairs with one diagonal per thread and 16 CTAs per
          * SM against 11.0 ms; from a half width of ~300 on the four-diagonal kernel wins) */
-        c->quad = !ascii && !d->no_quad && !ef && (!bt || c->ckpt) && n_want >= d->quad_min;
+        c->quad = !ascii && !d->no_quad && !ef && !p2 && (!bt || c->ckpt) && n_want >= d->quad_min;
         /* two scores per barrier: score d + 1 must not read the extended M of score d (x >= 2, o + e >= 2) and takes
          * its extend sources from registers (e == 1); costs one more row per ring */
         c->quad_pairs = c->quad && !d->no_quad_pairs && x >= 2 && o + e >= 2 && e == 1;
@@ -549,7 +553,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
          * the arithmetic allowed cost rank 3 of an 8-GPU run its fifth CTA per SM, 33.4 instead of 29.2 ms per step) */
         auto fits = [&](int k, size_t bytes, size_t budget) {
             if (bytes > budget) return false;
-            const int occ_k = c->quad ? quad_max_ctas_per_sm(64, bytes, bt) : exact_max_ctas_per_sm(64, 1, bytes, ascii, bt, c->ckpt, ef);
+            const int occ_k = c->quad ? quad_max_ctas_per_sm(64, bytes, bt) : exact_max_ctas_per_sm(64, 1, bytes, ascii, bt, c->ckpt, ef, p2);
             return occ_k >= k;
         };
         for (int k = kmax; k >= 1 && !best_k; --k) {
@@ -557,26 +561,26 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
             const size_t budget = std::min(smem_max, smem_sm / k - 1024);
             for (int st = 2; st >= 1; --st) {
                 if (d->force_stages && st != d->force_stages) continue;
-                if (!fits(k, exact_smem_bytes(RA, RE, rs(n_min), seq_words, 1, st, true), budget)) continue;
+                if (!fits(k, exact_smem_bytes(RA, RE, rs(n_min), seq_words, 1, st, sched, E2), budget)) continue;
                 int lo = n_min, hi = n_want;             /* widest rings that still fit k CTAs */
                 while (lo < hi) {
                     const int mid = (lo + hi + 1) / 2;
-                    if (fits(k, exact_smem_bytes(RA, RE, rs(mid), seq_words, 1, st, true), budget)) lo = mid; else hi = mid - 1;
+                    if (fits(k, exact_smem_bytes(RA, RE, rs(mid), seq_words, 1, st, sched, E2), budget)) lo = mid; else hi = mid - 1;
                 }
                 best_k = k; stages = st; n_cap = lo;
-                smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, st, true);
+                smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, st, sched, E2);
                 break;
             }
         }
         if (!best_k) {
             /* does not fit even alone: hold as many diagonals as one CTA can */
             stages = 1;
-            const size_t fixed = exact_smem_bytes(RA, RE, 0, seq_words, 1, stages, true);
-            const int rows_q = RA + 2 * RE;
+            const size_t fixed = exact_smem_bytes(RA, RE, 0, seq_words, 1, stages, sched, E2);
+            const int rows_q = RA + 2 * RE + 2 * E2;
             if (fixed + (size_t)rows_q * rs(1) * 2 > smem_max) return -2;   /* the sequences alone do not fit */
             n_cap = (int)((smem_max - fixed - 64) / ((size_t)rows_q * 4)) - 2 * G - (ck ? 16 : 2);
             if (n_cap < 1) return -2;
-            smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, stages, true);
+            smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, stages, sched, E2);
             best_k = 1;
         }
         c->stages = stages;
@@ -602,7 +606,7 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
     }
     const int threads = warp ? 32 * c->groups_per_cta : c->group_threads;
     int occ = c->quad ? quad_max_ctas_per_sm(c->group_threads, c->smem, bt)
-                      : exact_max_ctas_per_sm(c->group_threads, c->groups_per_cta, c->smem, ascii, bt, c->ckpt, ef);
+                      : exact_max_ctas_per_sm(c->group_threads, c->groups_per_cta, c->smem, ascii, bt, c->ckpt, ef, p2);
     if (occ < 1) {
         fprintf(stderr, "[wfagpu] kernel configuration does not fit (threads=%d smem=%zu)\n", threads, c->smem);
         return -1;
@@ -684,23 +688,27 @@ static int ensure_ck_table(Slot &s, const wfagpu_plan_t &plan, int period)
 /* Step table for a budget of `max_steps` wavefront steps (cached per slot; host copy in s.h_steps). */
 static int ensure_step_table(Slot &s, const wfagpu_plan_t &plan, int max_steps)
 {
-    const int max_dist = std::min<long long>((long long)max_steps * (std::max(plan.x, plan.o + plan.e) + 1) + 16, 1 << 30);
+    const bool p2 = plan.e2 > 0;
+    const int widest = std::max(std::max(plan.x, plan.o + plan.e), p2 ? plan.o2 + plan.e2 : 0);
+    const int max_dist = std::min<long long>((long long)max_steps * (widest + 1) + 16, 1 << 30);
     const int tab_win = plan.band > 0 ? (plan.band_width > 0 ? plan.band_width : 512) : 0;
     const int extra = s.ef ? s.ef_w : 0;   /* ends-free: the start row widens every score's range */
+    const int o2 = p2 ? plan.o2 : 0, e2 = p2 ? plan.e2 : 0;
     if (s.tab_key[0] == plan.x && s.tab_key[1] == plan.o && s.tab_key[2] == plan.e && s.tab_key[3] == max_steps &&
-        s.tab_key[4] == tab_win && s.tab_key[5] == extra)
+        s.tab_key[4] == tab_win && s.tab_key[5] == extra && s.tab_key[6] == o2 && s.tab_key[7] == e2)
         return 0;
     if (s.h_steps.ensure((size_t)max_dist + 1)) return -1;
     if (tables_idle(s)) return -1;        /* a previous pass may still be reading the pinned table */
     uint64_t units = 0;
-    const int de = extra ? wfagpu_build_step_table_span(plan.x, plan.o, plan.e, max_steps, max_dist, extra, s.h_steps.p, &units)
+    const int de = p2 ? wfagpu_build_step_table_affine2p(plan.x, plan.o, plan.e, o2, e2, max_steps, max_dist, s.h_steps.p, &units)
+                 : extra ? wfagpu_build_step_table_span(plan.x, plan.o, plan.e, max_steps, max_dist, extra, s.h_steps.p, &units)
                          : wfagpu_build_step_table(plan.x, plan.o, plan.e, max_steps, max_dist, tab_win, s.h_steps.p, &units);
     if (de < 1) return -1;
     if (s.steps.ensure((size_t)de + 1)) return -1;
     CK(cudaMemcpyAsync(s.steps.p, s.h_steps.p, (size_t)de * sizeof(wfagpu_step_t), cudaMemcpyHostToDevice, s.stream));
     if (tables_sent(s)) return -1;
     s.tab_key[0] = plan.x; s.tab_key[1] = plan.o; s.tab_key[2] = plan.e; s.tab_key[3] = max_steps; s.tab_key[4] = tab_win;
-    s.tab_key[5] = extra;
+    s.tab_key[5] = extra; s.tab_key[6] = o2; s.tab_key[7] = e2;
     s.tab_d_end = de;
     s.tab_arena_units = units;
     s.ck_key[0] = -1;     /* snapshot offsets follow the table */
@@ -713,6 +721,7 @@ static int ensure_step_table(Slot &s, const wfagpu_plan_t &plan, int max_steps)
 static int run_bound_only(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int max_steps, const uint32_t *order_dev,
                           size_t n_items)
 {
+    if (plan.e2 > 0) return -2;           /* the bound kernel and its step table are single-piece */
     if (ensure_step_table(s, plan, max_steps)) return -1;
     if (s.bound.ensure(s.n + 1)) return -1;
     KernelParams kp{};
@@ -748,7 +757,9 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
 {
     HostTrace tr;
     if (first_pass) pull_hint(d);            /* what the last batch on this GPU needed (any context) */
-    if (first_pass && s.ef) { d->hint_dist = 0; d->hint_mean = 0; }     /* ends-free: hints of global batches do not apply */
+    const bool p2 = plan.e2 > 0;
+    /* ends-free, 2-piece: hints of (single-piece) global batches do not apply */
+    if (first_pass && (s.ef || p2)) { d->hint_dist = 0; d->hint_mean = 0; }
     if (ensure_step_table(s, plan, max_steps)) return -1;
     const wfagpu_step_t *tab = s.h_steps.p;
     const int d_full = s.tab_d_end;
@@ -769,7 +780,8 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
      * gap for the length difference: a generous -e (or a stale hint) does not widen the rings */
     int d_reach = d_full;                    /* scores beyond this cannot occur in this batch */
     if (plan.band <= 0) {
-        const long long cap = (long long)plan.x * s.minlen_max + plan.o + (long long)plan.e * s.kt_max + 2;
+        long long cap = (long long)plan.x * s.minlen_max + plan.o + (long long)plan.e * s.kt_max + 2;
+        if (p2) cap = std::min(cap, (long long)plan.x * s.minlen_max + plan.o2 + (long long)plan.e2 * s.kt_max + 2);   /* the cheaper piece */
         if (cap < d_reach) d_reach = (int)std::max<long long>(cap, 2);
         if (d_reach < d_want) d_want = d_reach;
     }
@@ -779,7 +791,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
      * host round trip per pass (bounds back: 4 bytes per pair). */
     int d_p99 = 0;                           /* 99 % of the bounded pairs finish below this score (0 = unknown) */
     size_t n_seed = 0;                       /* pairs at the end of the order list that skip this pass (no bound within the budget) */
-    if (first_pass && !have_bounds && plan.band <= 0 && !ascii && !d->no_bound && !d->no_prebound && n_items == s.n &&
+    if (first_pass && !have_bounds && plan.band <= 0 && !ascii && !p2 && !d->no_bound && !d->no_prebound && n_items == s.n &&
         bound_max_ctas_per_sm(std::max(plan.o + plan.e, plan.x) + 1, plan.e + 1, 8) >= 1) {   /* penalties whose rings fit the bound kernel */
         bool pays = d->force_bound;
         if (!pays) {
@@ -859,7 +871,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
             }
         }
     }
-    const int pen_e = plan.e;
+    const int pen_e = p2 ? std::min(plan.e, plan.e2) : plan.e;     /* 2-piece: the pruning's min(e1, e2) */
     const long long kt_max = s.kt_max;
     auto n_need = [&](int d_end) -> int {
         /* n_d grows, kt + (Dmax - d) / e shrinks: the largest min sits where they cross.  A global pair with |kt| > Dmax / e
@@ -922,7 +934,8 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         if (occ < 1) return -1;
         c.ctas = (int)std::max<size_t>(1, std::min<size_t>((size_t)occ * d->prop.multiProcessorCount, n_items));
     } else {
-        rc = choose_cfg(d, plan.x, plan.o, plan.e, n_want, n_min, s.max_len, n_items, ascii, plan.with_cigar != 0, s.ef, &c);
+        rc = choose_cfg(d, plan.x, plan.o, plan.e, n_want, n_min, s.max_len, n_items, ascii, plan.with_cigar != 0, s.ef,
+                        p2 ? plan.o2 : 0, p2 ? plan.e2 : 0, &c);
     }
     if (rc) return rc;
     tr.mark("cfg");
@@ -1003,7 +1016,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         s.budget_cache = arena_budget;
     }
     const size_t groups = (size_t)c.ctas * c.groups_per_cta;
-    const uint64_t gring_elems = c.global_ring ? (uint64_t)(c.A + 2 * c.E1) * (uint64_t)c.row_stride : 0;
+    const uint64_t gring_elems = c.global_ring ? (uint64_t)(c.A + 2 * c.E1 + 2 * c.E2) * (uint64_t)c.row_stride : 0;
     if (s.gring.ensure(groups * gring_elems + 1)) return -1;
     const uint32_t scratch_words = plan.with_cigar ? (uint32_t)((2 * (size_t)d_end + 31) / 16 + 2) : 1;
     const size_t arenas = (c.ckpt || band_tb) ? items_per_launch : groups;
@@ -1044,7 +1057,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
     /* per-pair bounds: first pass of the packed exact path only (a re-dispatched pair never
      * depends on them) */
     /* have_bounds: s.bound already holds this pass's bounds (run_bound_only) */
-    bool use_bound = !banded && !ascii && (first_pass || have_bounds) && !d->no_bound;
+    bool use_bound = !banded && !ascii && !p2 && (first_pass || have_bounds) && !d->no_bound;
     if (use_bound && !d->force_bound && !have_bounds) {
         /* Worth it?  With D = d_end - 1 and a typical score m, the launch bound leaves
          * cells(D/m) * m^2 cells per pair (cells(r) = r^2/4 + (1.5r - 1)(1 - r/2), 1 from r = 2 on), the
@@ -1096,6 +1109,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         kp.ef_tb = s.span.text_begin_free; kp.ef_te = s.span.text_end_free;
         kp.ends = s.ends.p;
     }
+    if (p2) { kp.o2 = plan.o2; kp.e2 = plan.e2; kp.E2 = c.E2; }
     if (env_int("WFAGPU_VERBOSE", 0))
         fprintf(stderr, "[wfagpu] pass: items=%zu max_steps=%d n_cap=%d d_end=%d group=%d x%d ctas=%d stages=%d smem=%zu ascii=%d band=%d tier=%s period=%d arena=%.1f MB\n",
                 n_items, max_steps, c.n_cap, d_end, c.group_threads, c.groups_per_cta, c.ctas, c.stages, c.smem,
@@ -1230,6 +1244,16 @@ extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, 
         fprintf(stderr, "[wfagpu] ends-free alignment is exact only: it cannot be combined with the adaptive band\n");
         return -3;
     }
+    if (plan->o2 < 0 || plan->e2 < 0) {
+        fprintf(stderr, "[wfagpu] gap-affine 2-piece penalties must be >= 0 (got o2=%d e2=%d)\n", plan->o2, plan->e2);
+        return -3;
+    }
+    const bool p2 = plan->e2 > 0;
+    if (p2 && (plan->band > 0 || ef)) {
+        fprintf(stderr, "[wfagpu] gap-affine 2-piece alignment is global and exact only: it cannot be combined with %s\n",
+                ef ? "an ends-free span" : "the adaptive band");
+        return -3;
+    }
     if (plan->x < 1 || plan->e < 1 || plan->o < 0) {
         /* x = 0 or e = 0 make a wavefront its own source (and divide by zero in the pruning quotient) */
         fprintf(stderr, "[wfagpu] penalties must satisfy x >= 1, e >= 1, o >= 0 (got %d,%d,%d)\n", plan->x, plan->o, plan->e);
@@ -1274,7 +1298,7 @@ extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, 
      * given that budget straight away: 100 k x 1 kbp / 10 % with -e 300 re-dispatched 4.4 % of its pairs in every chunk. */
     int first_steps = plan->max_steps;
     pull_hint(d);
-    if (!ef && plan->band <= 0 && d->hint_dist > 0 && d->hint_lift_pm > 0 && d->hint_key[0] == plan->x && d->hint_key[1] == plan->o &&
+    if (!ef && !p2 && plan->band <= 0 && d->hint_dist > 0 && d->hint_lift_pm > 0 && d->hint_key[0] == plan->x && d->hint_key[1] == plan->o &&
         d->hint_key[2] == plan->e && d->hint_key[3] == length_class(s.max_len)) {
         const long long want = (long long)d->hint_dist + (long long)d->hint_dist * d->hint_margin_pm / 1000 + 12;
         const long long most = (long long)plan->max_steps + (long long)plan->max_steps * d->hint_lift_pm / 1000;
@@ -1426,7 +1450,7 @@ extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wf
     }
     s.stats.failed_pairs = (uint32_t)failed.size();
     memcpy(out, s.h_out.p, n * sizeof(wfagpu_pair_out_t));
-    if (!d->independent && !s.ef) learn_hint(d, s, n);
+    if (!d->independent && !s.ef && s.plan.e2 <= 0) learn_hint(d, s, n);
     if (pair_flags)
         for (size_t i = 0; i < n; ++i) pair_flags[i] = s.h_pairs.p[i].flags;
     if (ops) *ops = s.h_pool.p;
@@ -1497,7 +1521,7 @@ extern "C" int wfagpu_device_wait(wfagpu_device_t *d, int slot, float *ms_pack, 
         CK(cudaStreamSynchronize(s.stream));
         s.stats.pending_pairs = s.h_counters.p[CTR_RETRY] + s.h_counters.p[CTR_ASCII];
     }
-    if (s.n && d->use_hint && !s.ef) {
+    if (s.n && d->use_hint && !s.ef && s.plan.e2 <= 0) {
         /* read the result records back (16 B per pair) so that a re-run of the resident
          * batch is provisioned like the next batch of a stream would be */
         if (s.h_out.ensure(s.n)) return -1;

@@ -6,6 +6,7 @@
 
 #include <climits>
 #include <mutex>
+#include <type_traits>
 #include <unordered_map>
 #include <unordered_set>
 
@@ -469,6 +470,16 @@ constexpr uint32_t kRecLive = 4u, kRecStop = 8u, kRecTarget = 16u, kRecSnap = 32
 constexpr int kSchedBlock = 16;                 /* scores per block of records (power of two, <= 32) */
 constexpr uint32_t kSchedBytes = 2u * kSchedBlock * (uint32_t)sizeof(StepRec);
 
+/* Gap-affine 2-piece state of wfa_exact_kernel<..., P2 = true>: the second piece and its I2 / D2 rings (after D, depth
+ * e2 + 1), and the rows of the current score.  One piece uses the empty NoPiece2, so those kernels carry nothing extra. */
+template <typename RA>
+struct Piece2 {
+    int e2, oe2, ep;            /* e2, o2 + e2, min(e1, e2) (pruning)                                    */
+    RA I0, D0, Iend, Dend;      /* the I2 / D2 rings                                                      */
+    RA Ic, Dc, Mo, Ie, De;      /* rows of score d: I2 / D2 at d and d - e2, M at d - o2 - e2             */
+};
+struct NoPiece2 {};
+
 /* CKPT (CTA per pair, shared-memory rings, with backtrace): instead of a decision byte per
  * cell the forward pass snapshots the ring rows every p.ck_period scores, and the traceback
  * recomputes the offsets it needs on the dependency cone below the cell it stands on
@@ -478,15 +489,16 @@ constexpr uint32_t kSchedBytes = 2u * kSchedBlock * (uint32_t)sizeof(StepRec);
  * [-pb, tb]; the pruning measures the distance to the target range [kt - te, kt + pe] instead of kt; an M cell on
  * a target diagonal finishes when its offset reaches min(tlen, plen + k), the lowest such k of the first finishing
  * score wins; the traceback starts there and stops at score 0.  k_begin / k_end go to p.ends[idx]. */
-template <bool WARP, bool ASCII, bool BT, typename R, bool CKPT, bool EF = false>
+template <bool WARP, bool ASCII, bool BT, typename R, bool CKPT, bool EF = false, bool P2 = false>
 __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_kernel(const __grid_constant__ KernelParams p)
 {
     static_assert(!CKPT || (BT && !WARP && R::kElem == 2), "checkpointed traceback: CTA groups with shared-memory rings");
     static_assert(!(EF && CKPT), "ends-free: decision-byte traceback only");
+    static_assert(!(P2 && (CKPT || EF)), "gap-affine 2-piece: global alignment, decision-byte traceback only");
     using G = Group<WARP>;
     using RA = typename R::addr_t;
     constexpr bool GR = (R::kElem == 4);          /* rings in global memory */
-    constexpr bool SCHED = !WARP && !GR;          /* per-score schedule records (see StepRec) */
+    constexpr bool SCHED = !WARP && !GR && !P2;   /* per-score schedule records (see StepRec); 2-piece: rows in registers */
     constexpr int NULLV = R::kNull;
     extern __shared__ __align__(16) unsigned char smem_raw[];
 
@@ -496,7 +508,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
     const uint32_t group = blockIdx.x * groups_per_cta + G::id_in_cta();
 
     /* ---- carve shared memory: [rings][sequence stages][ctl] per group ---- */
-    const int rows = p.A + 2 * p.E1;
+    const int rows = p.A + 2 * p.E1 + (P2 ? 2 * p.E2 : 0);
     const uint32_t row_bytes = (uint32_t)p.row_stride * R::kElem;
     const uint32_t ring_bytes = GR ? 0u : (((uint32_t)rows * row_bytes + 15u) & ~15u);
     const uint32_t seq_bytes = (uint32_t)p.seq_words * 4u;          /* one sequence, one stage */
@@ -518,6 +530,15 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
     }
     const RA I0 = R::add(M0, (uint32_t)A * row_bytes);
     const RA D0 = R::add(I0, (uint32_t)E1 * row_bytes);
+    /* 2-piece: state of the second gap piece (an empty struct for one piece) */
+    std::conditional_t<P2, Piece2<RA>, NoPiece2> q2;
+    if constexpr (P2) {
+        q2.e2 = p.e2; q2.oe2 = p.o2 + p.e2; q2.ep = min(e, p.e2);
+        q2.I0 = R::add(D0, (uint32_t)E1 * row_bytes);
+        q2.D0 = R::add(q2.I0, (uint32_t)p.E2 * row_bytes);
+        q2.Iend = R::add(q2.I0, (uint32_t)p.E2 * row_bytes);
+        q2.Dend = R::add(q2.D0, (uint32_t)p.E2 * row_bytes);
+    }
 
     uint4 *arena = p.arena + (size_t)group * p.arena_units;    /* CKPT: one arena per pair, set below */
     uint32_t *const scratch = p.ops_scratch + (size_t)group * p.ops_scratch_words;
@@ -710,6 +731,17 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                 RA aMo = R::add(M0, (uint32_t)((A - oe % A) % A) * row_bytes);      /* row of score d - o - e */
                 RA aIe = R::add(I0, (uint32_t)((E1 - e % E1) % E1) * row_bytes);    /* row of score d - e     */
                 RA aDe = R::add(D0, (uint32_t)((E1 - e % E1) % E1) * row_bytes);
+                /* 2-piece: rows of I2 / D2 at d and d - e2, and of M at d - o2 - e2.  In an M/I/D step driven by
+                 * piece 1 with d < o2 + e2 (or the other way round) the M row of d - o2 - e2 is a row no score has
+                 * written yet: it reads as NULL only because the prologue covers [-2G, 2G] and the windows of the
+                 * first A scores (half width <= d < A = G) stay inside it. */
+                if constexpr (P2) {
+                    const int E2 = p.E2;
+                    q2.Ic = q2.I0; q2.Dc = q2.D0;
+                    q2.Mo = R::add(M0, (uint32_t)((A - q2.oe2 % A) % A) * row_bytes);
+                    q2.Ie = R::add(q2.I0, (uint32_t)((E2 - q2.e2 % E2) % E2) * row_bytes);
+                    q2.De = R::add(q2.D0, (uint32_t)((E2 - q2.e2 % E2) % E2) * row_bytes);
+                }
                 int ck_left = p.ck_period, ck_j = 0;
                 /* snapshot of the ring rows the scores above d can still read: M of scores d .. d-A+2,
                  * I and D of d .. d-e+1.  A snapshot row covers [-n, n] rounded out to 16-byte units;
@@ -741,6 +773,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                     }
                 };
                 int pr_q = Dmax / e, pr_r = Dmax % e;        /* (Dmax - d) = q * e + r */
+                if constexpr (P2) { pr_q = Dmax / q2.ep; pr_r = Dmax % q2.ep; }     /* 2-piece: q * min(e1, e2) + r */
                 unsigned long long n_cells = 0;              /* cells computed for this pair (optional counter) */
                 for (int d = 1; d <= Dmax; ++d) {
                     int n, lo, hi, kind;
@@ -767,7 +800,11 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                         n = st.n;
                         kind = st.kind;
                         row_off = st.row_off;
-                        if (pr_r == 0) { pr_r = e - 1; --pr_q; } else --pr_r;
+                        if constexpr (P2) {
+                            if (pr_r == 0) { pr_r = q2.ep - 1; --pr_q; } else --pr_r;
+                        } else {
+                            if (pr_r == 0) { pr_r = e - 1; --pr_q; } else --pr_r;
+                        }
                         live = EF ? prune_window_range(n, klo_t, khi_t, pr_q, p.n_cap, lo, hi)
                                   : prune_window(n, kt, pr_q, p.n_cap, lo, hi);
                         if (live && (lo < -p.n_cap || hi > p.n_cap)) break;     /* wider than the rings of this launch */
@@ -780,6 +817,13 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                         aIe = R::add(aIe, row_bytes); if (aIe == Iend) aIe = I0;
                         aDc = R::add(aDc, row_bytes); if (aDc == Dend) aDc = D0;
                         aDe = R::add(aDe, row_bytes); if (aDe == Dend) aDe = D0;
+                        if constexpr (P2) {
+                            q2.Mo = R::add(q2.Mo, row_bytes); if (q2.Mo == Mend) q2.Mo = M0;
+                            q2.Ic = R::add(q2.Ic, row_bytes); if (q2.Ic == q2.Iend) q2.Ic = q2.I0;
+                            q2.Ie = R::add(q2.Ie, row_bytes); if (q2.Ie == q2.Iend) q2.Ie = q2.I0;
+                            q2.Dc = R::add(q2.Dc, row_bytes); if (q2.Dc == q2.Dend) q2.Dc = q2.D0;
+                            q2.De = R::add(q2.De, row_bytes); if (q2.De == q2.Dend) q2.De = q2.D0;
+                        }
                         snap_now = false;
                         if (CKPT && --ck_left == 0) { ck_left = p.ck_period; ++ck_j; snap_now = true; }
                     }
@@ -789,6 +833,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                             R::st(aMc, k, NULLV);
                             R::st(aIc, k, NULLV);
                             R::st(aDc, k, NULLV);
+                            if constexpr (P2) { R::st(q2.Ic, k, NULLV); R::st(q2.Dc, k, NULLV); }
                         }
                         G::sync();
                         if (CKPT && snap_now) checkpoint(n, lo, hi);
@@ -799,6 +844,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                         for (int k = lo - GW + tid; k <= hi + GW; k += gsz) {
                             R::st(aIc, k, NULLV);
                             R::st(aDc, k, NULLV);
+                            if constexpr (P2) { R::st(q2.Ic, k, NULLV); R::st(q2.Dc, k, NULLV); }
                             int m = NULLV;
                             if (k >= lo && k <= hi) {
                                 m = R::ld(aMx, k) + 1;
@@ -814,10 +860,38 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                             R::st(aMc, k, NULLV);
                             R::st(aIc, k, NULLV);
                             R::st(aDc, k, NULLV);
+                            if constexpr (P2) { R::st(q2.Ic, k, NULLV); R::st(q2.Dc, k, NULLV); }
                         }
                         /* one decision byte per cell: bit0 I extends, bit1 D extends, bits 3:2 the winner of M
                          * (1 = I, 2 = X, 3 = D); a warp writes 32 consecutive bytes of the pair's row */
                         uint8_t *const rowb = reinterpret_cast<uint8_t *>(arena + row_off) + n;
+                        if constexpr (P2) {
+                            /* 2-piece decision byte: bit0 I1 extends, bit1 D1, bit2 I2, bit3 D2; bits 5:4 the op of M's
+                             * source (1 = I, 2 = X, 3 = D); bit6 that source is piece 2.  M: D1 > D2 > X > I1 > I2. */
+                            for (int k = lo + tid; k <= hi; k += gsz) {
+                                const int io1 = R::ld(aMo, k - 1) + 1, ie1 = R::ld(aIe, k - 1) + 1;
+                                const int io2 = R::ld(q2.Mo, k - 1) + 1, ie2 = R::ld(q2.Ie, k - 1) + 1;
+                                const int do1 = R::ld(aMo, k + 1), de1 = R::ld(aDe, k + 1);
+                                const int do2 = R::ld(q2.Mo, k + 1), de2 = R::ld(q2.De, k + 1);
+                                const int X = R::ld(aMx, k) + 1;
+                                const int I1 = max(io1, ie1), D1 = max(do1, de1);
+                                const int I2 = max(io2, ie2), D2 = max(do2, de2);
+                                const int I = max(I1, I2), D = max(D1, D2);
+                                int M = max(max(X, D), I);
+                                uint32_t src;
+                                if (D >= X && D >= I) src = D1 >= D2 ? 0x30u : 0x70u;
+                                else if (X >= I) src = 0x20u;
+                                else src = I1 >= I2 ? 0x10u : 0x50u;
+                                if (M >= 0) M = extend(k, M);
+                                R::st(aIc, k, I1);
+                                R::st(aDc, k, D1);
+                                R::st(q2.Ic, k, I2);
+                                R::st(q2.Dc, k, D2);
+                                R::st(aMc, k, M);
+                                if (BT) rowb[k] = (uint8_t)((ie1 >= io1 ? 1u : 0u) | (de1 >= do1 ? 2u : 0u) |
+                                                            (ie2 >= io2 ? 4u : 0u) | (de2 >= do2 ? 8u : 0u) | src);
+                            }
+                        } else
                         for (int k = lo + tid; k <= hi; k += gsz) {
                             const int io = R::ld(aMo, k - 1) + 1;
                             const int ie = R::ld(aIe, k - 1) + 1;
@@ -883,11 +957,22 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                             const int ii = ck + (int)st.n;
                             if (ii < 0 || ii > 2 * (int)st.n) { n_ops = 0; finished = false; break; }
                             const uint32_t dec = reinterpret_cast<const uint8_t *>(arena + st.row_off)[ii];
-                            const int mop = (int)(dec >> 2) & 3;
+                            const int mop = (int)(dec >> (P2 ? 4 : 2)) & 3;
                             if (mop == OP_SUB) cd -= x;
-                            else if (mop == OP_INS) comp = 1;
-                            else comp = 2;
+                            else if (mop == OP_INS) comp = (P2 && (dec & 64u)) ? 3 : 1;
+                            else comp = (P2 && (dec & 64u)) ? 4 : 2;
                         }
+                    } else if constexpr (P2) {
+                        /* comp 1 I1, 2 D1, 3 I2, 4 D2: the extend bit of comp c is bit c - 1; closing a gap of piece i
+                         * steps o_i + e_i down */
+                        const int ii = ck + (int)st.n;
+                        if (ii < 0 || ii > 2 * (int)st.n || st.kind != WFAGPU_STEP_MDI) { n_ops = 0; finished = false; break; }
+                        const uint32_t dec = reinterpret_cast<const uint8_t *>(arena + st.row_off)[ii];
+                        const bool ins = (comp & 1) != 0, second = comp >= 3;
+                        op = ins ? OP_INS : OP_DEL;
+                        ck += ins ? -1 : 1;
+                        if (dec & (1u << (comp - 1))) cd -= second ? q2.e2 : e;
+                        else { cd -= second ? q2.oe2 : oe; comp = 0; }
                     } else {
                         const int ii = ck + (int)st.n;
                         if (ii < 0 || ii > 2 * (int)st.n || st.kind != WFAGPU_STEP_MDI) { n_ops = 0; finished = false; break; }
@@ -3177,29 +3262,29 @@ void launch_cigar_text(const CigarParams &p, cudaStream_t s)
 
 /* ---- host-side launch helpers ---------------------------------------------- */
 
-template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false>
+template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false, bool P2 = false>
 static cudaError_t launch_one(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
 {
-    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF>;
+    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF, P2>;
     cudaError_t err = allow_max_smem(kfn);
     if (err != cudaSuccess) return err;
     kfn<<<ctas, threads, smem, s>>>(p);
     return cudaGetLastError();
 }
 
-template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false>
+template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false, bool P2 = false>
 static int occupancy_one(int threads, size_t smem)
 {
-    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF>;
+    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF, P2>;
     int n = 0;
     if (allow_max_smem(kfn) != cudaSuccess) return 0;
     if (occupancy_of(&n, kfn, threads, smem) != cudaSuccess) return 0;
     return n;
 }
 
-size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched)
+size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched, int E2)
 {
-    const int rows = A + 2 * E1;
+    const int rows = A + 2 * E1 + 2 * E2;
     const size_t ring_bytes = ((size_t)rows * row_stride * sizeof(int16_t) + 15) & ~(size_t)15;
     const size_t seq_bytes = (size_t)seq_words * 4;
     const size_t group_bytes = (ring_bytes + 2 * (size_t)stages * seq_bytes + sizeof(GroupCtl) + (sched ? kSchedBytes : 0) + 15) & ~(size_t)15;
@@ -3282,6 +3367,18 @@ template <bool WARP, bool ASCII, bool BT>
 static int occupancy_one_ef(int threads, size_t smem)
 {
     return occupancy_one<WARP, ASCII, BT, RingS16, false, true>(threads, smem);
+}
+
+/* gap-affine 2-piece instantiations: FN<WARP, ASCII, BT, R, false, false, true> */
+template <bool WARP, bool ASCII, bool BT>
+static cudaError_t launch_one_p2(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
+{
+    return launch_one<WARP, ASCII, BT, RingS16, false, false, true>(p, threads, ctas, smem, s);
+}
+template <bool WARP, bool ASCII, bool BT>
+static int occupancy_one_p2(int threads, size_t smem)
+{
+    return occupancy_one<WARP, ASCII, BT, RingS16, false, false, true>(threads, smem);
 }
 
 template <bool BT, bool COUNT>
@@ -3369,6 +3466,17 @@ cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_pe
         }
         return WFAGPU_DISPATCH(launch_one_ef, p, threads, ctas, smem_bytes, s);
     }
+    if (p.e2 > 0) {
+        /* gap-affine 2-piece: decision-byte traceback on every tier */
+        if (p.ck_off) return cudaErrorInvalidValue;
+        if (p.gring) {
+            if (ascii) return bt ? launch_one<false, true, true, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s)
+                                 : launch_one<false, true, false, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s);
+            return bt ? launch_one<false, false, true, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s)
+                      : launch_one<false, false, false, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s);
+        }
+        return WFAGPU_DISPATCH(launch_one_p2, p, threads, ctas, smem_bytes, s);
+    }
     if (p.gring) {
         /* large tier: CTA per pair, rings in global memory, int32 offsets */
         if (ascii) return bt ? launch_one<false, true, true, RingG32>(p, threads, ctas, smem_bytes, s)
@@ -3385,8 +3493,14 @@ cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_pe
     return WFAGPU_DISPATCH(launch_one, p, threads, ctas, smem_bytes, s);
 }
 
-int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii, bool bt, bool ef)
+int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii, bool bt, bool ef, bool p2)
 {
+    if (p2) {
+        if (ascii) return bt ? occupancy_one<false, true, true, RingG32, false, false, true>(threads, smem_bytes)
+                             : occupancy_one<false, true, false, RingG32, false, false, true>(threads, smem_bytes);
+        return bt ? occupancy_one<false, false, true, RingG32, false, false, true>(threads, smem_bytes)
+                  : occupancy_one<false, false, false, RingG32, false, false, true>(threads, smem_bytes);
+    }
     if (ef) {
         if (ascii) return bt ? occupancy_one<false, true, true, RingG32, false, true>(threads, smem_bytes)
                              : occupancy_one<false, true, false, RingG32, false, true>(threads, smem_bytes);
@@ -3400,10 +3514,11 @@ int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii, bool bt, b
 }
 
 int exact_max_ctas_per_sm(int group_threads, int groups_per_cta, size_t smem_bytes, bool ascii, bool bt, bool ckpt,
-                          bool ef)
+                          bool ef, bool p2)
 {
     const bool warp = (group_threads == 32);
     const int threads = warp ? 32 * groups_per_cta : group_threads;
+    if (p2) return WFAGPU_DISPATCH(occupancy_one_p2, threads, smem_bytes);
     if (ef) return WFAGPU_DISPATCH(occupancy_one_ef, threads, smem_bytes);
     if (ckpt) return ascii ? occupancy_one<false, true, true, RingS16, true>(threads, smem_bytes)
                            : occupancy_one<false, false, true, RingS16, true>(threads, smem_bytes);

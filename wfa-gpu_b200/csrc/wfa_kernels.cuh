@@ -91,6 +91,9 @@ struct KernelParams {
      * text, clamped per pair; the step table's half widths include the start row's max(pb, tb) */
     int ef_pb, ef_pe, ef_tb, ef_te;
     int2 *ends;                   /* ends-free: per pair {k_begin, k_end}; null in global mode */
+    /* gap-affine 2-piece (wfa_exact_kernel<..., P2 = true>): second gap piece and the depth of its I2 / D2 rings (e2 + 1);
+     * e2 == 0: one piece.  With P2, A = max(x, o + e, o2 + e2) + 1 */
+    int o2, e2, E2;
 };
 
 struct PackParams {
@@ -119,7 +122,7 @@ struct CigarParams {
 void launch_pack(const PackParams &p, cudaStream_t s);
 void launch_cigar_text(const CigarParams &p, cudaStream_t s);
 /* group_threads == 32 -> warp-per-pair variant; otherwise CTA-per-pair.  p.ends != null runs the ends-free
- * variant (decision-byte traceback only: p.ck_off must be null) */
+ * variant, p.e2 > 0 the gap-affine 2-piece variant (both: decision-byte traceback only, p.ck_off must be null) */
 cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_per_cta, int ctas,
                          size_t smem_bytes, bool ascii_extend, cudaStream_t s);
 /* CTA per pair, four diagonals per thread (packed sequences, shared-memory rings whose diagonal 0 is 16-byte
@@ -138,8 +141,10 @@ int bound_max_ctas_per_sm(int A, int E1, int warps);
 cudaError_t launch_traceback(const KernelParams &p, int ctas, int warps, bool ascii_extend, cudaStream_t s);
 size_t traceback_smem_bytes(int A, int period, int warps);
 int traceback_max_ctas_per_sm(int A, int period, int warps, bool ascii_extend);
-/* sched: CTA-per-pair kernels with shared-memory rings keep per-score schedule records (3 KB) */
-size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched = false);
+/* sched: CTA-per-pair kernels with shared-memory rings keep per-score schedule records (3 KB; not the 2-piece kernels).
+ * E2 > 0: the two extra I2 / D2 rings of a 2-piece launch */
+size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched = false,
+                        int E2 = 0);
 cudaError_t launch_banded(const KernelParams &p, int threads, int ctas, size_t smem_bytes, bool ascii_extend,
                           cudaStream_t s);
 size_t banded_smem_bytes(int A, int win, int seq_words, int stages);
@@ -150,8 +155,9 @@ size_t bandq_smem_bytes(int A, int win, int seq_words, int stages);
 int bandq_max_ctas_per_sm(int threads, size_t smem_bytes, bool with_bt);
 /* decision bytes of wfa_bandq_kernel -> 2-bit ops, one thread per pair of the launch */
 cudaError_t launch_band_traceback(const KernelParams &p, cudaStream_t s);
-int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii_extend, bool with_bt, bool ef = false);
+int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii_extend, bool with_bt, bool ef = false,
+                          bool p2 = false);
 int exact_max_ctas_per_sm(int group_threads, int groups_per_cta, size_t smem_bytes, bool ascii_extend, bool with_bt,
-                          bool ckpt = false, bool ef = false);
+                          bool ckpt = false, bool ef = false, bool p2 = false);
 
 } // namespace wfagpu

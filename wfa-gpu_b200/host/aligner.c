@@ -264,6 +264,25 @@ bool wfagpu_align_span(wfagpu_aligner_t *aligner, const wfagpu_span_t *span)
     return wfagpu_last_launch_ok();
 }
 
+bool wfagpu_align_affine2p(wfagpu_aligner_t *aligner, const wfagpu_affine2p_t *pen)
+{
+    if (!pen) return wfagpu_align(aligner);
+    if (!aligner) { ERR("Invalid aligner."); return false; }
+    if (!aligner->results || !aligner->sequences_metadata) { ERR("Aligner parameters are not initialized."); return false; }
+    if (pen->x < 1 || pen->o1 < 0 || pen->e1 < 1 || pen->o2 < 0 || pen->e2 < 1) {
+        ERR("Gap-affine 2-piece penalties must satisfy x >= 1, o1, o2 >= 0, e1, e2 >= 1.");
+        return false;
+    }
+    if (aligner->alignment_options.band > 0) {
+        ERR("Gap-affine 2-piece alignment cannot be combined with the adaptive band.");
+        return false;
+    }
+    wfagpu_launch_alignments_affine2p(aligner->sequences_buffer, aligner->sequences_buffer_len,
+                                      aligner->sequences_metadata, aligner->results, aligner->alignment_options,
+                                      aligner->alignment_options.compute_cigar, false, pen);
+    return wfagpu_last_launch_ok();
+}
+
 /* Extension: forget the pairs, keep the buffers (streaming: the next window is read into the same pinned memory). */
 void wfagpu_clear_sequences(wfagpu_aligner_t *aligner)
 {

@@ -113,6 +113,8 @@ typedef struct {
     bool host_cigar;        /* WFAGPU_HOST_CIGAR=1: print the CIGAR text on the host instead of the GPU */
     bool ef;                /* ends-free call: `span` is not all zero */
     wfagpu_span_t span;
+    bool p2;                /* gap-affine 2-piece call: `pen2` replaces opt.penalties */
+    wfagpu_affine2p_t pen2;
     int decode_threads;
     /* accumulated */
     wfagpu_run_stats_t stats;
@@ -273,6 +275,7 @@ static void fill_plan(const job_t *j, bool cigar, wfagpu_plan_t *plan)
     plan->with_cigar = cigar;
     plan->threads_hint = j->opt.threads_per_block;
     plan->workers_hint = j->opt.num_workers;
+    if (j->p2) { plan->o2 = j->pen2.o2; plan->e2 = j->pen2.e2; }
 }
 
 static int submit(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
@@ -334,7 +337,10 @@ static void check_chunk(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
     for (long i = 0; i < (long)f->n; ++i) {
         if (!(f->out[i].status & WFAGPU_ST_FINISHED)) continue;
         bool ok = true;
-        if (j->cigar)
+        if (j->cigar && j->p2)
+            ok = wfagpu_check_result_affine2p(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
+                                              m[i].text_len, &j->pen2, res[i].error, res[i].cigar.buffer);
+        else if (j->cigar)
             ok = wfagpu_check_result_span(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
                                           m[i].text_len, j->opt.penalties, j->ef ? &j->span : NULL, res[i].error,
                                           res[i].cigar.buffer);
@@ -502,12 +508,25 @@ void wfagpu_plan_chunks(size_t n, size_t batch_size, int n_devices, size_t ascii
 }
 
 static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_alignment_result_t *res,
-                    wfa_alignment_options_t opt, bool cigar, bool check, const wfagpu_span_t *ends_free)
+                    wfa_alignment_options_t opt, bool cigar, bool check, const wfagpu_span_t *ends_free,
+                    const wfagpu_affine2p_t *affine2p)
 {
     const double t0 = now_s();
     memset(&t_last_stats, 0, sizeof(t_last_stats));
     t_last_ok = false;
     if (!buf || !meta || !res) { fprintf(stderr, "[!] ERROR: invalid buffers.\n"); return; }
+    if (affine2p) {
+        const wfagpu_affine2p_t *q = affine2p;
+        if (q->x < 1 || q->o1 < 0 || q->e1 < 1 || q->o2 < 0 || q->e2 < 1) {
+            fprintf(stderr, "[!] ERROR: gap-affine 2-piece penalties must satisfy x >= 1, o1, o2 >= 0, e1, e2 >= 1.\n");
+            return;
+        }
+        if (opt.band > 0) {
+            fprintf(stderr, "[!] ERROR: gap-affine 2-piece alignment cannot be combined with the adaptive band (-B).\n");
+            return;
+        }
+        opt.penalties.x = q->x; opt.penalties.o = q->o1; opt.penalties.e = q->e1;
+    }
     if (opt.num_alignments == 0) { t_last_ok = true; return; }
     if (opt.penalties.x < 1 || opt.penalties.e < 1 || opt.penalties.o < 0) {
         /* x = 0 or e = 0 make a wavefront depend on itself; the reference reads
@@ -525,6 +544,10 @@ static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_align
         fprintf(stderr, "[!] ERROR: ends-free alignment cannot be combined with the adaptive band (-B).\n");
         return;
     }
+    if (ef && affine2p) {
+        fprintf(stderr, "[!] ERROR: gap-affine 2-piece alignment cannot be combined with an ends-free span.\n");
+        return;
+    }
     int devs[MAX_DEVICES];
     const int ndev = select_devices(devs);
     if (ndev < 1) return;
@@ -535,6 +558,8 @@ static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_align
     job.check = check;
     job.ef = ef;
     if (ef) job.span = *sp;
+    job.p2 = affine2p != NULL;
+    if (affine2p) job.pen2 = *affine2p;
     job.n = opt.num_alignments;
     job.pageable = !wfagpu_host_is_pinned(buf);
     const size_t span = meta[job.n - 1].text_offset + meta[job.n - 1].text_len + 1 - meta[0].pattern_offset;
@@ -627,7 +652,7 @@ void launch_alignments(char *sequences_buffer, const size_t sequences_buffer_siz
                        wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, true,
-            check_correctness, NULL);
+            check_correctness, NULL, NULL);
 }
 
 void launch_alignments_distance(char *sequences_buffer, const size_t sequences_buffer_size,
@@ -636,7 +661,7 @@ void launch_alignments_distance(char *sequences_buffer, const size_t sequences_b
                                 wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, false,
-            check_correctness, NULL);
+            check_correctness, NULL, NULL);
 }
 
 void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buffer_size,
@@ -645,5 +670,14 @@ void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buff
                                    const wfagpu_span_t *span)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
-            check_correctness, span);
+            check_correctness, span, NULL);
+}
+
+void wfagpu_launch_alignments_affine2p(char *sequences_buffer, size_t sequences_buffer_size,
+                                       sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                       wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                       const wfagpu_affine2p_t *pen)
+{
+    run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
+            check_correctness, NULL, pen);
 }

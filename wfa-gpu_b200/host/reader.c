@@ -243,6 +243,39 @@ bool wfagpu_check_result_span(const char *pattern, size_t plen, const char *text
     return v == plen && h == tlen && score == error;
 }
 
+/* The same under gap-affine 2-piece penalties: a gap run of length L costs min(o1 + e1 L, o2 + e2 L). */
+bool wfagpu_check_result_affine2p(const char *pattern, size_t plen, const char *text, size_t tlen,
+                                  const wfagpu_affine2p_t *pen, unsigned int error, const char *cigar)
+{
+    if (!pen || pen->x < 1 || pen->o1 < 0 || pen->e1 < 1 || pen->o2 < 0 || pen->e2 < 1) return false;
+    size_t v = 0, h = 0;
+    unsigned long score = 0;
+    const char *c = cigar;
+    if (!c) return false;
+    while (*c) {
+        unsigned long rep = 0;
+        if (*c < '0' || *c > '9') return false;
+        while (*c >= '0' && *c <= '9') rep = rep * 10 + (unsigned long)(*c++ - '0');
+        const char op = *c++;
+        if (op == 'M' || op == 'X') {
+            if (v + rep > plen || h + rep > tlen) return false;
+            for (unsigned long i = 0; i < rep; ++i)
+                if ((pattern[v + i] == text[h + i]) != (op == 'M')) return false;
+            v += rep; h += rep;
+            if (op == 'X') score += rep * (unsigned long)pen->x;
+        } else if (op == 'I' || op == 'D') {
+            const unsigned long c1 = (unsigned long)pen->o1 + rep * (unsigned long)pen->e1;
+            const unsigned long c2 = (unsigned long)pen->o2 + rep * (unsigned long)pen->e2;
+            score += c1 < c2 ? c1 : c2;
+            if (op == 'I') h += rep; else v += rep;
+        } else {
+            return false;
+        }
+        if (v > plen || h > tlen) return false;
+    }
+    return v == plen && h == tlen && score == error;
+}
+
 /* ---------------------------------------------------------------------------------------------
  * The reference library's validators under their own names, argument order (text first) and input format
  * (utils/verification.h:37-58).  The reference hands them the UNROLLED op string that its recover_cigar

@@ -60,7 +60,8 @@ class Step(C.Structure):
 
 class Plan(C.Structure):
     _fields_ = [("x", C.c_int), ("o", C.c_int), ("e", C.c_int), ("max_steps", C.c_int), ("band", C.c_int),
-                ("band_width", C.c_int), ("with_cigar", C.c_int), ("threads_hint", C.c_int), ("workers_hint", C.c_int)]
+                ("band_width", C.c_int), ("with_cigar", C.c_int), ("threads_hint", C.c_int), ("workers_hint", C.c_int),
+                ("o2", C.c_int), ("e2", C.c_int)]      # gap-affine 2-piece: second piece; e2 = 0 (default): one piece
 
 
 class PairOut(C.Structure):
@@ -80,6 +81,11 @@ class Span(C.Structure):
     """wfagpu_span_t: ends-free span in WFA2-lib's order (pattern begin / end, text begin / end)."""
     _fields_ = [("pattern_begin_free", C.c_int), ("pattern_end_free", C.c_int), ("text_begin_free", C.c_int),
                 ("text_end_free", C.c_int)]
+
+
+class Affine2p(C.Structure):
+    """wfagpu_affine2p_t: gap-affine 2-piece penalties; a gap of L bases costs min(o1 + e1 L, o2 + e2 L)."""
+    _fields_ = [("x", C.c_int), ("o1", C.c_int), ("e1", C.c_int), ("o2", C.c_int), ("e2", C.c_int)]
 
 
 class DevPair(C.Structure):
@@ -104,7 +110,8 @@ EXPORTS = [
     "wfagpu_host_is_pinned", "wfagpu_host_alloc", "wfagpu_host_free", "wfagpu_reserve", "wfagpu_parse_devices",
     "wfagpu_set_host_threads", "wfagpu_align_span", "wfagpu_launch_alignments_span", "wfagpu_device_align_span",
     "wfagpu_device_download_ends", "wfagpu_device_rescore_span", "wfagpu_ops_to_cigar_span",
-    "wfagpu_check_result_span", "wfagpu_build_step_table_span",
+    "wfagpu_check_result_span", "wfagpu_build_step_table_span", "wfagpu_align_affine2p",
+    "wfagpu_launch_alignments_affine2p", "wfagpu_check_result_affine2p", "wfagpu_build_step_table_affine2p",
 ]
 
 _lib = None
@@ -208,6 +215,15 @@ def load():
                                            C.c_uint, C.c_char_p]
     L.wfagpu_check_result_span.restype = C.c_bool
     L.wfagpu_build_step_table_span.argtypes = [C.c_int] * 6 + [P(Step), P(C.c_uint64)]
+    L.wfagpu_align_affine2p.argtypes = [P(AlignerStruct), P(Affine2p)]
+    L.wfagpu_align_affine2p.restype = C.c_bool
+    L.wfagpu_launch_alignments_affine2p.argtypes = [C.c_void_p, C.c_size_t, P(SequencePair), P(AlignmentResult),
+                                                    AlignmentOptions, C.c_bool, C.c_bool, P(Affine2p)]
+    L.wfagpu_launch_alignments_affine2p.restype = None
+    L.wfagpu_check_result_affine2p.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_size_t, P(Affine2p), C.c_uint,
+                                               C.c_char_p]
+    L.wfagpu_check_result_affine2p.restype = C.c_bool
+    L.wfagpu_build_step_table_affine2p.argtypes = [C.c_int] * 7 + [P(Step), P(C.c_uint64)]
     _lib = L
     return L
 
@@ -220,6 +236,16 @@ def span_of(ends_free):
     if len(vals) != 4:
         raise ValueError("ends_free takes four values: pattern_begin_free, pattern_end_free, text_begin_free, text_end_free")
     return Span(*vals)
+
+
+def affine2p_of(pen):
+    """A 5-tuple (x, o1, e1, o2, e2) -> Affine2p (None -> None)."""
+    if pen is None:
+        return None
+    vals = tuple(int(v) for v in pen)
+    if len(vals) != 5:
+        raise ValueError("affine2p takes five values: x, o1, e1, o2, e2")
+    return Affine2p(*vals)
 
 
 def _b(s):
@@ -250,10 +276,19 @@ class Aligner:
     def options(self):
         return self.s.alignment_options
 
-    def align(self, ends_free=None):
+    def align(self, ends_free=None, affine2p=None):
         """ends_free: None (global) or (pattern_begin_free, pattern_end_free, text_begin_free, text_end_free),
-        WFA2-lib's order: that many leading / trailing bases of either sequence are free (wfagpu_align_span)."""
+        WFA2-lib's order: that many leading / trailing bases of either sequence are free (wfagpu_align_span).
+        affine2p: None or (x, o1, e1, o2, e2), gap-affine 2-piece penalties for this call in place of the aligner's
+        (wfagpu_align_affine2p); global alignment only."""
         sp = span_of(ends_free)
+        pen2 = affine2p_of(affine2p)
+        if pen2 is not None:
+            if sp is not None:
+                raise ValueError("affine2p cannot be combined with ends_free")
+            if not self.L.wfagpu_align_affine2p(C.byref(self.s), C.byref(pen2)):
+                raise RuntimeError("wfagpu_align_affine2p failed (see stderr); there is no CPU fallback")
+            return True
         if sp is None:
             if not self.L.wfagpu_align(C.byref(self.s)):
                 raise RuntimeError("wfagpu_align failed (see stderr); there is no CPU fallback")

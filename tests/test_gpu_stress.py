@@ -13,7 +13,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 @pytest.mark.parametrize("env", [{}, {"WFAGPU_FORCE_BOUND": "1"}, {"WFAGPU_QUAD_MIN": "1"},
                                  {"WFAGPU_QUAD_MIN": "1", "WFAGPU_QUAD_PAIRS": "1", "WFAGPU_FORCE_BOUND": "1"},
-                                 {"WFAGPU_FORCE_LARGE": "1"}, {"WFAGPU_DEVICES": "0,0"}])
+                                 {"WFAGPU_FORCE_LARGE": "1"}, {"WFAGPU_DEVICES": "0,0"}, {"WFAGPU_STAGES": "1"},
+                                 {"WFAGPU_THREADS": "64"}])
 def test_randomised_sweep(env):
     pr = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "stress_parity.py"), "15", "7"],
                         env=dict(os.environ, **env), capture_output=True, text=True, timeout=600)

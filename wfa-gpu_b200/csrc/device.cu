@@ -108,6 +108,7 @@ struct HostTrace {
 enum { CTR_QUEUE = 0, CTR_POOL = 1, CTR_RETRY = 2, CTR_ASCII = 3, CTR_TBQ = 4, CTR_BQ = 5, CTR_WORDS = 8 };
 
 struct LaunchCfg {
+    KernelChoice k;       /* the wavefront kernel: the occupancy questions and the launch ask with this value */
     int group_threads;   /* 32 = warp per pair */
     int groups_per_cta;
     int ctas;
@@ -118,11 +119,9 @@ struct LaunchCfg {
     size_t smem;
     int A, E1, G;
     int E2;               /* gap-affine 2-piece: depth of the I2 / D2 rings (0: one piece) */
-    bool global_ring;     /* large tier: rings in global memory, int32 offsets */
-    bool ckpt;            /* checkpointed traceback (ring snapshots) instead of decision bytes */
-    bool quad;            /* wfa_quad_kernel: four diagonals per thread, packed int16 SIMD */
-    bool quad_pairs;      /* ... and two scores per barrier interval: rings one row deeper */
+    bool quad_pairs;      /* wfa_quad_kernel: two scores per barrier interval, rings one row deeper */
     int ring_m, ring_g;   /* rows of the M ring / of the I and D rings */
+    int win;              /* adaptive band: window width in diagonals (0: exact) */
 };
 
 struct Slot {
@@ -183,6 +182,8 @@ struct Slot {
     wfagpu_span_t span{};
     int ef_w = 0;                      /* half width of the start row: max(pb, tb), at most the longest sequence */
     int ef_ext = 0;                    /* widest end of the target range: max(pe, te), likewise */
+    bool plain = true;                 /* global single-piece batch (neither ends-free nor 2-piece): it reads and learns the
+                                        * provisioning hint, runs the packed-SIMD kernels and ring snapshots */
     DevBuf<int2> ends;                 /* per pair {k_begin, k_end} */
     PinBuf<int2> h_ends;
     size_t budget_cache = 0;           /* arena budget from the last cudaMemGetInfo (0 = ask again) */
@@ -439,76 +440,91 @@ extern "C" int wfagpu_device_upload(wfagpu_device_t *d, int slot, const char *as
     return 0;
 }
 
-/* Shared-memory / launch-shape policy (replaces available_shared_mem_per_block and
+/* Ring depths of a plan: M (A, also the guard width G), I / D (E1), I2 / D2 of a 2-piece plan (E2; 0 for one piece). */
+struct RingDepths {
+    int A, E1, E2;
+};
+static RingDepths ring_depths(const wfagpu_plan_t &plan)
+{
+    const bool p2 = plan.e2 > 0;
+    return {std::max(std::max(plan.o + plan.e, plan.x), p2 ? plan.o2 + plan.e2 : 0) + 1, plan.e + 1, p2 ? plan.e2 + 1 : 0};
+}
+
+/* Ring row geometry for a half width `ncap` and guard width G.  Aligned rows (snapshots copy 16-byte units, the quad
+ * kernels load 8 or 16 bytes): diagonal 0 sits on an 8-element boundary and a row has 8 spare cells on both sides. */
+static int ring_center(int ncap, int G, bool aligned) { return aligned ? ((ncap + 2 * G + 8 + 7) & ~7) : ncap + 2 * G + 1; }
+static int ring_stride(int ncap, int G, bool aligned)
+{
+    return aligned ? 2 * ring_center(ncap, G, true) : 2 * (ncap + 2 * G + 1) + 2;
+}
+
+static int occupancy(const KernelChoice &k, size_t smem) { return max_ctas_per_sm(wavefront_kernel(k), k.threads, smem); }
+
+/* Large tier (long sequences, or rings that do not fit one CTA's shared memory even single-buffered): a CTA per pair,
+ * int32 rings in global memory. */
+static int choose_large_cfg(wfagpu_device *d, const Slot &s, int n_want, size_t n_items, LaunchCfg *c)
+{
+    KernelChoice &kc = c->k;
+    kc.gring = true;
+    c->groups_per_cta = 1;
+    c->stages = 1;
+    c->n_cap = n_want;
+    /* packed pairs: four diagonals per thread with 128-bit loads (wfa_quadg_kernel): rows 16-byte aligned */
+    const bool quad = !kc.ascii && !d->no_quad && s.plain;       /* ends-free, 2-piece: one diagonal per thread */
+    kc.family = quad ? Family::QuadG : Family::Exact;
+    c->row_stride = ring_stride(n_want, c->G, quad);
+    c->center = ring_center(n_want, c->G, quad);
+    c->smem = exact_smem_bytes(c->A, c->E1, 0, c->seq_words, 1, 1, quad);     /* sequences + control (+ schedule records) only */
+    if (!kc.ascii && c->smem > d->prop.sharedMemPerBlockOptin) {
+        fprintf(stderr, "[wfagpu] sequences of %u bases do not fit in shared memory; not supported yet\n", s.max_len);
+        return -2;
+    }
+    int most;
+    if (quad) {
+        /* one CTA per SM -- 148 x 0.7 MB of rings stay resident in the 126 MB L2 (two per SM: 681 instead of 902 pairs/s
+         * at 50 kbp / 15 %); measured on B200, 592 pairs: 512 threads 1030, 768 1077, 1024 (64 registers) 1098 pairs/s */
+        c->group_threads = d->force_threads ? d->force_threads : (n_want >= 2048 ? 1024 : (n_want >= 512 ? 512 : 256));
+        most = 1;
+    } else {
+        /* wide wavefronts (50 kbp / 15 %: ~10 k diagonals per score) keep 1024 threads busy: 581 vs 416
+         * pairs/s against 512 threads on B200 */
+        c->group_threads = d->force_threads ? d->force_threads : (n_want >= 2048 ? 1024 : 512);
+        most = 2;
+    }
+    kc.threads = c->group_threads;
+    int occ = occupancy(kc, c->smem);
+    if (occ < 1) return -1;
+    occ = std::min(occ, d->force_ctas_per_sm ? d->force_ctas_per_sm : most);
+    c->ctas = (int)std::max<size_t>(1, std::min<size_t>((size_t)occ * d->prop.multiProcessorCount, n_items));
+    return 0;
+}
+
+/* Shared-memory / launch-shape policy of the exact kernels (replaces available_shared_mem_per_block and
  * the <<<num_workers, tpb>>> choice of lib/sequence_alignment.cu:81-108,211-330).
  *
  * The wavefront rings live in shared memory, so their width decides how many CTAs
  * share an SM.  Measured on B200 (10 kbp / 5 %): 1 CTA x 1024 threads 62 k pairs/s,
  * 2 x 512 95 k, 3 x 384 109 k -- more, smaller CTAs hide the per-score barrier.
  * `n_want` is the half width the launch should be able to hold. */
-static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_min, uint32_t max_len, size_t n_items,
-                      bool ascii, bool bt, bool ef, int o2, int e2, LaunchCfg *c)
+static int choose_cfg(wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan, int n_want, int n_min, size_t n_items,
+                      bool ascii, LaunchCfg *c)
 {
-    /* 2-piece (e2 > 0): one diagonal per thread, decision bytes, no schedule records; two more rings of e2 + 1 rows */
-    const bool p2 = e2 > 0;
-    const int A = std::max(std::max(o + e, x), p2 ? o2 + e2 : 0) + 1, E1 = e + 1, G = A, E2 = p2 ? e2 + 1 : 0;
-    const bool sched = !p2;
+    /* 2-piece: one diagonal per thread, decision bytes, no schedule records; two more rings of e2 + 1 rows */
+    const bool p2 = plan.e2 > 0, sched = !p2, bt = plan.with_cigar != 0;
+    const RingDepths rd = ring_depths(plan);
+    const int A = rd.A, E1 = rd.E1, G = A, E2 = rd.E2;
     const size_t smem_max = d->prop.sharedMemPerBlockOptin;        /* 227 KB on B200 */
     const size_t smem_sm = d->prop.sharedMemPerMultiprocessor;     /* 228 KB */
-    const int seq_words = (int)packed_words_for(max_len);
+    const int seq_words = (int)packed_words_for(s.max_len);
     c->A = A; c->E1 = E1; c->G = G; c->E2 = E2; c->seq_words = seq_words;
-    n_want = std::max(1, n_want);
-    /* ring row geometry.  Checkpointed traceback copies rows in 16-byte units: diagonal 0 sits on
-     * an 8-element boundary and a row has 8 spare cells on both sides. */
-    bool ck = false;       /* aligned row geometry: snapshots (16-byte units) and the quad kernel (LDS.64) need it */
-    auto ctr = [&](int ncap) { return ck ? ((ncap + 2 * G + 8 + 7) & ~7) : ncap + 2 * G + 1; };
-    auto rs = [&](int ncap) { return ck ? 2 * ctr(ncap) : 2 * (ncap + 2 * G + 1) + 2; };
-
-    c->global_ring = false;
-    c->ckpt = false;
-    c->quad = false;
-    c->quad_pairs = false;
     c->ring_m = A; c->ring_g = E1;
-    bool large = d->force_large || max_len >= (1u << 15);
-    if (!large) {
-        /* rings that do not fit one CTA's shared memory even single-buffered go to the large tier */
-        if (exact_smem_bytes(A, E1, rs(n_want), seq_words, 1, 1, sched, E2) > smem_max) large = true;
-    }
-    if (large) {
-        c->global_ring = true;
-        c->groups_per_cta = 1;
-        c->stages = 1;
-        c->n_cap = n_want;
-        /* packed pairs: four diagonals per thread with 128-bit loads (wfa_quadg_kernel): rows 16-byte aligned */
-        c->quad = !ascii && !d->no_quad && !ef && !p2;       /* ends-free, 2-piece: one diagonal per thread */
-        ck = c->quad;
-        c->row_stride = rs(n_want);
-        c->center = c->quad ? ctr(n_want) : n_want + 2 * G + 1;
-        c->smem = exact_smem_bytes(A, E1, 0, seq_words, 1, 1, c->quad);     /* sequences + control (+ schedule records) only */
-        if (!ascii && c->smem > smem_max) {
-            fprintf(stderr, "[wfagpu] sequences of %u bases do not fit in shared memory; not supported yet\n", max_len);
-            return -2;
-        }
-        int occ;
-        if (c->quad) {
-            /* one CTA per SM -- 148 x 0.7 MB of rings stay resident in the 126 MB L2 (two per SM: 681 instead of 902 pairs/s
-             * at 50 kbp / 15 %); measured on B200, 592 pairs: 512 threads 1030, 768 1077, 1024 (64 registers) 1098 pairs/s */
-            c->group_threads = d->force_threads ? d->force_threads : (n_want >= 2048 ? 1024 : (n_want >= 512 ? 512 : 256));
-            occ = quadg_max_ctas_per_sm(c->group_threads, c->smem, bt);
-            if (occ < 1) return -1;
-            occ = std::min(occ, d->force_ctas_per_sm ? d->force_ctas_per_sm : 1);
-        } else {
-            /* wide wavefronts (50 kbp / 15 %: ~10 k diagonals per score) keep 1024 threads busy: 581 vs 416
-             * pairs/s against 512 threads on B200 */
-            c->group_threads = d->force_threads ? d->force_threads : (n_want >= 2048 ? 1024 : 512);
-            occ = large_max_ctas_per_sm(c->group_threads, c->smem, ascii, bt, ef, p2);
-            if (occ < 1) return -1;
-            occ = std::min(occ, d->force_ctas_per_sm ? d->force_ctas_per_sm : 2);
-        }
-        c->ctas = (int)std::max<size_t>(1, std::min<size_t>((size_t)occ * d->prop.multiProcessorCount, n_items));
-        return 0;
-    }
-    bool warp = (rs(n_want) <= 400) && max_len <= 1024;
+    KernelChoice &kc = c->k;
+    kc.ascii = ascii; kc.bt = bt; kc.ef = s.ef; kc.p2 = p2;
+    n_want = std::max(1, n_want);
+    if (d->force_large || s.max_len >= (1u << 15) ||
+        exact_smem_bytes(A, E1, ring_stride(n_want, G, false), seq_words, 1, 1, sched, E2) > smem_max)
+        return choose_large_cfg(d, s, n_want, n_items, c);
+    bool warp = (ring_stride(n_want, G, false) <= 400) && s.max_len <= 1024;
     if (d->force_warp >= 0) warp = d->force_warp != 0;
 
     if (warp) {
@@ -516,8 +532,8 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
         c->groups_per_cta = 8;
         c->stages = 2;
         c->n_cap = n_want;
-        c->row_stride = rs(c->n_cap);
-        c->center = c->n_cap + 2 * G + 1;
+        c->row_stride = ring_stride(c->n_cap, G, false);
+        c->center = ring_center(c->n_cap, G, false);
         c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages, false, E2);
         while (c->smem > smem_max && c->groups_per_cta > 1) {
             c->groups_per_cta >>= 1;
@@ -527,15 +543,17 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
     }
     if (!warp) {
         c->groups_per_cta = 1;
-        c->ckpt = bt && !d->no_ckpt && !ef && !p2;     /* ends-free, 2-piece: decision bytes */
+        kc.ckpt = bt && !d->no_ckpt && s.plain;     /* ends-free, 2-piece: decision bytes */
         /* packed pairs on shared-memory rings run four diagonals per thread (with backtrace: snapshots only) */
         /* (measured on B200: 1 kbp / 10 %, ring half width 196: 9.5 ms per 50 k pairs with one diagonal per thread and 16 CTAs per
          * SM against 11.0 ms; from a half width of ~300 on the four-diagonal kernel wins) */
-        c->quad = !ascii && !d->no_quad && !ef && !p2 && (!bt || c->ckpt) && n_want >= d->quad_min;
+        const bool quad = !ascii && !d->no_quad && s.plain && (!bt || kc.ckpt) && n_want >= d->quad_min;
+        kc.family = quad ? Family::Quad : Family::Exact;
         /* two scores per barrier: score d + 1 must not read the extended M of score d (x >= 2, o + e >= 2) and takes
          * its extend sources from registers (e == 1); costs one more row per ring */
-        c->quad_pairs = c->quad && !d->no_quad_pairs && x >= 2 && o + e >= 2 && e == 1;
-        ck = c->ckpt || c->quad;
+        c->quad_pairs = quad && !d->no_quad_pairs && plan.x >= 2 && plan.o + plan.e >= 2 && plan.e == 1;
+        const bool ck = kc.ckpt || quad;       /* aligned row geometry */
+        auto rs = [&](int ncap) { return ring_stride(ncap, G, ck); };
         const int RA = A + (c->quad_pairs ? 1 : 0), RE = E1 + (c->quad_pairs ? 1 : 0);
         c->ring_m = RA; c->ring_g = RE;
         int best_k = 0, stages = 1, n_cap = n_want;
@@ -548,14 +566,15 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
         /* n_min <= n_want: the rings may be provisioned below n_want (down to n_min) when that buys
          * another resident CTA -- the few pairs that then outgrow them are re-dispatched */
         n_min = std::max(1, std::min(n_min, n_want));
+        auto occ_at = [&](int threads, size_t bytes) {
+            KernelChoice probe = kc;
+            probe.threads = threads;
+            return occupancy(probe, bytes);
+        };
         /* do k CTAs of the smallest shape really fit with this much dynamic shared memory?  The arithmetic budget below is
          * a first filter; the runtime's occupancy calculator decides (allocation granularity: a ring 6 diagonals wider than
          * the arithmetic allowed cost rank 3 of an 8-GPU run its fifth CTA per SM, 33.4 instead of 29.2 ms per step) */
-        auto fits = [&](int k, size_t bytes, size_t budget) {
-            if (bytes > budget) return false;
-            const int occ_k = c->quad ? quad_max_ctas_per_sm(64, bytes, bt) : exact_max_ctas_per_sm(64, 1, bytes, ascii, bt, c->ckpt, ef, p2);
-            return occ_k >= k;
-        };
+        auto fits = [&](int k, size_t bytes, size_t budget) { return bytes <= budget && occ_at(64, bytes) >= k; };
         for (int k = kmax; k >= 1 && !best_k; --k) {
             /* every resident CTA also reserves 1 KB of system shared memory */
             const size_t budget = std::min(smem_max, smem_sm / k - 1024);
@@ -586,17 +605,17 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
         c->stages = stages;
         c->n_cap = n_cap;
         c->row_stride = rs(n_cap);
-        c->center = ctr(n_cap);
+        c->center = ring_center(n_cap, G, ck);
         c->smem = smem;
         /* about 1152 threads per SM in total, never more threads than half the widest wavefront */
         /* (measured on B200: 3 x 384, 5 x 192 -- the per-score overhead is paid per warp) */
         int t = best_k == 1 ? 1024 : (best_k == 2 ? 512 : (best_k == 3 ? 384 : ((960 / best_k) / 32) * 32));
         const int width = 2 * n_cap + 1;
-        if (c->quad) {
+        if (quad) {
             /* a thread covers four diagonals per trip: one to two trips over the average window (~ n_cap);
              * the kernel needs ~80 registers: never so many threads that the registers cost a resident CTA */
             t = std::min(std::min(t, 512), std::max(64, ((n_cap / 6) + 31) & ~31));
-            while (t > 64 && !d->force_threads && quad_max_ctas_per_sm(t, smem, bt) < best_k) t -= 32;
+            while (t > 64 && !d->force_threads && occ_at(t, smem) < best_k) t -= 32;
         } else {
             while (t > 64 && t * 2 > width) t -= 32;
         }
@@ -604,17 +623,63 @@ static int choose_cfg(wfagpu_device *d, int x, int o, int e, int n_want, int n_m
         if (d->force_threads) t = d->force_threads;
         c->group_threads = t;
     }
-    const int threads = warp ? 32 * c->groups_per_cta : c->group_threads;
-    int occ = c->quad ? quad_max_ctas_per_sm(c->group_threads, c->smem, bt)
-                      : exact_max_ctas_per_sm(c->group_threads, c->groups_per_cta, c->smem, ascii, bt, c->ckpt, ef, p2);
+    kc.warp = c->group_threads == 32;     /* 32 threads per group run the warp kernel, also when WFAGPU_THREADS=32 */
+    kc.threads = kc.warp ? 32 * c->groups_per_cta : c->group_threads;
+    int occ = occupancy(kc, c->smem);
     if (occ < 1) {
-        fprintf(stderr, "[wfagpu] kernel configuration does not fit (threads=%d smem=%zu)\n", threads, c->smem);
+        fprintf(stderr, "[wfagpu] kernel configuration does not fit (threads=%d smem=%zu)\n", kc.threads, c->smem);
         return -1;
     }
     if (d->force_ctas_per_sm) occ = std::min(occ, d->force_ctas_per_sm);
     size_t ctas = (size_t)occ * d->prop.multiProcessorCount;
     const size_t need = (n_items + c->groups_per_cta - 1) / c->groups_per_cta;
     c->ctas = (int)std::max<size_t>(1, std::min(ctas, need));
+    return 0;
+}
+
+/* Launch shape of the adaptive band: window = the reference's threads_per_block (lib/sequence_alignment.cu:270-277). */
+static int choose_band_cfg(wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan, size_t n_items, bool ascii,
+                           LaunchCfg *c)
+{
+    const int win = plan.band_width > 0 ? plan.band_width : 512;
+    const int d_full = s.tab_d_end;
+    int n_full = 0;
+    for (int dd = d_full - 1; dd >= 0 && dd >= d_full - 4; --dd) n_full = std::max(n_full, (int)s.h_steps.p[dd].n);
+    c->win = win;
+    c->A = ring_depths(plan).A; c->E1 = plan.e + 1; c->G = c->A;
+    c->seq_words = (int)packed_words_for(s.max_len);
+    c->groups_per_cta = 1;
+    /* a few diagonals per thread: the per-score overhead (window bookkeeping, barrier) is paid
+     * per thread, and small CTAs let more pairs share an SM (measured on B200, W = 512:
+     * 512 threads 114 k, 256 threads 165 k, 128 threads 189 k pairs/s at 10 kbp / 5 %) */
+    c->group_threads = std::min(1024, std::max(64, ((win / 4) + 31) & ~31));
+    /* packed pairs: four diagonals per thread (wfa_bandq_kernel), one quad per thread and score */
+    const bool quad = !ascii && !d->no_quad;
+    c->k.family = quad ? Family::BandQ : Family::Banded;
+    c->k.ascii = ascii;
+    c->k.bt = plan.with_cigar != 0;
+    /* a window spans win / 4 + 1 quads: two trips of half of them (measured on B200, W = 512, 10 kbp / 5 %:
+     * 64 threads 32.5 ms, 96 threads 31.4 ms, 128 threads 33.0 ms per 8192 pairs end to end) */
+    if (quad) c->group_threads = std::min(512, std::max(64, (((win / 4 + 2) / 2) + 31) & ~31));
+    if (d->force_threads) c->group_threads = d->force_threads;
+    auto band_smem = [&](int stages) {
+        return quad ? bandq_smem_bytes(c->A, win, c->seq_words, stages) : banded_smem_bytes(c->A, win, c->seq_words, stages);
+    };
+    c->stages = 2;
+    c->smem = band_smem(c->stages);
+    if (c->smem > d->prop.sharedMemPerBlockOptin) {
+        c->stages = 1;
+        c->smem = band_smem(c->stages);
+    }
+    if (c->smem > d->prop.sharedMemPerBlockOptin) {
+        fprintf(stderr, "[wfagpu] band of %d diagonals does not fit in shared memory\n", win);
+        return -2;
+    }
+    c->n_cap = n_full; c->row_stride = win; c->center = 0;
+    c->k.threads = c->group_threads;
+    const int occ = occupancy(c->k, c->smem);
+    if (occ < 1) return -1;
+    c->ctas = (int)std::max<size_t>(1, std::min<size_t>((size_t)occ * d->prop.multiProcessorCount, n_items));
     return 0;
 }
 
@@ -635,6 +700,31 @@ static void learn_hint(wfagpu_device *d, Slot &s, size_t n)
     d->hint_mean = cnt ? sum / (double)cnt : 0;
     d->hint_key[0] = s.plan.x; d->hint_key[1] = s.plan.o; d->hint_key[2] = s.plan.e; d->hint_key[3] = length_class(s.max_len);
     push_hint(d);
+}
+
+/* the hint was learnt on a batch like this one: exact alignment, same penalties, same length class */
+static bool hint_applies(const wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan)
+{
+    return plan.band <= 0 && d->hint_dist > 0 && d->hint_key[0] == plan.x && d->hint_key[1] == plan.o &&
+           d->hint_key[2] == plan.e && d->hint_key[3] == length_class(s.max_len);
+}
+
+/* the hint's largest score plus `pm` per mille plus `k` */
+static long long hint_plus(const wfagpu_device *d, int pm, int k)
+{
+    return (long long)d->hint_dist + (long long)d->hint_dist * pm / 1000 + k;
+}
+
+/* Does bounding every pair pay?  With D = d_end - 1 and a typical score m (the hint's mean score, or D / 2 when `m_hint`
+ * is 0), the launch bound leaves cells(D/m) * m^2 cells per pair (cells(r) = r^2/4 + (1.5r - 1)(1 - r/2), 1 from r = 2 on),
+ * the pair's own bound 0.5 * m^2; the bound pass costs ~32 cells per score at ~3x the cost per cell (measured on B200:
+ * ~240 against ~2.75 warp instructions). */
+static bool bound_pays(int d_end, double m_hint)
+{
+    const double m = m_hint > 0 ? m_hint : 0.5 * (d_end - 1);
+    const double r = std::min(2.0, std::max(1.0, (d_end - 1) / std::max(1.0, m)));
+    const double cells = r * r / 4 + (1.5 * r - 1) * (1 - r / 2);
+    return (cells - 0.5) * m > 130.0;
 }
 
 /* The host-built tables are uploaded from pinned memory that the next pass rewrites.  Waiting for the last such upload
@@ -661,8 +751,7 @@ static int ensure_ck_table(Slot &s, const wfagpu_plan_t &plan, int period)
 {
     if (s.ck_key[0] == period) return 0;
     const int de = s.tab_d_end;
-    const int A = std::max(plan.o + plan.e, plan.x) + 1;
-    const uint64_t rows_ck = (uint64_t)(A - 1 + 2 * plan.e);
+    const uint64_t rows_ck = (uint64_t)(ring_depths(plan).A - 1 + 2 * plan.e);
     const int n_ck = (de - 1) / period + 2;
     s.h_ck_off.assign((size_t)n_ck + 1, 0);
     if (s.h_ck32.ensure((size_t)n_ck + 1)) return -1;
@@ -689,7 +778,7 @@ static int ensure_ck_table(Slot &s, const wfagpu_plan_t &plan, int period)
 static int ensure_step_table(Slot &s, const wfagpu_plan_t &plan, int max_steps)
 {
     const bool p2 = plan.e2 > 0;
-    const int widest = std::max(std::max(plan.x, plan.o + plan.e), p2 ? plan.o2 + plan.e2 : 0);
+    const int widest = ring_depths(plan).A - 1;
     const int max_dist = std::min<long long>((long long)max_steps * (widest + 1) + 16, 1 << 30);
     const int tab_win = plan.band > 0 ? (plan.band_width > 0 ? plan.band_width : 512) : 0;
     const int extra = s.ef ? s.ef_w : 0;   /* ends-free: the start row widens every score's range */
@@ -715,10 +804,11 @@ static int ensure_step_table(Slot &s, const wfagpu_plan_t &plan, int max_steps)
     return 0;
 }
 
-/* Score upper bounds only (wfa_bound_kernel) for `n_items` entries of `order_dev`, with a budget of
- * `max_steps`: the re-dispatch loop uses them to pick a budget that is enough in one go and to prune
- * that pass per pair.  Leaves the step table of `max_steps` cached. */
-static int run_bound_only(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int max_steps, const uint32_t *order_dev,
+/* Score upper bounds only (wfa_bound_kernel) for `n_items` entries of `order_dev`, with a budget of `max_steps`, queued for the
+ * host: s.h_bound (indexed by pair) holds them after the next stream sync.  The first pass sizes its rings from them; the
+ * re-dispatch loop picks a budget that is enough in one go and prunes that pass per pair.  -2: the bound kernel does not serve
+ * these penalties.  Leaves the step table of `max_steps` cached. */
+static int bounds_to_host(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int max_steps, const uint32_t *order_dev,
                           size_t n_items)
 {
     if (plan.e2 > 0) return -2;           /* the bound kernel and its step table are single-piece */
@@ -732,7 +822,7 @@ static int run_bound_only(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, 
     kp.steps = s.steps.p;
     kp.d_end = s.tab_d_end;
     kp.x = plan.x; kp.o = plan.o; kp.e = plan.e;
-    kp.A = std::max(plan.o + plan.e, plan.x) + 1;
+    kp.A = ring_depths(plan).A;
     kp.E1 = plan.e + 1;
     kp.bound = s.bound.p;
     kp.bound_queue = s.counters.p + CTR_BQ;
@@ -747,257 +837,231 @@ static int run_bound_only(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, 
         return -1;
     }
     s.stats.launches += 1;
+    if (s.h_bound.ensure(s.n + 1)) return -1;
+    CK(cudaMemcpyAsync(s.h_bound.p, s.bound.p, s.n * sizeof(int32_t), cudaMemcpyDeviceToHost, s.stream));
     return 0;
 }
 
-/* Launch one pass over `n_items` entries of `order_dev`. */
-static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int max_steps, const uint32_t *order_dev,
-                       size_t n_items, uint32_t *retry_dev, bool ascii, bool first_pass, bool use_hint,
-                       bool *capped_out, bool have_bounds = false)
+/* What one pass aligns. */
+struct PassRequest {
+    const uint32_t *order;      /* device list of pair indices */
+    size_t n_items;             /* entries of `order` this pass aligns */
+    uint32_t *retry;            /* device list the pass appends the pairs it does not finish to */
+    int max_steps;              /* wavefront-step budget */
+    bool ascii = false;         /* byte-compare kernels on the ASCII copy (pairs with non-ACGT bytes) */
+    bool first_pass = false;    /* the batch's first pass: hints, bound pre-pass, wavefront timing, launch-shape stats */
+    bool have_bounds = false;   /* s.bound already holds the bounds of these pairs */
+    size_t n_seed = 0;          /* bound pre-pass: entries after the first n_items that skip this pass (straight to `retry`) */
+};
+
+/* Scores a pass provisions for. */
+struct Scores {
+    int d_full = 0;             /* the full budget: the step table's d_end */
+    int d_reach = 0;            /* scores beyond this cannot occur in this batch */
+    int d_want = 0;             /* scores the rings are provisioned for */
+    bool hinted = false;        /* d_want comes from the hint */
+    int d_p99 = 0;              /* 99 % of the bounded pairs finish below this score (0 = unknown) */
+    int n_want = 0;             /* exact: ring half width for d_want */
+};
+
+/* Ring half width for scores below d_end.  The kernel prunes every cell that cannot reach the target diagonal within
+ * d_end - 1 (score-bound pruning), so the rings only have to hold max_d min(n_d, kt_max + (d_end - 1 - d) / e). */
+static int n_need(const Slot &s, const wfagpu_plan_t &plan, int d_end)
 {
-    HostTrace tr;
-    if (first_pass) pull_hint(d);            /* what the last batch on this GPU needed (any context) */
-    const bool p2 = plan.e2 > 0;
-    /* ends-free, 2-piece: hints of (single-piece) global batches do not apply */
-    if (first_pass && (s.ef || p2)) { d->hint_dist = 0; d->hint_mean = 0; }
-    if (ensure_step_table(s, plan, max_steps)) return -1;
     const wfagpu_step_t *tab = s.h_steps.p;
-    const int d_full = s.tab_d_end;
-    int n_full = 0;
-    for (int dd = d_full - 1; dd >= 0 && dd >= d_full - 4; --dd) n_full = std::max(n_full, (int)tab[dd].n);
-    /* Scores to provision for: the full budget, or (first pass only) what recent batches with
-     * these penalties needed plus a margin -- pairs that outgrow it are re-dispatched.  The kernel
-     * prunes every cell that cannot reach the target diagonal within d_end - 1 (score-bound
-     * pruning), so the rings only have to hold max_d min(n_d, kt_max + (d_end - 1 - d) / e). */
-    int d_want = d_full;
-    bool hinted = false;
-    if (use_hint && plan.band <= 0 && d->hint_dist > 0 && d->hint_key[0] == plan.x && d->hint_key[1] == plan.o && d->hint_key[2] == plan.e &&
-        d->hint_key[3] == length_class(s.max_len)) {
-        d_want = (int)std::min<long long>((long long)d->hint_dist + (long long)d->hint_dist * d->hint_margin_pm / 1000 + 8, d_full - 1) + 1;
-        hinted = d_want < d_full;
+    const int pen_e = plan.e2 > 0 ? std::min(plan.e, plan.e2) : plan.e;     /* 2-piece: the pruning's min(e1, e2) */
+    const long long kt_max = s.kt_max;
+    /* n_d grows, kt + (Dmax - d) / e shrinks: the largest min sits where they cross.  A global pair with |kt| > Dmax / e
+     * cannot finish; an ends-free one can (the start row and the target range may meet at no cost), and its window
+     * reaches max(pe, te) beyond kt: no clamp, n_d bounds it */
+    const long long Dmax = d_end - 1;
+    const long long ktm = s.ef ? kt_max + s.ef_ext : std::min<long long>(kt_max, Dmax / pen_e);
+    int lo = 0, hi = d_end;                      /* first d with n_d >= ktm + (Dmax - d) / e */
+    while (lo < hi) {
+        const int mid = (lo + hi) / 2;
+        if ((long long)tab[mid].n >= ktm + (Dmax - mid) / pen_e) hi = mid; else lo = mid + 1;
     }
-    /* no pair of the batch can score more than substitutions all along the shorter sequence plus one
-     * gap for the length difference: a generous -e (or a stale hint) does not widen the rings */
-    int d_reach = d_full;                    /* scores beyond this cannot occur in this batch */
+    long long best = 1;
+    for (int dd = std::max(0, lo - 2); dd < std::min(d_end, lo + 3); ++dd)
+        best = std::max(best, std::min<long long>(tab[dd].n, ktm + (Dmax - dd) / pen_e));
+    return (int)best;
+}
+
+/* Stage 1: the full budget, or (first pass only) what recent batches with these penalties needed plus a margin -- pairs
+ * that outgrow it are re-dispatched.  No pair of the batch can score more than substitutions all along the shorter
+ * sequence plus one gap for the length difference: a generous -e (or a stale hint) does not widen the rings. */
+static Scores provision_scores(const wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan, bool first_pass)
+{
+    Scores sc;
+    sc.d_full = s.tab_d_end;
+    sc.d_want = sc.d_full;
+    if (first_pass && hint_applies(d, s, plan)) {
+        sc.d_want = (int)std::min<long long>(hint_plus(d, d->hint_margin_pm, 8), sc.d_full - 1) + 1;
+        sc.hinted = sc.d_want < sc.d_full;
+    }
+    sc.d_reach = sc.d_full;
     if (plan.band <= 0) {
         long long cap = (long long)plan.x * s.minlen_max + plan.o + (long long)plan.e * s.kt_max + 2;
-        if (p2) cap = std::min(cap, (long long)plan.x * s.minlen_max + plan.o2 + (long long)plan.e2 * s.kt_max + 2);   /* the cheaper piece */
-        if (cap < d_reach) d_reach = (int)std::max<long long>(cap, 2);
-        if (d_reach < d_want) d_want = d_reach;
+        if (plan.e2 > 0) cap = std::min(cap, (long long)plan.x * s.minlen_max + plan.o2 + (long long)plan.e2 * s.kt_max + 2);   /* the cheaper piece */
+        if (cap < sc.d_reach) sc.d_reach = (int)std::max<long long>(cap, 2);
+        if (sc.d_reach < sc.d_want) sc.d_want = sc.d_reach;
     }
-    /* Packed exact first pass where the per-pair score bounds pay (long reads): the bound kernel runs first and its
-     * largest bound sizes the rings -- what this batch needs, not what the last one needed, so a first call, a call
-     * without hints and a call after a batch of another kind all run at the speed of a well-hinted one.  Costs one
-     * host round trip per pass (bounds back: 4 bytes per pair). */
-    int d_p99 = 0;                           /* 99 % of the bounded pairs finish below this score (0 = unknown) */
-    size_t n_seed = 0;                       /* pairs at the end of the order list that skip this pass (no bound within the budget) */
-    if (first_pass && !have_bounds && plan.band <= 0 && !ascii && !p2 && !d->no_bound && !d->no_prebound && n_items == s.n &&
-        bound_max_ctas_per_sm(std::max(plan.o + plan.e, plan.x) + 1, plan.e + 1, 8) >= 1) {   /* penalties whose rings fit the bound kernel */
-        bool pays = d->force_bound;
-        if (!pays) {
-            const bool h = d_want < d_full && d->hint_mean > 0 && d->hint_dist > 0;
-            const double m = h ? d->hint_mean : 0.5 * (d_want - 1);
-            const double r = std::min(2.0, std::max(1.0, (d_want - 1) / std::max(1.0, m)));
-            const double cells = r * r / 4 + (1.5 * r - 1) * (1 - r / 2);
-            pays = (cells - 0.5) * m > 130.0;
+    return sc;
+}
+
+/* Stage 2, the first pass of a packed exact batch where the per-pair score bounds pay (long reads): the bound kernel runs
+ * first and its largest bound sizes the rings -- what this batch needs, not what the last one needed, so a first call, a
+ * call without hints and a call after a batch of another kind all run at the speed of a well-hinted one.  Costs one host
+ * round trip per pass (bounds back: 4 bytes per pair); the only stage that waits for the GPU. */
+static int bound_prepass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, PassRequest &r, Scores &sc)
+{
+    if (!r.first_pass || r.have_bounds || plan.band > 0 || r.ascii || plan.e2 > 0 || d->no_bound || d->no_prebound ||
+        r.n_items != s.n || bound_max_ctas_per_sm(ring_depths(plan).A, plan.e + 1, 8) < 1)   /* penalties whose rings fit the bound kernel */
+        return 0;
+    const int d_full = sc.d_full;
+    bool pays = d->force_bound ||
+                bound_pays(sc.d_want, (sc.d_want < d_full && d->hint_mean > 0 && d->hint_dist > 0) ? d->hint_mean : 0);
+    if (!pays && sc.d_want < d_full && d->hint_dist > 0 && s.max_len >= 2000 && r.n_items >= 1024 && r.order == s.order.p) {
+        /* a hint tight enough that bounding every pair does not pay: is it still true for this batch?  Bound the first
+         * 128 pairs of the queue; if they already outgrow the hint (every pair would be re-dispatched) or stay far
+         * below it (rings wider than needed), provision from this batch's own bounds after all */
+        constexpr size_t kSample = 128;
+        if (int rc = bounds_to_host(d, s, plan, r.max_steps, r.order, kSample)) return rc;
+        CK(cudaStreamSynchronize(s.stream));
+        long long smax = 0;
+        for (size_t i = 0; i < kSample; ++i) {
+            const uint32_t idx = s.h_order.p[i];
+            if (idx < s.n) smax = std::max<long long>(smax, std::min<int32_t>(s.h_bound.p[idx], d_full));
         }
-        if (!pays && d_want < d_full && d->hint_dist > 0 && s.max_len >= 2000 && n_items >= 1024 && order_dev == s.order.p) {
-            /* a hint tight enough that bounding every pair does not pay: is it still true for this batch?  Bound the first
-             * 128 pairs of the queue; if they already outgrow the hint (every pair would be re-dispatched) or stay far
-             * below it (rings wider than needed), provision from this batch's own bounds after all */
-            constexpr size_t kSample = 128;
-            int rcb = run_bound_only(d, s, plan, max_steps, order_dev, kSample);
-            if (rcb) return rcb;
-            if (s.h_bound.ensure(s.n + 1)) return -1;
-            CK(cudaMemcpyAsync(s.h_bound.p, s.bound.p, s.n * sizeof(int32_t), cudaMemcpyDeviceToHost, s.stream));
-            CK(cudaStreamSynchronize(s.stream));
-            long long smax = 0;
-            for (size_t i = 0; i < kSample; ++i) {
-                const uint32_t idx = s.h_order.p[i];
-                if (idx < s.n) smax = std::max<long long>(smax, std::min<int32_t>(s.h_bound.p[idx], d_full));
-            }
-            const long long covered = (long long)d->hint_dist + (long long)d->hint_dist * d->hint_min_pm / 1000;
-            pays = smax > covered || smax * 13 < (long long)d->hint_dist * 10;
-        }
-        if (pays) {
-            int rcb = run_bound_only(d, s, plan, max_steps, order_dev, n_items);
-            if (rcb) return rcb;
-            if (s.h_bound.ensure(s.n + 1)) return -1;
-            CK(cudaMemcpyAsync(s.h_bound.p, s.bound.p, s.n * sizeof(int32_t), cudaMemcpyDeviceToHost, s.stream));
-            CK(cudaStreamSynchronize(s.stream));
-            std::vector<int32_t> &bv = s.bound_sorted;
-            bv.clear();
-            for (size_t i = 0; i < s.n; ++i)
-                if (s.h_bound.p[i] < d_full - 1) bv.push_back(s.h_bound.p[i]);
-            have_bounds = true;
-            if (order_dev == s.order.p && !d->no_bound_order) {
-                /* longest first by the pair's own bound (work ~ bound^2): the queue's tail is made of the cheapest pairs
-                 * (counting sort, descending).  Pairs the bound pass could not bound within this budget go to the end of
-                 * the list and straight to the re-dispatch tier: their first pass would run to the end of the budget for
-                 * nothing (a pair flagged for the byte-compare kernel stays: the wavefront kernel routes it).
-                 * The order list was uploaded before the sync. */
-                std::vector<uint32_t> &cnt = s.bound_count;
-                cnt.assign((size_t)d_full + 2, 0u);
-                auto key_of = [&](int32_t b) -> size_t {
-                    if (b == 0x7fffffff) return (size_t)d_full;              /* flagged: first */
-                    if (b >= d_full - 1) return (size_t)d_full + 1;          /* open: last (descending order below) */
-                    return (size_t)std::max(b, 0);
-                };
-                size_t n_open = 0;
-                for (size_t i = 0; i < s.n; ++i) {
-                    const size_t k = key_of(s.h_bound.p[i]);
-                    cnt[k] += 1;
-                    n_open += (k == (size_t)d_full + 1);
-                }
-                uint32_t acc = 0;
-                for (int b = d_full; b >= 0; --b) { const uint32_t c0 = cnt[(size_t)b]; cnt[(size_t)b] = acc; acc += c0; }
-                cnt[(size_t)d_full + 1] = acc;
-                for (size_t i = 0; i < s.n; ++i) s.h_order.p[cnt[key_of(s.h_bound.p[i])]++] = (uint32_t)i;
-                CK(cudaMemcpyAsync(s.order.p, s.h_order.p, s.n * sizeof(uint32_t), cudaMemcpyHostToDevice, s.stream));
-                if (n_open > 0 && !d->no_skip_open) {
-                    n_seed = n_open;
-                    n_items = s.n - n_open;
-                }
-            }
-            if (!bv.empty()) {
-                const size_t k99 = (bv.size() - 1) - (bv.size() - 1) / 100;
-                std::nth_element(bv.begin(), bv.begin() + (long)k99, bv.end());
-                const int b99 = bv[k99];
-                const int bmax = *std::max_element(bv.begin() + (long)k99, bv.end());
-                d_want = std::min(d_full, bmax + 2);
-                d_want = std::min(d_want, d_reach);
-                d_p99 = std::min(d_want, b99 + 2);
-                hinted = false;
-            }
-        }
+        const long long covered = hint_plus(d, d->hint_min_pm, 0);
+        pays = smax > covered || smax * 13 < (long long)d->hint_dist * 10;
     }
-    const int pen_e = p2 ? std::min(plan.e, plan.e2) : plan.e;     /* 2-piece: the pruning's min(e1, e2) */
-    const long long kt_max = s.kt_max;
-    auto n_need = [&](int d_end) -> int {
-        /* n_d grows, kt + (Dmax - d) / e shrinks: the largest min sits where they cross.  A global pair with |kt| > Dmax / e
-         * cannot finish; an ends-free one can (the start row and the target range may meet at no cost), and its window
-         * reaches max(pe, te) beyond kt: no clamp, n_d bounds it */
-        const long long Dmax = d_end - 1;
-        const long long ktm = s.ef ? kt_max + s.ef_ext : std::min<long long>(kt_max, Dmax / pen_e);
-        int lo = 0, hi = d_end;                      /* first d with n_d >= ktm + (Dmax - d) / e */
-        while (lo < hi) {
-            const int mid = (lo + hi) / 2;
-            if ((long long)tab[mid].n >= ktm + (Dmax - mid) / pen_e) hi = mid; else lo = mid + 1;
-        }
-        long long best = 1;
-        for (int dd = std::max(0, lo - 2); dd < std::min(d_end, lo + 3); ++dd)
-            best = std::max(best, std::min<long long>(tab[dd].n, ktm + (Dmax - dd) / pen_e));
-        return (int)best;
-    };
-    int n_want = plan.band > 0 ? n_full : n_need(d_want);
-    /* with a hint, rings for hint + 3 % are enough for (almost) every pair */
-    int n_min = n_want;
-    if (hinted && plan.band <= 0)
-        n_min = std::min(n_want, n_need((int)std::min<long long>((long long)d->hint_dist + (long long)d->hint_dist * d->hint_min_pm / 1000 + 4, d_full - 1) + 1));
-    if (d_p99 > 0) n_min = std::min(n_want, n_need(d_p99));      /* rings for 99 % of the pairs when that buys a resident CTA */
-    const bool banded = plan.band > 0;
-    LaunchCfg c{};
-    int rc = 0;
-    int win = 0;
-    if (banded) {
-        /* adaptive band: window = the reference's threads_per_block (lib/sequence_alignment.cu:270-277) */
-        win = plan.band_width > 0 ? plan.band_width : 512;
-        c.A = std::max(plan.o + plan.e, plan.x) + 1; c.E1 = plan.e + 1; c.G = c.A;
-        c.seq_words = (int)packed_words_for(s.max_len);
-        c.groups_per_cta = 1;
-        /* a few diagonals per thread: the per-score overhead (window bookkeeping, barrier) is paid
-         * per thread, and small CTAs let more pairs share an SM (measured on B200, W = 512:
-         * 512 threads 114 k, 256 threads 165 k, 128 threads 189 k pairs/s at 10 kbp / 5 %) */
-        c.group_threads = std::min(1024, std::max(64, ((win / 4) + 31) & ~31));
-        /* packed pairs: four diagonals per thread (wfa_bandq_kernel), one quad per thread and score */
-        c.quad = !ascii && !d->no_quad;
-        /* a window spans win / 4 + 1 quads: two trips of half of them (measured on B200, W = 512, 10 kbp / 5 %:
-         * 64 threads 32.5 ms, 96 threads 31.4 ms, 128 threads 33.0 ms per 8192 pairs end to end) */
-        if (c.quad) c.group_threads = std::min(512, std::max(64, (((win / 4 + 2) / 2) + 31) & ~31));
-        if (d->force_threads) c.group_threads = d->force_threads;
-        auto band_smem = [&](int stages) {
-            return c.quad ? bandq_smem_bytes(c.A, win, c.seq_words, stages) : banded_smem_bytes(c.A, win, c.seq_words, stages);
+    if (!pays) return 0;
+    if (int rc = bounds_to_host(d, s, plan, r.max_steps, r.order, r.n_items)) return rc;
+    CK(cudaStreamSynchronize(s.stream));
+    std::vector<int32_t> &bv = s.bound_sorted;
+    bv.clear();
+    for (size_t i = 0; i < s.n; ++i)
+        if (s.h_bound.p[i] < d_full - 1) bv.push_back(s.h_bound.p[i]);
+    r.have_bounds = true;
+    if (r.order == s.order.p && !d->no_bound_order) {
+        /* longest first by the pair's own bound (work ~ bound^2): the queue's tail is made of the cheapest pairs
+         * (counting sort, descending).  Pairs the bound pass could not bound within this budget go to the end of
+         * the list and straight to the re-dispatch tier: their first pass would run to the end of the budget for
+         * nothing (a pair flagged for the byte-compare kernel stays: the wavefront kernel routes it).
+         * The order list was uploaded before the sync. */
+        std::vector<uint32_t> &cnt = s.bound_count;
+        cnt.assign((size_t)d_full + 2, 0u);
+        auto key_of = [&](int32_t b) -> size_t {
+            if (b == 0x7fffffff) return (size_t)d_full;              /* flagged: first */
+            if (b >= d_full - 1) return (size_t)d_full + 1;          /* open: last (descending order below) */
+            return (size_t)std::max(b, 0);
         };
-        c.stages = 2;
-        c.smem = band_smem(c.stages);
-        if (c.smem > d->prop.sharedMemPerBlockOptin) {
-            c.stages = 1;
-            c.smem = band_smem(c.stages);
+        size_t n_open = 0;
+        for (size_t i = 0; i < s.n; ++i) {
+            const size_t k = key_of(s.h_bound.p[i]);
+            cnt[k] += 1;
+            n_open += (k == (size_t)d_full + 1);
         }
-        if (c.smem > d->prop.sharedMemPerBlockOptin) {
-            fprintf(stderr, "[wfagpu] band of %d diagonals does not fit in shared memory\n", win);
-            return -2;
+        uint32_t acc = 0;
+        for (int b = d_full; b >= 0; --b) { const uint32_t c0 = cnt[(size_t)b]; cnt[(size_t)b] = acc; acc += c0; }
+        cnt[(size_t)d_full + 1] = acc;
+        for (size_t i = 0; i < s.n; ++i) s.h_order.p[cnt[key_of(s.h_bound.p[i])]++] = (uint32_t)i;
+        CK(cudaMemcpyAsync(s.order.p, s.h_order.p, s.n * sizeof(uint32_t), cudaMemcpyHostToDevice, s.stream));
+        if (n_open > 0 && !d->no_skip_open) {
+            r.n_seed = n_open;
+            r.n_items = s.n - n_open;
         }
-        c.n_cap = n_full; c.row_stride = win; c.center = 0;
-        int occ = c.quad ? bandq_max_ctas_per_sm(c.group_threads, c.smem, plan.with_cigar != 0)
-                         : banded_max_ctas_per_sm(c.group_threads, c.smem, ascii, plan.with_cigar != 0);
-        if (occ < 1) return -1;
-        c.ctas = (int)std::max<size_t>(1, std::min<size_t>((size_t)occ * d->prop.multiProcessorCount, n_items));
-    } else {
-        rc = choose_cfg(d, plan.x, plan.o, plan.e, n_want, n_min, s.max_len, n_items, ascii, plan.with_cigar != 0, s.ef,
-                        p2 ? plan.o2 : 0, p2 ? plan.e2 : 0, &c);
     }
-    if (rc) return rc;
-    tr.mark("cfg");
+    if (!bv.empty()) {
+        const size_t k99 = (bv.size() - 1) - (bv.size() - 1) / 100;
+        std::nth_element(bv.begin(), bv.begin() + (long)k99, bv.end());
+        const int b99 = bv[k99];
+        const int bmax = *std::max_element(bv.begin() + (long)k99, bv.end());
+        sc.d_want = std::min(d_full, bmax + 2);
+        sc.d_want = std::min(sc.d_want, sc.d_reach);
+        sc.d_p99 = std::min(sc.d_want, b99 + 2);
+        sc.hinted = false;
+    }
+    return 0;
+}
+
+/* What a launch computes and where its backtrace state goes. */
+struct Arenas {
+    int d_end = 0;                /* scores 1 .. d_end - 1 may be computed */
+    int period = 0;               /* ring-snapshot period (0: no snapshots) */
+    bool band_tb = false;         /* adaptive band on packed pairs: decision rows walked by a traceback kernel after the launch */
+    uint64_t arena_units = 0;     /* uint4 units per arena */
+    size_t arenas = 0;            /* snapshots, band_tb: one per pair of a sub-launch; else one per resident group */
+    size_t items_per_launch = 0;
+    uint64_t gring_elems = 0;     /* large tier: ring elements per group */
+    uint32_t scratch_words = 0, band_lo_words = 0;
+};
+
+/* Stage 4: the scores the launch can reach, the snapshot period, the arenas within a third of the free device memory, and
+ * every buffer the launch writes. */
+static int size_arenas(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, const PassRequest &r, const Scores &sc,
+                       LaunchCfg &c, Arenas &a, HostTrace &tr)
+{
+    const bool banded = plan.band > 0;
+    const size_t n_items = r.n_items;
     /* scores this launch can reach and the decision units they need */
-    int d_end = banded ? d_full : d_want;
+    a.d_end = banded ? sc.d_full : sc.d_want;
     uint64_t arena_units = s.tab_arena_units;
     if (!banded) {
-        if (c.n_cap < n_want) {
-            int lo = 1, hi = d_want;                 /* largest d_end whose pruned wavefronts fit the rings */
+        if (c.n_cap < sc.n_want) {
+            int lo = 1, hi = sc.d_want;              /* largest d_end whose pruned wavefronts fit the rings */
             while (lo < hi) {
                 const int mid = (lo + hi + 1) / 2;
-                if (n_need(mid) <= c.n_cap) lo = mid; else hi = mid - 1;
+                if (n_need(s, plan, mid) <= c.n_cap) lo = mid; else hi = mid - 1;
             }
-            d_end = lo;
+            a.d_end = lo;
         }
-        arena_units = d_end < d_full ? tab[d_end].row_off : s.tab_arena_units;
+        arena_units = a.d_end < sc.d_full ? s.h_steps.p[a.d_end].row_off : s.tab_arena_units;
     }
-    *capped_out = d_end < d_reach;          /* provisioned below what the budget (and the lengths) allow */
 
-    /* memory budget of the arenas: a third of the free device memory */
-    size_t arena_budget = 0;
-    {
-        /* cudaMemGetInfo takes 0.2 - 15 ms on a busy box and would leave the GPU idle between the pack
-         * kernel and this pass: ask only when the answer can have changed (first use, arena grew) */
-        if (d->arena_mb > 0) {
-            s.budget_cache = (size_t)d->arena_mb << 20;          /* WFAGPU_ARENA_MB: fixed budget (tests) */
-        } else if (s.budget_cache == 0) {
-            size_t free_b = 0, total_b = 0;
-            cudaMemGetInfo(&free_b, &total_b);
-            s.budget_cache = std::max<size_t>((free_b + s.arena.cap * sizeof(uint4)) / 3, (size_t)64 << 20);
-        }
-        arena_budget = s.budget_cache;
+    /* memory budget of the arenas: a third of the free device memory.  cudaMemGetInfo takes 0.2 - 15 ms on a busy box and
+     * would leave the GPU idle between the pack kernel and this pass: ask only when the answer can have changed (first use,
+     * arena grew) */
+    if (d->arena_mb > 0) {
+        s.budget_cache = (size_t)d->arena_mb << 20;          /* WFAGPU_ARENA_MB: fixed budget (tests) */
+    } else if (s.budget_cache == 0) {
+        size_t free_b = 0, total_b = 0;
+        cudaMemGetInfo(&free_b, &total_b);
+        s.budget_cache = std::max<size_t>((free_b + s.arena.cap * sizeof(uint4)) / 3, (size_t)64 << 20);
     }
+    size_t arena_budget = s.budget_cache;
     tr.mark("meminfo");
-    int period = 0;
-    if (c.ckpt) {
+    if (c.k.ckpt) {
         /* Snapshot period: the traceback recomputes ~ score * P cells per pair against ~ score^2 in
          * the forward pass, the snapshots take ~ 1/P of the cells: short periods for low scores,
          * longer ones when memory is tight. */
-        const int d_expect = hinted ? std::min(d_end, d->hint_dist + 1) : d_end;
-        period = d->force_period ? d->force_period : (d_expect >= 3000 ? 31 : 15);   /* measured on B200: shorter never wins */
+        const int d_expect = sc.hinted ? std::min(a.d_end, d->hint_dist + 1) : a.d_end;
+        int period = d->force_period ? d->force_period : (d_expect >= 3000 ? 31 : 15);   /* measured on B200: shorter never wins */
         for (;;) {
             if (ensure_ck_table(s, plan, period)) return -1;
-            arena_units = s.h_ck_off[(size_t)(d_end - 1) / period + 1];      /* snapshots of scores j * P < d_end */
+            arena_units = s.h_ck_off[(size_t)(a.d_end - 1) / period + 1];      /* snapshots of scores j * P < d_end */
             if (period >= 31 || d->force_period || (arena_units * sizeof(uint4) + 1) * n_items <= arena_budget) break;
             period = 2 * period + 1;
         }
         if (arena_units >= 0xffffffffull) { fprintf(stderr, "[wfagpu] snapshot arena exceeds 32-bit offsets\n"); return -1; }
+        a.period = period;
     }
 
     if (!plan.with_cigar) arena_units = 0;
+    a.arena_units = arena_units;
     /* adaptive band on packed pairs: decision rows per pair, walked by a traceback kernel after the launch */
-    const bool band_tb = banded && c.quad && plan.with_cigar && !d->no_band_tb;
+    a.band_tb = banded && c.k.quad() && plan.with_cigar && !d->no_band_tb;
+    const bool per_pair = c.k.ckpt || a.band_tb;
     /* keep the arenas within a third of the free device memory: fewer, not smaller, groups
      * (decision bytes: one arena per resident group; snapshots: one per pair of a sub-launch) */
-    size_t items_per_launch = n_items;
+    a.items_per_launch = n_items;
     for (int attempt = 0;; ++attempt) {
         const size_t budget = arena_budget;
-        if (c.ckpt || band_tb) {
-            const size_t per_pair = (size_t)arena_units * sizeof(uint4) + (band_tb ? ((size_t)d_end + 1) * sizeof(int32_t) : 0) + 1;
-            items_per_launch = std::max<size_t>(1, std::min<size_t>(n_items, budget / per_pair));
-            c.ctas = (int)std::min<size_t>((size_t)c.ctas, items_per_launch);
+        if (per_pair) {
+            const size_t per_item = (size_t)arena_units * sizeof(uint4) + (a.band_tb ? ((size_t)a.d_end + 1) * sizeof(int32_t) : 0) + 1;
+            a.items_per_launch = std::max<size_t>(1, std::min<size_t>(n_items, budget / per_item));
+            c.ctas = (int)std::min<size_t>((size_t)c.ctas, a.items_per_launch);
         } else {
             const size_t per_group = (size_t)arena_units * sizeof(uint4) * (size_t)c.groups_per_cta + 1;
             const size_t max_ctas = std::max<size_t>(1, budget / per_group);
@@ -1005,7 +1069,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         }
         /* an arena that has to grow is checked against the memory that is free right now (the budget may date from an
          * emptier device: other slots, contexts and processes allocate too); the old arena is given back first */
-        const size_t want = (((c.ckpt || band_tb) ? items_per_launch : (size_t)c.ctas * c.groups_per_cta) * arena_units + 1);
+        const size_t want = ((per_pair ? a.items_per_launch : (size_t)c.ctas * c.groups_per_cta) * arena_units + 1);
         if (want <= s.arena.cap || d->arena_mb > 0 || attempt >= 4) break;
         size_t free_b = 0, total_b = 0;
         if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); break; }
@@ -1016,31 +1080,39 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         s.budget_cache = arena_budget;
     }
     const size_t groups = (size_t)c.ctas * c.groups_per_cta;
-    const uint64_t gring_elems = c.global_ring ? (uint64_t)(c.A + 2 * c.E1 + 2 * c.E2) * (uint64_t)c.row_stride : 0;
-    if (s.gring.ensure(groups * gring_elems + 1)) return -1;
-    const uint32_t scratch_words = plan.with_cigar ? (uint32_t)((2 * (size_t)d_end + 31) / 16 + 2) : 1;
-    const size_t arenas = (c.ckpt || band_tb) ? items_per_launch : groups;
-    if (arenas * arena_units + 1 > s.arena.cap) s.budget_cache = 0;      /* the arena grows: re-read the free memory next time */
-    if (s.arena.ensure(arenas * arena_units + 1) || s.scratch.ensure(groups * scratch_words + 1)) return -1;
-    const uint32_t band_lo_words = (banded && plan.with_cigar) ? (uint32_t)d_end + 1 : 0;
-    if (s.band_lo.ensure((band_tb ? items_per_launch : groups) * (size_t)band_lo_words + 1)) return -1;
+    a.gring_elems = c.k.gring ? (uint64_t)(c.A + 2 * c.E1 + 2 * c.E2) * (uint64_t)c.row_stride : 0;
+    if (s.gring.ensure(groups * a.gring_elems + 1)) return -1;
+    a.scratch_words = plan.with_cigar ? (uint32_t)((2 * (size_t)a.d_end + 31) / 16 + 2) : 1;
+    a.arenas = per_pair ? a.items_per_launch : groups;
+    if (a.arenas * arena_units + 1 > s.arena.cap) s.budget_cache = 0;      /* the arena grows: re-read the free memory next time */
+    if (s.arena.ensure(a.arenas * arena_units + 1) || s.scratch.ensure(groups * a.scratch_words + 1)) return -1;
+    a.band_lo_words = (banded && plan.with_cigar) ? (uint32_t)a.d_end + 1 : 0;
+    if (s.band_lo.ensure((a.band_tb ? a.items_per_launch : groups) * (size_t)a.band_lo_words + 1)) return -1;
     /* op pool: worst case for this pass on top of what is already used */
     /* later passes run after read_counters(): the host copy of the pool head is current */
-    const uint32_t pool_used = first_pass ? 0u : s.h_counters.p[CTR_POOL];
-    const size_t pool_need = (size_t)pool_used + (plan.with_cigar ? n_items * (size_t)scratch_words : 0) + 16;
+    const uint32_t pool_used = r.first_pass ? 0u : s.h_counters.p[CTR_POOL];
+    const size_t pool_need = (size_t)pool_used + (plan.with_cigar ? n_items * (size_t)a.scratch_words : 0) + 16;
     if (pool_need >= (1ull << 32)) {
         fprintf(stderr, "[wfagpu] op pool exceeds 32-bit offsets; use a smaller batch_size\n");
         return -1;
     }
     if (s.pool.ensure(pool_need, true, s.stream)) return -1;
-
     tr.mark("buffers");
-    if (n_seed > 0) {
+    return 0;
+}
+
+/* Stage 5: the retry list's seed, the kernel parameters, and the sub-launches (bound, wavefront and traceback kernels). */
+static int enqueue_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, const PassRequest &r, const Scores &sc,
+                        const LaunchCfg &c, const Arenas &a, HostTrace &tr)
+{
+    const bool banded = plan.band > 0;
+    const size_t n_items = r.n_items;
+    if (r.n_seed > 0) {
         /* the re-dispatch list starts with the pairs that skip this pass */
         if (s.h_seed.ensure(1)) return -1;
-        s.h_seed.p[0] = (uint32_t)n_seed;
+        s.h_seed.p[0] = (uint32_t)r.n_seed;
         CK(cudaMemcpyAsync(s.counters.p + CTR_RETRY, s.h_seed.p, sizeof(uint32_t), cudaMemcpyHostToDevice, s.stream));
-        CK(cudaMemcpyAsync(retry_dev, s.order.p + n_items, n_seed * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s.stream));
+        CK(cudaMemcpyAsync(r.retry, s.order.p + n_items, r.n_seed * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s.stream));
     } else {
         CK(cudaMemsetAsync(s.counters.p + CTR_RETRY, 0, sizeof(uint32_t), s.stream));
     }
@@ -1049,29 +1121,19 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
     kp.packed = s.packed.p;
     kp.ascii = s.ascii.p;
     kp.pairs = s.pairs.p;
-    kp.order = order_dev;
+    kp.order = r.order;
     kp.n_items = (uint32_t)n_items;
     kp.queue = s.counters.p + CTR_QUEUE;
     kp.tb_queue = s.counters.p + CTR_TBQ;
     kp.bound_queue = s.counters.p + CTR_BQ;
-    /* per-pair bounds: first pass of the packed exact path only (a re-dispatched pair never
-     * depends on them) */
-    /* have_bounds: s.bound already holds this pass's bounds (run_bound_only) */
-    bool use_bound = !banded && !ascii && !p2 && (first_pass || have_bounds) && !d->no_bound;
-    if (use_bound && !d->force_bound && !have_bounds) {
-        /* Worth it?  With D = d_end - 1 and a typical score m, the launch bound leaves
-         * cells(D/m) * m^2 cells per pair (cells(r) = r^2/4 + (1.5r - 1)(1 - r/2), 1 from r = 2 on), the
-         * pair's own bound 0.5 * m^2; the bound pass costs ~32 cells per score at ~3x the cost per
-         * cell (measured on B200: ~240 against ~2.75 warp instructions). */
-        const double m = (hinted && d->hint_mean > 0) ? d->hint_mean : 0.5 * (d_end - 1);
-        const double r = std::min(2.0, std::max(1.0, (d_end - 1) / std::max(1.0, m)));
-        const double cells = r * r / 4 + (1.5 * r - 1) * (1 - r / 2);
-        use_bound = (cells - 0.5) * m > 130.0;
-    }
+    /* per-pair bounds: first pass of the packed exact path only (a re-dispatched pair never depends on them), or the
+     * bounds s.bound already holds (bounds_to_host) */
+    bool use_bound = !banded && !r.ascii && plan.e2 <= 0 && (r.first_pass || r.have_bounds) && !d->no_bound;
+    if (use_bound && !d->force_bound && !r.have_bounds) use_bound = bound_pays(a.d_end, sc.hinted ? d->hint_mean : 0);
     if (use_bound && s.bound.ensure(s.n + 1)) return -1;
     kp.bound = use_bound ? s.bound.p : nullptr;
     kp.steps = s.steps.p;
-    kp.d_end = d_end;
+    kp.d_end = a.d_end;
     kp.n_cap = c.n_cap;
     kp.x = plan.x; kp.o = plan.o; kp.e = plan.e;
     kp.A = c.A; kp.E1 = c.E1; kp.G = c.G;
@@ -1083,23 +1145,23 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
     kp.quad_pairs = c.quad_pairs ? 1 : 0;
     kp.ring_m = c.ring_m; kp.ring_g = c.ring_g;
     kp.band = plan.band;
-    kp.win = win;
+    kp.win = c.win;
     kp.band_lo = s.band_lo.p;
-    kp.band_lo_words = band_lo_words;
-    kp.band_tb = band_tb ? 1 : 0;
-    kp.gring = c.global_ring ? s.gring.p : nullptr;
-    kp.gring_elems = gring_elems;
+    kp.band_lo_words = a.band_lo_words;
+    kp.band_tb = a.band_tb ? 1 : 0;
+    kp.gring = c.k.gring ? s.gring.p : nullptr;
+    kp.gring_elems = a.gring_elems;
     kp.arena = s.arena.p;
-    kp.arena_units = arena_units;
-    kp.ck_off = c.ckpt ? s.ck_off.p : nullptr;
-    kp.ck_period = period;
+    kp.arena_units = a.arena_units;
+    kp.ck_off = c.k.ckpt ? s.ck_off.p : nullptr;
+    kp.ck_period = a.period;
     kp.ops_scratch = s.scratch.p;
-    kp.ops_scratch_words = scratch_words;
+    kp.ops_scratch_words = a.scratch_words;
     kp.ops_pool = s.pool.p;
     kp.ops_pool_head = s.counters.p + CTR_POOL;
     kp.ops_pool_words = (uint32_t)std::min<size_t>(s.pool.cap, 0xffffffffu);
     kp.out = s.out.p;
-    kp.retry_list = retry_dev;
+    kp.retry_list = r.retry;
     kp.retry_count = s.counters.p + CTR_RETRY;
     kp.ascii_list = s.ascii_list.p;
     kp.ascii_count = s.counters.p + CTR_ASCII;
@@ -1109,30 +1171,33 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         kp.ef_tb = s.span.text_begin_free; kp.ef_te = s.span.text_end_free;
         kp.ends = s.ends.p;
     }
-    if (p2) { kp.o2 = plan.o2; kp.e2 = plan.e2; kp.E2 = c.E2; }
-    if (env_int("WFAGPU_VERBOSE", 0))
+    if (plan.e2 > 0) { kp.o2 = plan.o2; kp.e2 = plan.e2; kp.E2 = c.E2; }
+    if (env_int("WFAGPU_VERBOSE", 0)) {
+        const bool quad = c.k.quad(), ckpt = c.k.ckpt;
         fprintf(stderr, "[wfagpu] pass: items=%zu max_steps=%d n_cap=%d d_end=%d group=%d x%d ctas=%d stages=%d smem=%zu ascii=%d band=%d tier=%s period=%d arena=%.1f MB\n",
-                n_items, max_steps, c.n_cap, d_end, c.group_threads, c.groups_per_cta, c.ctas, c.stages, c.smem,
-                (int)ascii, plan.band > 0 ? win : 0, c.global_ring ? (c.quad ? "global-int32x4" : "global-int32") : (c.quad ? (c.quad_pairs ? (c.ckpt ? "smem-int16x4x2+ckpt" : "smem-int16x4x2") : (c.ckpt ? "smem-int16x4+ckpt" : "smem-int16x4")) : (c.ckpt ? "smem-int16+ckpt" : "smem-int16")), period, arenas * arena_units * 16.0 / 1e6);
+                n_items, r.max_steps, c.n_cap, a.d_end, c.group_threads, c.groups_per_cta, c.ctas, c.stages, c.smem,
+                (int)r.ascii, c.win, c.k.gring ? (quad ? "global-int32x4" : "global-int32") : (quad ? (c.quad_pairs ? (ckpt ? "smem-int16x4x2+ckpt" : "smem-int16x4x2") : (ckpt ? "smem-int16x4+ckpt" : "smem-int16x4")) : (ckpt ? "smem-int16+ckpt" : "smem-int16")), a.period, a.arenas * a.arena_units * 16.0 / 1e6);
+    }
     int tb_ctas = 0;
     constexpr int kTbWarps = 8;
-    if (c.ckpt) {
-        const int occ = traceback_max_ctas_per_sm(c.A, period, kTbWarps, ascii);
+    if (c.k.ckpt) {
+        const int occ = traceback_max_ctas_per_sm(c.A, a.period, kTbWarps, r.ascii);
         if (occ < 1) { fprintf(stderr, "[wfagpu] traceback kernel does not fit\n"); return -1; }
         tb_ctas = occ * d->prop.multiProcessorCount;
     }
     int bound_ctas = 0;
     constexpr int kBoundWarps = 8;
-    if (use_bound && !have_bounds) {
+    if (use_bound && !r.have_bounds) {
         const int occ = bound_max_ctas_per_sm(c.A, c.E1, kBoundWarps);
         if (occ < 1) kp.bound = nullptr; else bound_ctas = occ * d->prop.multiProcessorCount;
     }
+    const kernel_fn wavefront = wavefront_kernel(c.k, d->count_cells);
     tr.mark("occ");
-    for (size_t off = 0; off < n_items; off += items_per_launch) {
-        const size_t cnt = std::min(items_per_launch, n_items - off);
-        kp.order = order_dev + off;
+    for (size_t off = 0; off < n_items; off += a.items_per_launch) {
+        const size_t cnt = std::min(a.items_per_launch, n_items - off);
+        kp.order = r.order + off;
         kp.n_items = (uint32_t)cnt;
-        if (kp.bound && !have_bounds) {
+        if (kp.bound && !r.have_bounds) {
             CK(cudaMemsetAsync(s.counters.p + CTR_BQ, 0, sizeof(uint32_t), s.stream));
             const int ctas = (int)std::min<size_t>((size_t)bound_ctas, (cnt + kBoundWarps - 1) / kBoundWarps);
             cudaError_t eb = launch_bound(kp, ctas, kBoundWarps, s.stream);
@@ -1143,13 +1208,11 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
             s.stats.launches += 1;
         }
         CK(cudaMemsetAsync(s.counters.p + CTR_QUEUE, 0, sizeof(uint32_t), s.stream));
-        const bool time_it = first_pass && items_per_launch >= n_items && s.ev[6] && s.ev[7];
+        const bool time_it = r.first_pass && a.items_per_launch >= n_items && s.ev[6] && s.ev[7];
         if (time_it) CK(cudaEventRecord(s.ev[6], s.stream));
-        cudaError_t e = (banded && c.quad) ? launch_bandq(kp, c.group_threads, c.ctas, c.smem, s.stream)
-                      : banded ? launch_banded(kp, c.group_threads, c.ctas, c.smem, ascii, s.stream)
-                      : (c.quad && c.global_ring) ? launch_quadg(kp, c.group_threads, (int)std::min<size_t>(c.ctas, cnt), c.smem, s.stream)
-                      : c.quad ? launch_quad(kp, c.group_threads, (int)std::min<size_t>(c.ctas, cnt), c.smem, s.stream)
-                               : launch_exact(kp, c.group_threads, c.groups_per_cta, (int)std::min<size_t>(c.ctas, cnt), c.smem, ascii, s.stream);
+        /* the banded kernels always launch the full shape */
+        const int ctas = banded ? c.ctas : (int)std::min<size_t>(c.ctas, cnt);
+        cudaError_t e = launch(wavefront, kp, ctas, c.k.threads, c.smem, s.stream);
         if (e != cudaSuccess) {
             fprintf(stderr, "[wfagpu] alignment kernel launch failed: %s\n", cudaGetErrorString(e));
             return -1;
@@ -1157,7 +1220,7 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         if (time_it) { CK(cudaEventRecord(s.ev[7], s.stream)); s.wf_timed = true; }
         tr.mark("fwd");
         s.stats.launches += 1;
-        if (band_tb) {
+        if (a.band_tb) {
             e = launch_band_traceback(kp, s.stream);
             if (e != cudaSuccess) {
                 fprintf(stderr, "[wfagpu] band traceback kernel launch failed: %s\n", cudaGetErrorString(e));
@@ -1165,11 +1228,11 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
             }
             s.stats.launches += 1;
         }
-        if (c.ckpt) {
+        if (c.k.ckpt) {
             /* ring snapshots -> 2-bit ops, a warp per pair */
             CK(cudaMemsetAsync(s.counters.p + CTR_TBQ, 0, sizeof(uint32_t), s.stream));
-            const int ctas = (int)std::min<size_t>((size_t)tb_ctas, (cnt + kTbWarps - 1) / kTbWarps);
-            e = launch_traceback(kp, ctas, kTbWarps, ascii, s.stream);
+            const int ctas_tb = (int)std::min<size_t>((size_t)tb_ctas, (cnt + kTbWarps - 1) / kTbWarps);
+            e = launch_traceback(kp, ctas_tb, kTbWarps, r.ascii, s.stream);
             if (e != cudaSuccess) {
                 fprintf(stderr, "[wfagpu] traceback kernel launch failed: %s\n", cudaGetErrorString(e));
                 return -1;
@@ -1178,15 +1241,49 @@ static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, int
         }
     }
     tr.mark("tb");
-    if (first_pass) {
+    if (r.first_pass) {
         s.stats.n_cap = (uint32_t)c.n_cap;
-        s.stats.cta_threads = (uint32_t)(c.group_threads * c.groups_per_cta);
+        s.stats.cta_threads = (uint32_t)c.k.threads;
         s.stats.ctas = (uint32_t)c.ctas;
-        s.stats.d_end = (uint32_t)d_end;
+        s.stats.d_end = (uint32_t)a.d_end;
     }
-    s.last_d_end = std::max(s.last_d_end, d_end);
+    s.last_d_end = std::max(s.last_d_end, a.d_end);
     s.text_queued = false;
     return 0;
+}
+
+/* One pass over a request's pairs, in five stages: the scores to provision for, the bound pre-pass (first pass only), the
+ * launch shape, the scores and arenas, the launches.  Returns < 0 on error, else 1 if the pass was capped: provisioned
+ * for fewer scores than the budget and the lengths allow (the pairs it leaves over may only need wider rings), else 0. */
+static int launch_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, PassRequest r)
+{
+    HostTrace tr;
+    if (r.first_pass) {
+        pull_hint(d);                        /* what the last batch on this GPU needed (any context) */
+        if (!s.plain) { d->hint_dist = 0; d->hint_mean = 0; }   /* hints are learnt on global single-piece batches */
+    }
+    if (ensure_step_table(s, plan, r.max_steps)) return -1;
+    Scores sc = provision_scores(d, s, plan, r.first_pass);
+    if (int rc = bound_prepass(d, s, plan, r, sc)) return rc;
+    LaunchCfg c{};
+    int rc;
+    if (plan.band > 0) {
+        rc = choose_band_cfg(d, s, plan, r.n_items, r.ascii, &c);
+    } else {
+        sc.n_want = n_need(s, plan, sc.d_want);
+        /* with a hint, rings for hint + 3 % are enough for (almost) every pair; with bounds, rings for 99 % of the pairs
+         * when that buys a resident CTA */
+        int n_min = sc.n_want;
+        if (sc.hinted)
+            n_min = std::min(sc.n_want, n_need(s, plan, (int)std::min<long long>(hint_plus(d, d->hint_min_pm, 4), sc.d_full - 1) + 1));
+        if (sc.d_p99 > 0) n_min = std::min(sc.n_want, n_need(s, plan, sc.d_p99));
+        rc = choose_cfg(d, s, plan, sc.n_want, n_min, r.n_items, r.ascii, &c);
+    }
+    if (rc) return rc;
+    tr.mark("cfg");
+    Arenas a;
+    if (size_arenas(d, s, plan, r, sc, c, a, tr) || enqueue_pass(d, s, plan, r, sc, c, a, tr)) return -1;
+    return a.d_end < sc.d_reach ? 1 : 0;
 }
 
 /* CIGAR text on the device: queued right behind the alignment kernel so that it overlaps with
@@ -1264,6 +1361,7 @@ extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, 
     if (n != s.n) return -1;
     s.plan = *plan;
     s.ef = ef;
+    s.plain = !ef && !p2;
     s.span = sp;
     /* the span clamped to every pair, then the widest of the batch: the start row's half width and the reach of the
      * target range beyond kt (the step table and the rings are shared by the pairs of a batch) */
@@ -1298,15 +1396,17 @@ extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, 
      * given that budget straight away: 100 k x 1 kbp / 10 % with -e 300 re-dispatched 4.4 % of its pairs in every chunk. */
     int first_steps = plan->max_steps;
     pull_hint(d);
-    if (!ef && !p2 && plan->band <= 0 && d->hint_dist > 0 && d->hint_lift_pm > 0 && d->hint_key[0] == plan->x && d->hint_key[1] == plan->o &&
-        d->hint_key[2] == plan->e && d->hint_key[3] == length_class(s.max_len)) {
-        const long long want = (long long)d->hint_dist + (long long)d->hint_dist * d->hint_margin_pm / 1000 + 12;
+    if (s.plain && d->hint_lift_pm > 0 && hint_applies(d, s, *plan)) {
+        const long long want = hint_plus(d, d->hint_margin_pm, 12);
         const long long most = (long long)plan->max_steps + (long long)plan->max_steps * d->hint_lift_pm / 1000;
         if (want > first_steps && d->hint_dist <= most) first_steps = (int)std::min<long long>(want, d->max_steps_cap);
     }
     s.first_steps = first_steps;
-    int rc = launch_pass(d, s, *plan, first_steps, s.order.p, n, s.retry[0].p, false, true, true, &s.capped);
-    if (rc) return rc;
+    PassRequest first{s.order.p, n, s.retry[0].p, first_steps};
+    first.first_pass = true;
+    const int rc = launch_pass(d, s, *plan, first);
+    if (rc < 0) return rc;
+    s.capped = rc > 0;
     d->device_text = env_int("WFAGPU_HOST_CIGAR", 0) == 0;   /* re-read: tests flip it between runs */
     if (plan->with_cigar && d->device_text && enqueue_text(d, s, n, s.last_d_end)) return -1;
     CK(cudaEventRecord(s.ev[4], s.stream));                  /* align time = bound + wavefronts + traceback + CIGAR text */
@@ -1341,12 +1441,10 @@ extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wf
      * -> the number of wavefront steps that is enough for all of them, 0 if one has no bound. */
     auto bound_budget = [&](int cur, uint32_t pending, long long *need) -> int {
         *need = 0;
-        const int kMaxSteps = d->max_steps_cap;
-        int rc = run_bound_only(d, s, replan, kMaxSteps, s.retry[cur].p, pending);
+        if (s.h_retry.ensure(pending + 1)) return -1;
+        int rc = bounds_to_host(d, s, replan, d->max_steps_cap, s.retry[cur].p, pending);
         if (rc == -2) return 0;                     /* the bound kernel does not fit these penalties: keep doubling */
         if (rc) return rc;
-        if (s.h_bound.ensure(s.n + 1) || s.h_retry.ensure(pending + 1)) return -1;
-        CK(cudaMemcpyAsync(s.h_bound.p, s.bound.p, s.n * sizeof(int32_t), cudaMemcpyDeviceToHost, s.stream));
         CK(cudaMemcpyAsync(s.h_retry.p, s.retry[cur].p, pending * sizeof(uint32_t), cudaMemcpyDeviceToHost, s.stream));
         CK(cudaStreamSynchronize(s.stream));
         const int d_big = s.tab_d_end;
@@ -1401,12 +1499,13 @@ extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wf
                 return fail_pending(cur, pending);
             }
             steps = next;
-            bool now_capped = false;
-            int rc = launch_pass(d, s, replan, (int)steps, s.retry[cur].p, pending, s.retry[cur ^ 1].p, ascii, false, false,
-                                 &now_capped, have_bounds);
-            if (rc) return rc;
+            PassRequest r{s.retry[cur].p, pending, s.retry[cur ^ 1].p, (int)steps};
+            r.ascii = ascii;
+            r.have_bounds = have_bounds;
+            const int rc = launch_pass(d, s, replan, r);
+            if (rc < 0) return rc;
             if (read_counters()) return -1;
-            if (now_capped && s.h_counters.p[CTR_RETRY] > 0) {
+            if (rc > 0 && s.h_counters.p[CTR_RETRY] > 0) {
                 fprintf(stderr, "[wfagpu] %u pairs exceed the wavefront capacity of one CTA; reported as failed\n",
                         s.h_counters.p[CTR_RETRY]);
                 return fail_pending(cur ^ 1, s.h_counters.p[CTR_RETRY]);
@@ -1424,11 +1523,12 @@ extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wf
     const uint32_t n_ascii = s.h_counters.p[CTR_ASCII];
     if (n_ascii > 0) {
         s.stats.ascii_pairs = n_ascii;
-        bool capped = false;
-        rc = launch_pass(d, s, plan, plan.max_steps, s.ascii_list.p, n_ascii, s.retry[0].p, true, false, false, &capped);
-        if (rc) return rc;
+        PassRequest r{s.ascii_list.p, n_ascii, s.retry[0].p, plan.max_steps};
+        r.ascii = true;
+        rc = launch_pass(d, s, plan, r);
+        if (rc < 0) return rc;
         if (read_counters()) return -1;
-        rc = redispatch(true, plan.max_steps, capped);
+        rc = redispatch(true, plan.max_steps, rc > 0);
         if (rc) return rc;
     }
     CK(cudaEventRecord(s.ev[5], s.stream));
@@ -1450,7 +1550,7 @@ extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wf
     }
     s.stats.failed_pairs = (uint32_t)failed.size();
     memcpy(out, s.h_out.p, n * sizeof(wfagpu_pair_out_t));
-    if (!d->independent && !s.ef && s.plan.e2 <= 0) learn_hint(d, s, n);
+    if (!d->independent && s.plain) learn_hint(d, s, n);
     if (pair_flags)
         for (size_t i = 0; i < n; ++i) pair_flags[i] = s.h_pairs.p[i].flags;
     if (ops) *ops = s.h_pool.p;
@@ -1521,7 +1621,7 @@ extern "C" int wfagpu_device_wait(wfagpu_device_t *d, int slot, float *ms_pack, 
         CK(cudaStreamSynchronize(s.stream));
         s.stats.pending_pairs = s.h_counters.p[CTR_RETRY] + s.h_counters.p[CTR_ASCII];
     }
-    if (s.n && d->use_hint && !s.ef && s.plan.e2 <= 0) {
+    if (s.n && d->use_hint && s.plain) {
         /* read the result records back (16 B per pair) so that a re-run of the resident
          * batch is provisioned like the next batch of a stream would be */
         if (s.h_out.ensure(s.n)) return -1;

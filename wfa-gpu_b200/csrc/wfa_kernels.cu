@@ -2513,41 +2513,6 @@ size_t banded_smem_bytes(int A, int win, int seq_words, int stages)
     return ring_bytes + lohi_bytes + 2 * (size_t)stages * seq_words * 4 + sizeof(BandCtl) + 16;
 }
 
-template <bool ASCII, bool BT>
-static cudaError_t launch_banded_one(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
-{
-    auto kfn = wfa_banded_kernel<ASCII, BT>;
-    cudaError_t err = allow_max_smem(kfn);
-    if (err != cudaSuccess) return err;
-    kfn<<<ctas, threads, smem, s>>>(p);
-    return cudaGetLastError();
-}
-
-template <bool ASCII, bool BT>
-static int occupancy_banded_one(int threads, size_t smem)
-{
-    auto kfn = wfa_banded_kernel<ASCII, BT>;
-    int n = 0;
-    if (allow_max_smem(kfn) != cudaSuccess) return 0;
-    if (occupancy_of(&n, kfn, threads, smem) != cudaSuccess) return 0;
-    return n;
-}
-
-cudaError_t launch_banded(const KernelParams &p, int threads, int ctas, size_t smem_bytes, bool ascii, cudaStream_t s)
-{
-    const bool bt = p.with_bt != 0;
-    if (ascii) return bt ? launch_banded_one<true, true>(p, threads, ctas, smem_bytes, s)
-                         : launch_banded_one<true, false>(p, threads, ctas, smem_bytes, s);
-    return bt ? launch_banded_one<false, true>(p, threads, ctas, smem_bytes, s)
-              : launch_banded_one<false, false>(p, threads, ctas, smem_bytes, s);
-}
-
-int banded_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii, bool bt)
-{
-    if (ascii) return bt ? occupancy_banded_one<true, true>(threads, smem_bytes) : occupancy_banded_one<true, false>(threads, smem_bytes);
-    return bt ? occupancy_banded_one<false, true>(threads, smem_bytes) : occupancy_banded_one<false, false>(threads, smem_bytes);
-}
-
 /* ======================================================================== */
 /*        adaptive band, four diagonals per thread on packed int16          */
 /* ======================================================================== */
@@ -3019,36 +2984,6 @@ size_t bandq_smem_bytes(int A, int win, int seq_words, int stages)
     return ring_bytes + win_bytes + 2 * (size_t)stages * seq_words * 4 + sizeof(BandQCtl) + 16;
 }
 
-cudaError_t launch_bandq(const KernelParams &p, int threads, int ctas, size_t smem_bytes, cudaStream_t s)
-{
-    cudaError_t err;
-    if (p.with_bt) {
-        auto kfn = wfa_bandq_kernel<true>;
-        if ((err = allow_max_smem(kfn)) != cudaSuccess) return err;
-        kfn<<<ctas, threads, smem_bytes, s>>>(p);
-    } else {
-        auto kfn = wfa_bandq_kernel<false>;
-        if ((err = allow_max_smem(kfn)) != cudaSuccess) return err;
-        kfn<<<ctas, threads, smem_bytes, s>>>(p);
-    }
-    return cudaGetLastError();
-}
-
-int bandq_max_ctas_per_sm(int threads, size_t smem_bytes, bool bt)
-{
-    int n = 0;
-    if (bt) {
-        auto kfn = wfa_bandq_kernel<true>;
-        if (allow_max_smem(kfn) != cudaSuccess) return 0;
-        if (occupancy_of(&n, kfn, threads, smem_bytes) != cudaSuccess) return 0;
-    } else {
-        auto kfn = wfa_bandq_kernel<false>;
-        if (allow_max_smem(kfn) != cudaSuccess) return 0;
-        if (occupancy_of(&n, kfn, threads, smem_bytes) != cudaSuccess) return 0;
-    }
-    return n;
-}
-
 /* ======================================================================== */
 /*                       CIGAR text emission on the device                  */
 /* ======================================================================== */
@@ -3262,23 +3197,19 @@ void launch_cigar_text(const CigarParams &p, cudaStream_t s)
 
 /* ---- host-side launch helpers ---------------------------------------------- */
 
-template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false, bool P2 = false>
-static cudaError_t launch_one(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
+cudaError_t launch(kernel_fn kfn, const KernelParams &p, int ctas, int threads, size_t smem, cudaStream_t s)
 {
-    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF, P2>;
+    if (!kfn) return cudaErrorInvalidValue;
     cudaError_t err = allow_max_smem(kfn);
     if (err != cudaSuccess) return err;
     kfn<<<ctas, threads, smem, s>>>(p);
     return cudaGetLastError();
 }
 
-template <bool WARP, bool ASCII, bool BT, typename R = RingS16, bool CKPT = false, bool EF = false, bool P2 = false>
-static int occupancy_one(int threads, size_t smem)
+int max_ctas_per_sm(kernel_fn kfn, int threads, size_t smem)
 {
-    auto kfn = wfa_exact_kernel<WARP, ASCII, BT, R, CKPT, EF, P2>;
     int n = 0;
-    if (allow_max_smem(kfn) != cudaSuccess) return 0;
-    if (occupancy_of(&n, kfn, threads, smem) != cudaSuccess) return 0;
+    if (!kfn || allow_max_smem(kfn) != cudaSuccess || occupancy_of(&n, kfn, threads, smem) != cudaSuccess) return 0;
     return n;
 }
 
@@ -3295,20 +3226,12 @@ size_t bound_smem_bytes(int A, int E1, int warps) { return (size_t)warps * (size
 
 cudaError_t launch_bound(const KernelParams &p, int ctas, int warps, cudaStream_t s)
 {
-    const size_t smem = bound_smem_bytes(p.A, p.E1, warps);
-    cudaError_t err = allow_max_smem(wfa_bound_kernel);
-    if (err != cudaSuccess) return err;
-    wfa_bound_kernel<<<ctas, 32 * warps, smem, s>>>(p);
-    return cudaGetLastError();
+    return launch(wfa_bound_kernel, p, ctas, 32 * warps, bound_smem_bytes(p.A, p.E1, warps), s);
 }
 
 int bound_max_ctas_per_sm(int A, int E1, int warps)
 {
-    const size_t smem = bound_smem_bytes(A, E1, warps);
-    int n = 0;
-    if (allow_max_smem(wfa_bound_kernel) != cudaSuccess) return 0;
-    if (occupancy_of(&n, wfa_bound_kernel, 32 * warps, smem) != cudaSuccess) return 0;
-    return n;
+    return max_ctas_per_sm(wfa_bound_kernel, 32 * warps, bound_smem_bytes(A, E1, warps));
 }
 
 size_t traceback_smem_bytes(int A, int period, int warps)
@@ -3317,8 +3240,7 @@ size_t traceback_smem_bytes(int A, int period, int warps)
     return per_warp * (size_t)warps;
 }
 
-using tb_kernel_t = void (*)(const KernelParams);
-static tb_kernel_t traceback_fn(bool ascii, int period)
+static kernel_fn traceback_fn(bool ascii, int period)
 {
     switch (period) {
     /* 2P + 1 diagonals at the base of a cone: 15 and 31 keep a level within one and two warp passes */
@@ -3331,198 +3253,59 @@ static tb_kernel_t traceback_fn(bool ascii, int period)
 
 cudaError_t launch_traceback(const KernelParams &p, int ctas, int warps, bool ascii, cudaStream_t s)
 {
-    const size_t smem = traceback_smem_bytes(p.A, p.ck_period, warps);
-    tb_kernel_t kfn = traceback_fn(ascii, p.ck_period);
-    if (!kfn) return cudaErrorInvalidValue;
-    cudaError_t err = allow_max_smem(kfn);
-    if (err != cudaSuccess) return err;
-    kfn<<<ctas, 32 * warps, smem, s>>>(p);
-    return cudaGetLastError();
+    return launch(traceback_fn(ascii, p.ck_period), p, ctas, 32 * warps, traceback_smem_bytes(p.A, p.ck_period, warps), s);
 }
 
 int traceback_max_ctas_per_sm(int A, int period, int warps, bool ascii)
 {
-    const size_t smem = traceback_smem_bytes(A, period, warps);
-    tb_kernel_t kfn = traceback_fn(ascii, period);
-    int n = 0;
-    if (!kfn) return 0;
-    if (allow_max_smem(kfn) != cudaSuccess) return 0;
-    if (occupancy_of(&n, kfn, 32 * warps, smem) != cudaSuccess) return 0;
-    return n;
+    return max_ctas_per_sm(traceback_fn(ascii, period), 32 * warps, traceback_smem_bytes(A, period, warps));
 }
 
-#define WFAGPU_DISPATCH(FN, ...)                                                              \
-    (warp ? (ascii ? (bt ? FN<true, true, true>(__VA_ARGS__) : FN<true, true, false>(__VA_ARGS__))       \
-                   : (bt ? FN<true, false, true>(__VA_ARGS__) : FN<true, false, false>(__VA_ARGS__)))    \
-          : (ascii ? (bt ? FN<false, true, true>(__VA_ARGS__) : FN<false, true, false>(__VA_ARGS__))     \
-                   : (bt ? FN<false, false, true>(__VA_ARGS__) : FN<false, false, false>(__VA_ARGS__))))
-
-/* ends-free instantiations: FN<WARP, ASCII, BT, RingS16, false, true> */
-template <bool WARP, bool ASCII, bool BT>
-static cudaError_t launch_one_ef(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
+/* wfa_exact_kernel of one tier (WARP, Ring) in the batch's mode: ends-free, 2-piece or single-piece global */
+template <bool WARP, bool ASCII, bool BT, typename R>
+static kernel_fn exact_mode(const KernelChoice &k)
 {
-    return launch_one<WARP, ASCII, BT, RingS16, false, true>(p, threads, ctas, smem, s);
-}
-template <bool WARP, bool ASCII, bool BT>
-static int occupancy_one_ef(int threads, size_t smem)
-{
-    return occupancy_one<WARP, ASCII, BT, RingS16, false, true>(threads, smem);
+    if (k.ef) return wfa_exact_kernel<WARP, ASCII, BT, R, false, true>;
+    if (k.p2) return wfa_exact_kernel<WARP, ASCII, BT, R, false, false, true>;
+    return wfa_exact_kernel<WARP, ASCII, BT, R, false>;
 }
 
-/* gap-affine 2-piece instantiations: FN<WARP, ASCII, BT, R, false, false, true> */
-template <bool WARP, bool ASCII, bool BT>
-static cudaError_t launch_one_p2(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
+template <bool ASCII, bool BT>
+static kernel_fn exact_fn(const KernelChoice &k)
 {
-    return launch_one<WARP, ASCII, BT, RingS16, false, false, true>(p, threads, ctas, smem, s);
-}
-template <bool WARP, bool ASCII, bool BT>
-static int occupancy_one_p2(int threads, size_t smem)
-{
-    return occupancy_one<WARP, ASCII, BT, RingS16, false, false, true>(threads, smem);
-}
-
-template <bool BT, bool COUNT>
-static cudaError_t launch_quad_one(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
-{
-    auto kfn = wfa_quad_kernel<BT, COUNT>;
-    cudaError_t err = allow_max_smem(kfn);
-    if (err != cudaSuccess) return err;
-    kfn<<<ctas, threads, smem, s>>>(p);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_quad(const KernelParams &p, int threads, int ctas, size_t smem_bytes, cudaStream_t s)
-{
-    if (p.with_bt && !p.ck_off) return cudaErrorInvalidValue;       /* with backtrace: ring snapshots only */
-    if (p.cells)        /* instrumented build of the same kernel: counts the cells of every window */
-        return p.with_bt ? launch_quad_one<true, true>(p, threads, ctas, smem_bytes, s) : launch_quad_one<false, true>(p, threads, ctas, smem_bytes, s);
-    return p.with_bt ? launch_quad_one<true, false>(p, threads, ctas, smem_bytes, s) : launch_quad_one<false, false>(p, threads, ctas, smem_bytes, s);
-}
-
-int quad_max_ctas_per_sm(int threads, size_t smem_bytes, bool bt)
-{
-    int n = 0;
-    if (bt) {
-        auto kfn = wfa_quad_kernel<true, false>;
-        if (allow_max_smem(kfn) != cudaSuccess) return 0;
-        if (occupancy_of(&n, kfn, threads, smem_bytes) != cudaSuccess) return 0;
-    } else {
-        auto kfn = wfa_quad_kernel<false, false>;
-        if (allow_max_smem(kfn) != cudaSuccess) return 0;
-        if (occupancy_of(&n, kfn, threads, smem_bytes) != cudaSuccess) return 0;
+    if (k.ckpt) {
+        /* ring snapshots: CTA per pair, shared-memory rings, CIGAR wanted, single-piece global alignment */
+        if (k.warp || !BT || k.gring || k.ef || k.p2) return nullptr;
+        return wfa_exact_kernel<false, ASCII, true, RingS16, true>;
     }
-    return n;
+    if (k.gring) return exact_mode<false, ASCII, BT, RingG32>(k);     /* large tier: CTA per pair, int32 rings in HBM */
+    return k.warp ? exact_mode<true, ASCII, BT, RingS16>(k) : exact_mode<false, ASCII, BT, RingS16>(k);
 }
 
-template <bool BT, int MAXT>
-static cudaError_t launch_quadg_one(const KernelParams &p, int threads, int ctas, size_t smem, cudaStream_t s)
+kernel_fn wavefront_kernel(const KernelChoice &k, bool count_cells)
 {
-    auto kfn = wfa_quadg_kernel<BT, MAXT>;
-    cudaError_t err = allow_max_smem(kfn);
-    if (err != cudaSuccess) return err;
-    kfn<<<ctas, threads, smem, s>>>(p);
-    return cudaGetLastError();
-}
-template <bool BT, int MAXT>
-static int occupancy_quadg_one(int threads, size_t smem)
-{
-    auto kfn = wfa_quadg_kernel<BT, MAXT>;
-    int n = 0;
-    if (allow_max_smem(kfn) != cudaSuccess) return 0;
-    if (occupancy_of(&n, kfn, threads, smem) != cudaSuccess) return 0;
-    return n;
-}
-
-/* three register budgets: <= 512 threads (107 registers), <= 768 (85), <= 1024 (64) */
-cudaError_t launch_quadg(const KernelParams &p, int threads, int ctas, size_t smem_bytes, cudaStream_t s)
-{
-    if (!p.gring) return cudaErrorInvalidValue;
-    if (threads <= 512) return p.with_bt ? launch_quadg_one<true, 512>(p, threads, ctas, smem_bytes, s) : launch_quadg_one<false, 512>(p, threads, ctas, smem_bytes, s);
-    if (threads <= 768) return p.with_bt ? launch_quadg_one<true, 768>(p, threads, ctas, smem_bytes, s) : launch_quadg_one<false, 768>(p, threads, ctas, smem_bytes, s);
-    return p.with_bt ? launch_quadg_one<true, 1024>(p, threads, ctas, smem_bytes, s) : launch_quadg_one<false, 1024>(p, threads, ctas, smem_bytes, s);
-}
-
-int quadg_max_ctas_per_sm(int threads, size_t smem_bytes, bool bt)
-{
-    if (threads <= 512) return bt ? occupancy_quadg_one<true, 512>(threads, smem_bytes) : occupancy_quadg_one<false, 512>(threads, smem_bytes);
-    if (threads <= 768) return bt ? occupancy_quadg_one<true, 768>(threads, smem_bytes) : occupancy_quadg_one<false, 768>(threads, smem_bytes);
-    return bt ? occupancy_quadg_one<true, 1024>(threads, smem_bytes) : occupancy_quadg_one<false, 1024>(threads, smem_bytes);
-}
-
-cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_per_cta, int ctas,
-                         size_t smem_bytes, bool ascii, cudaStream_t s)
-{
-    const bool warp = (group_threads == 32);
-    const bool bt = p.with_bt != 0;
-    const int threads = warp ? 32 * groups_per_cta : group_threads;
-    if (p.ends) {
-        /* ends-free: decision-byte traceback on every tier */
-        if (p.ck_off) return cudaErrorInvalidValue;
-        if (p.gring) {
-            if (ascii) return bt ? launch_one<false, true, true, RingG32, false, true>(p, threads, ctas, smem_bytes, s)
-                                 : launch_one<false, true, false, RingG32, false, true>(p, threads, ctas, smem_bytes, s);
-            return bt ? launch_one<false, false, true, RingG32, false, true>(p, threads, ctas, smem_bytes, s)
-                      : launch_one<false, false, false, RingG32, false, true>(p, threads, ctas, smem_bytes, s);
-        }
-        return WFAGPU_DISPATCH(launch_one_ef, p, threads, ctas, smem_bytes, s);
+    switch (k.family) {
+    case Family::Exact:
+        if (k.ascii) return k.bt ? exact_fn<true, true>(k) : exact_fn<true, false>(k);
+        return k.bt ? exact_fn<false, true>(k) : exact_fn<false, false>(k);
+    case Family::Quad:
+        if (k.bt && !k.ckpt) return nullptr;               /* with backtrace: ring snapshots only */
+        if (count_cells)   /* instrumented build of the same kernel: counts the cells of every window */
+            return k.bt ? wfa_quad_kernel<true, true> : wfa_quad_kernel<false, true>;
+        return k.bt ? wfa_quad_kernel<true, false> : wfa_quad_kernel<false, false>;
+    case Family::QuadG:
+        if (!k.gring) return nullptr;
+        /* three register budgets: <= 512 threads (107 registers), <= 768 (85), <= 1024 (64) */
+        if (k.threads <= 512) return k.bt ? wfa_quadg_kernel<true, 512> : wfa_quadg_kernel<false, 512>;
+        if (k.threads <= 768) return k.bt ? wfa_quadg_kernel<true, 768> : wfa_quadg_kernel<false, 768>;
+        return k.bt ? wfa_quadg_kernel<true, 1024> : wfa_quadg_kernel<false, 1024>;
+    case Family::Banded:
+        if (k.ascii) return k.bt ? wfa_banded_kernel<true, true> : wfa_banded_kernel<true, false>;
+        return k.bt ? wfa_banded_kernel<false, true> : wfa_banded_kernel<false, false>;
+    case Family::BandQ:
+        return k.bt ? wfa_bandq_kernel<true> : wfa_bandq_kernel<false>;
     }
-    if (p.e2 > 0) {
-        /* gap-affine 2-piece: decision-byte traceback on every tier */
-        if (p.ck_off) return cudaErrorInvalidValue;
-        if (p.gring) {
-            if (ascii) return bt ? launch_one<false, true, true, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s)
-                                 : launch_one<false, true, false, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s);
-            return bt ? launch_one<false, false, true, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s)
-                      : launch_one<false, false, false, RingG32, false, false, true>(p, threads, ctas, smem_bytes, s);
-        }
-        return WFAGPU_DISPATCH(launch_one_p2, p, threads, ctas, smem_bytes, s);
-    }
-    if (p.gring) {
-        /* large tier: CTA per pair, rings in global memory, int32 offsets */
-        if (ascii) return bt ? launch_one<false, true, true, RingG32>(p, threads, ctas, smem_bytes, s)
-                             : launch_one<false, true, false, RingG32>(p, threads, ctas, smem_bytes, s);
-        return bt ? launch_one<false, false, true, RingG32>(p, threads, ctas, smem_bytes, s)
-                  : launch_one<false, false, false, RingG32>(p, threads, ctas, smem_bytes, s);
-    }
-    if (p.ck_off) {
-        /* checkpointed traceback (CTA per pair, shared-memory rings, CIGAR wanted) */
-        if (warp || !bt) return cudaErrorInvalidValue;
-        return ascii ? launch_one<false, true, true, RingS16, true>(p, threads, ctas, smem_bytes, s)
-                     : launch_one<false, false, true, RingS16, true>(p, threads, ctas, smem_bytes, s);
-    }
-    return WFAGPU_DISPATCH(launch_one, p, threads, ctas, smem_bytes, s);
-}
-
-int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii, bool bt, bool ef, bool p2)
-{
-    if (p2) {
-        if (ascii) return bt ? occupancy_one<false, true, true, RingG32, false, false, true>(threads, smem_bytes)
-                             : occupancy_one<false, true, false, RingG32, false, false, true>(threads, smem_bytes);
-        return bt ? occupancy_one<false, false, true, RingG32, false, false, true>(threads, smem_bytes)
-                  : occupancy_one<false, false, false, RingG32, false, false, true>(threads, smem_bytes);
-    }
-    if (ef) {
-        if (ascii) return bt ? occupancy_one<false, true, true, RingG32, false, true>(threads, smem_bytes)
-                             : occupancy_one<false, true, false, RingG32, false, true>(threads, smem_bytes);
-        return bt ? occupancy_one<false, false, true, RingG32, false, true>(threads, smem_bytes)
-                  : occupancy_one<false, false, false, RingG32, false, true>(threads, smem_bytes);
-    }
-    if (ascii) return bt ? occupancy_one<false, true, true, RingG32>(threads, smem_bytes)
-                         : occupancy_one<false, true, false, RingG32>(threads, smem_bytes);
-    return bt ? occupancy_one<false, false, true, RingG32>(threads, smem_bytes)
-              : occupancy_one<false, false, false, RingG32>(threads, smem_bytes);
-}
-
-int exact_max_ctas_per_sm(int group_threads, int groups_per_cta, size_t smem_bytes, bool ascii, bool bt, bool ckpt,
-                          bool ef, bool p2)
-{
-    const bool warp = (group_threads == 32);
-    const int threads = warp ? 32 * groups_per_cta : group_threads;
-    if (p2) return WFAGPU_DISPATCH(occupancy_one_p2, threads, smem_bytes);
-    if (ef) return WFAGPU_DISPATCH(occupancy_one_ef, threads, smem_bytes);
-    if (ckpt) return ascii ? occupancy_one<false, true, true, RingS16, true>(threads, smem_bytes)
-                           : occupancy_one<false, false, true, RingS16, true>(threads, smem_bytes);
-    return WFAGPU_DISPATCH(occupancy_one, threads, smem_bytes);
+    return nullptr;
 }
 
 } // namespace wfagpu

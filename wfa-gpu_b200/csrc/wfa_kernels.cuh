@@ -121,18 +121,40 @@ struct CigarParams {
 
 void launch_pack(const PackParams &p, cudaStream_t s);
 void launch_cigar_text(const CigarParams &p, cudaStream_t s);
-/* group_threads == 32 -> warp-per-pair variant; otherwise CTA-per-pair.  p.ends != null runs the ends-free
- * variant, p.e2 > 0 the gap-affine 2-piece variant (both: decision-byte traceback only, p.ck_off must be null) */
-cudaError_t launch_exact(const KernelParams &p, int group_threads, int groups_per_cta, int ctas,
-                         size_t smem_bytes, bool ascii_extend, cudaStream_t s);
-/* CTA per pair, four diagonals per thread (packed sequences, shared-memory rings whose diagonal 0 is 16-byte
- * aligned; with backtrace it writes ring snapshots: p.ck_off must be set) */
-cudaError_t launch_quad(const KernelParams &p, int threads, int ctas, size_t smem_bytes, cudaStream_t s);
-int quad_max_ctas_per_sm(int threads, size_t smem_bytes, bool bt);
-/* large tier: int32 rings in global memory (p.gring, rows of p.row_stride elements, multiple of 4, diagonal 0 at p.center,
- * multiple of 4), four diagonals per thread; shared memory = exact_smem_bytes(A, E1, 0, seq_words, 1, 1, true) */
-cudaError_t launch_quadg(const KernelParams &p, int threads, int ctas, size_t smem_bytes, cudaStream_t s);
-int quadg_max_ctas_per_sm(int threads, size_t smem_bytes, bool bt);
+
+/* Which wavefront kernel a launch runs.  It is decided once per launch shape: the occupancy questions that size the
+ * launch and the launch itself ask with the same value. */
+enum class Family : uint8_t {
+    Exact,    /* wfa_exact_kernel: one diagonal per thread, warp or CTA per pair */
+    Quad,     /* wfa_quad_kernel: CTA per pair, four diagonals per thread on packed int16, shared-memory rings whose
+               * diagonal 0 is 16-byte aligned; with backtrace it writes ring snapshots (ckpt) */
+    QuadG,    /* wfa_quadg_kernel: the large tier's quad kernel, int32 rings in global memory (gring): rows a multiple of 4,
+               * diagonal 0 at a multiple of 4; shared memory = exact_smem_bytes(A, E1, 0, seq_words, 1, 1, true) */
+    Banded,   /* wfa_banded_kernel: adaptive band (-B) */
+    BandQ,    /* wfa_bandq_kernel: the same, four diagonals per thread on packed int16 (packed pairs only) */
+};
+struct KernelChoice {
+    Family family = Family::Exact;
+    bool warp = false;    /* exact: warp per pair (threads = 32 x pairs per CTA) */
+    bool ascii = false;   /* byte-compare extend on the ASCII copy */
+    bool bt = false;      /* backtrace (CIGAR) */
+    bool gring = false;   /* rings in global memory, int32 offsets (RingG32); else shared memory (RingS16) */
+    bool ckpt = false;    /* ring snapshots for wfa_traceback_kernel instead of decision bytes */
+    bool ef = false;      /* exact: ends-free (decision-byte traceback on every tier) */
+    bool p2 = false;      /* exact: gap-affine 2-piece (likewise) */
+    int threads = 0;      /* threads per CTA; QuadG picks its register budget (MAXT) from it */
+    bool quad() const { return family == Family::Quad || family == Family::QuadG || family == Family::BandQ; }
+};
+using kernel_fn = void (*)(const KernelParams);
+/* the __global__ function of `k`, null for a combination that has no kernel.  count_cells: the instrumented
+ * wfa_quad_kernel (COUNT = true) that fills p.cells; occupancy is always asked without it, so that counting cells does
+ * not change the launch shape */
+kernel_fn wavefront_kernel(const KernelChoice &k, bool count_cells = false);
+/* allow the opt-in shared memory, launch, and report the launch error (null kfn: cudaErrorInvalidValue) */
+cudaError_t launch(kernel_fn kfn, const KernelParams &p, int ctas, int threads, size_t smem, cudaStream_t s);
+/* resident CTAs per SM at that shape, 0 if none (or null kfn) */
+int max_ctas_per_sm(kernel_fn kfn, int threads, size_t smem);
+
 /* per-pair score upper bounds for the pruning (warp per pair) */
 cudaError_t launch_bound(const KernelParams &p, int ctas, int warps, cudaStream_t s);
 size_t bound_smem_bytes(int A, int E1, int warps);
@@ -145,19 +167,9 @@ int traceback_max_ctas_per_sm(int A, int period, int warps, bool ascii_extend);
  * E2 > 0: the two extra I2 / D2 rings of a 2-piece launch */
 size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched = false,
                         int E2 = 0);
-cudaError_t launch_banded(const KernelParams &p, int threads, int ctas, size_t smem_bytes, bool ascii_extend,
-                          cudaStream_t s);
 size_t banded_smem_bytes(int A, int win, int seq_words, int stages);
-int banded_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii_extend, bool with_bt);
-/* the same heuristic, four diagonals per thread on packed int16 (packed pairs only) */
-cudaError_t launch_bandq(const KernelParams &p, int threads, int ctas, size_t smem_bytes, cudaStream_t s);
 size_t bandq_smem_bytes(int A, int win, int seq_words, int stages);
-int bandq_max_ctas_per_sm(int threads, size_t smem_bytes, bool with_bt);
 /* decision bytes of wfa_bandq_kernel -> 2-bit ops, one thread per pair of the launch */
 cudaError_t launch_band_traceback(const KernelParams &p, cudaStream_t s);
-int large_max_ctas_per_sm(int threads, size_t smem_bytes, bool ascii_extend, bool with_bt, bool ef = false,
-                          bool p2 = false);
-int exact_max_ctas_per_sm(int group_threads, int groups_per_cta, size_t smem_bytes, bool ascii_extend, bool with_bt,
-                          bool ckpt = false, bool ef = false, bool p2 = false);
 
 } // namespace wfagpu

@@ -123,6 +123,8 @@ typedef struct {
     int threads_hint;
     int workers_hint;
     int o2, e2;      /* gap-affine 2-piece: second gap piece; e2 == 0 = one piece (o, e) */
+    int with_ends;   /* ends-free, with_cigar == 0: also find where every alignment begins (k_begin of
+                      * wfagpu_device_download_ends); 0 = score only, as before */
 } wfagpu_plan_t;
 
 /* Statistics of the last batch (kernel times from CUDA events on the launch
@@ -177,7 +179,9 @@ int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, const wfagp
                              const wfagpu_span_t *span);
 /* After wfagpu_device_download of an ends-free batch: per pair {k_begin, k_end} (2 n ints), the diagonals of the
  * alignment's first and last cell: it starts at (max(0, -k_begin), max(0, k_begin)) and ends at offset
- * min(tlen, plen + k_end).  Pairs that did not finish hold no record.  -1 for a global batch. */
+ * min(tlen, plen + k_end).  k_end is always valid; k_begin only when the batch was aligned with with_cigar or
+ * with_ends (a score-only batch without with_ends holds k_begin = k_end).  Pairs that did not finish hold no record.
+ * -1 for a global batch. */
 int wfagpu_device_download_ends(wfagpu_device_t *d, int slot, size_t n, int32_t *ends);
 /* A plan with e2 > 0 (gap-affine 2-piece, through wfagpu_device_align / _align_span / _rescore) runs the
  * one-diagonal-per-thread kernels with decision-byte traceback, no score-bound kernel (pruning uses the launch bound)
@@ -278,7 +282,7 @@ int wfagpu_parse_devices(const char *spec, int visible, int *devs, int max_devs)
  * one-diagonal-per-thread kernels, launch bound only -- no per-pair bounds, packed-SIMD kernel, snapshots or
  * provisioning hints.  scores[i] = -1 for a pair it could not finish. */
 int wfagpu_device_rescore(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int32_t *scores);
-/* The same for an ends-free span (NULL = global). */
+/* The same for an ends-free span (NULL = global).  with_cigar and with_ends of the plan are ignored. */
 int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
                                const wfagpu_span_t *span, int32_t *scores);
 
@@ -342,6 +346,21 @@ void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buff
                                    sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
                                    wfa_alignment_options_t options, bool cigar, bool check_correctness,
                                    const wfagpu_span_t *span);
+
+/* The aligned part: pattern[pattern_begin, pattern_end) against text[text_begin, text_end).  From {k_begin, k_end}:
+ * pattern_begin = max(0, -k_begin), text_begin = max(0, k_begin), text_end = min(tlen, plen + k_end),
+ * pattern_end = text_end - k_end.  Global call (NULL / zero span): (0, plen, 0, tlen).  Pair not aligned: all -1. */
+typedef struct {
+    int pattern_begin, pattern_end, text_begin, text_end;
+} wfagpu_coords_t;
+/* wfagpu_align_span that also fills `coords` (one entry per pair, owned by the caller) in CIGAR and score-only mode.
+ * NULL coords: exactly wfagpu_align_span. */
+bool wfagpu_align_span_coords(wfagpu_aligner_t *aligner, const wfagpu_span_t *span, wfagpu_coords_t *coords);
+/* wfagpu_launch_alignments_span that also fills `coords`; NULL coords: exactly wfagpu_launch_alignments_span. */
+void wfagpu_launch_alignments_span_coords(char *sequences_buffer, size_t sequences_buffer_size,
+                                          sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                          wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                          const wfagpu_span_t *span, wfagpu_coords_t *coords);
 
 /* The reference library's generic validators, same names, argument order (text first) and input format
  * (utils/verification.h:37-58): the op string may be UNROLLED ("MMXMMI", what the reference's recover_cigar

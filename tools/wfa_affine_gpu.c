@@ -21,8 +21,10 @@
  *   -G/--affine2p-penalties x,o1,e1,o2,e2
  *                                    gap-affine 2-piece penalties (WFA2-lib's affine2p): a gap of L bases costs
  *                                    min(o1 + e1 L, o2 + e2 L); signs are stripped, e1, e2 >= 1; not with -g, -B or -F
+ *   -P/--print-coords                append where each alignment lies: pattern_begin, pattern_end, text_begin, text_end
+ *                                    (pattern[pb, pe) against text[tb, te); the full sequences without -F); not with -G
  *   -o/--output-file FILE, -p/--print-output, -O/--output-verbose
- * Output lines: "-score\tCIGAR" (or "-score\tCIGAR\tpattern\ttext" with -O).
+ * Output lines: "-score\tCIGAR" (then "\tpb\tpe\ttb\tte" with -P, then "\tpattern\ttext" with -O).
  * Pairs whose score exceeds -e are NOT sent to a CPU: they are re-dispatched on the GPU.
  * Extra: -D/--devices SPEC ("all", "n:4", "0,1") shards the batches over several GPUs;
  *        -S/--stream N streams the input in windows of N pairs (the next window is read into page-locked memory
@@ -39,7 +41,7 @@
 typedef struct {
     const char *seq, *fq, *ft, *out, *pen, *devices, *ends_free, *pen2;
     long n, e, t, b, w, band, stream;
-    int have_e, have_t, have_b, have_w, have_band, have_stream, cigar, check, print, verbose;
+    int have_e, have_t, have_b, have_w, have_band, have_stream, cigar, check, print, verbose, coords;
 } args_t;
 
 static void usage(void)
@@ -53,6 +55,7 @@ static void usage(void)
             "\t-o, --output-file FILE          where the alignment output is saved\n"
             "\t-p, --print-output              print the output to stderr\n"
             "\t-O, --output-verbose            add query/target to the output\n"
+            "\t-P, --print-coords              add the aligned intervals: pattern begin, end, text begin, end\n"
             "[Alignment Options]\n"
             "\t-g, --affine-penalties x,o,e    gap-affine penalties (default 2,3,1)\n"
             "\t-x, --compute-cigar             compute the CIGAR, not only the score\n"
@@ -78,7 +81,7 @@ static const struct { char s; const char *l; int has_val; } OPTS[] = {
     {'g', "affine-penalties", 1}, {'x', "compute-cigar", 0}, {'c', "check", 0}, {'e', "max-distance", 1},
     {'t', "threads-per-block", 1}, {'b', "batch-size", 1}, {'w', "workers", 1}, {'B', "band", 1},
     {'o', "output-file", 1}, {'p', "print-output", 0}, {'O', "output-verbose", 0}, {'D', "devices", 1},
-    {'S', "stream", 1}, {'F', "ends-free", 1}, {'G', "affine2p-penalties", 1},
+    {'S', "stream", 1}, {'F', "ends-free", 1}, {'G', "affine2p-penalties", 1}, {'P', "print-coords", 0},
 };
 
 static int parse(int argc, char **argv, args_t *a)
@@ -118,6 +121,7 @@ static int parse(int argc, char **argv, args_t *a)
         case 'c': a->check = 1; break;
         case 'p': a->print = 1; break;
         case 'O': a->verbose = 1; break;
+        case 'P': a->coords = 1; break;
         }
     }
     return seen;
@@ -168,6 +172,7 @@ int main(int argc, char **argv)
         if (a.pen) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --affine-penalties (-g).\n"); return 1; }
         if (a.have_band) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with the band (-B).\n"); return 1; }
         if (a.ends_free) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --ends-free (-F).\n"); return 1; }
+        if (a.coords) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --print-coords (-P).\n"); return 1; }
         if (sscanf(a.pen2, "%d,%d,%d,%d,%d", &pen2.x, &pen2.o1, &pen2.e1, &pen2.o2, &pen2.e2) != 5) {
             fprintf(stderr, "[!] ERROR: --affine2p-penalties takes five values: x,o1,e1,o2,e2 (got %s).\n", a.pen2);
             return 1;
@@ -290,6 +295,8 @@ int main(int argc, char **argv)
             fprintf(stderr, "[!] ERROR: Can not initialise CIGAR buffer.\n");
             return -1;
         }
+        wfagpu_coords_t *coords = a.coords ? (wfagpu_coords_t *)malloc((size_t)pairs * sizeof(wfagpu_coords_t)) : NULL;
+        if (a.coords && !coords) { fprintf(stderr, "[!] ERROR: Can not allocate the coordinates.\n"); return -1; }
         wfa_alignment_options_t opt;
         memset(&opt, 0, sizeof(opt));
         opt.max_error = max_distance;
@@ -306,9 +313,9 @@ int main(int argc, char **argv)
         if (a.pen2)
             wfagpu_launch_alignments_affine2p(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results,
                                               opt, a.cigar, a.check, &pen2);
-        else if (a.ends_free)
-            wfagpu_launch_alignments_span(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt,
-                                          a.cigar, a.check, &span);
+        else if (a.ends_free || a.coords)
+            wfagpu_launch_alignments_span_coords(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata,
+                                                 results, opt, a.cigar, a.check, a.ends_free ? &span : NULL, coords);
         else if (a.cigar) launch_alignments(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt, a.check);
         else launch_alignments_distance(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results, opt, a.check);
         t_align += now_s() - t0;
@@ -327,13 +334,16 @@ int main(int argc, char **argv)
                     fprintf(fp, "NA\t\n");
                     continue;
                 }
+                fprintf(fp, "%d\t%s", -(int)results[i].error, cigar);
+                if (coords)
+                    fprintf(fp, "\t%d\t%d\t%d\t%d", coords[i].pattern_begin, coords[i].pattern_end, coords[i].text_begin,
+                            coords[i].text_end);
                 if (a.verbose)
-                    fprintf(fp, "%d\t%s\t%s\t%s\n", -(int)results[i].error, cigar, A->sequences_buffer + m->pattern_offset,
-                            A->sequences_buffer + m->text_offset);
-                else
-                    fprintf(fp, "%d\t%s\n", -(int)results[i].error, cigar);
+                    fprintf(fp, "\t%s\t%s", A->sequences_buffer + m->pattern_offset, A->sequences_buffer + m->text_offset);
+                fputc('\n', fp);
             }
         }
+        free(coords);
         destroy_wfa_results(results, (size_t)pairs);
         total += pairs;
         pairs = 0;

@@ -509,7 +509,8 @@ static int choose_large_cfg(wfagpu_device *d, const Slot &s, int n_want, size_t 
 static int choose_cfg(wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan, int n_want, int n_min, size_t n_items,
                       bool ascii, LaunchCfg *c)
 {
-    /* 2-piece: one diagonal per thread, decision bytes, no schedule records; two more rings of e2 + 1 rows */
+    /* 2-piece: one diagonal per thread, decision bytes, no schedule records; two more rings of e2 + 1 rows.  Score-only
+     * ends-free with coordinates: an origin row beside every ring row */
     const bool p2 = plan.e2 > 0, sched = !p2, bt = plan.with_cigar != 0;
     const RingDepths rd = ring_depths(plan);
     const int A = rd.A, E1 = rd.E1, G = A, E2 = rd.E2;
@@ -519,10 +520,10 @@ static int choose_cfg(wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan
     c->A = A; c->E1 = E1; c->G = G; c->E2 = E2; c->seq_words = seq_words;
     c->ring_m = A; c->ring_g = E1;
     KernelChoice &kc = c->k;
-    kc.ascii = ascii; kc.bt = bt; kc.ef = s.ef; kc.p2 = p2;
+    kc.ascii = ascii; kc.bt = bt; kc.ef = s.ef; kc.p2 = p2; kc.org = s.ef && !bt && plan.with_ends;
     n_want = std::max(1, n_want);
     if (d->force_large || s.max_len >= (1u << 15) ||
-        exact_smem_bytes(A, E1, ring_stride(n_want, G, false), seq_words, 1, 1, sched, E2) > smem_max)
+        exact_smem_bytes(A, E1, ring_stride(n_want, G, false), seq_words, 1, 1, sched, E2, kc.org) > smem_max)
         return choose_large_cfg(d, s, n_want, n_items, c);
     bool warp = (ring_stride(n_want, G, false) <= 400) && s.max_len <= 1024;
     if (d->force_warp >= 0) warp = d->force_warp != 0;
@@ -534,10 +535,10 @@ static int choose_cfg(wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan
         c->n_cap = n_want;
         c->row_stride = ring_stride(c->n_cap, G, false);
         c->center = ring_center(c->n_cap, G, false);
-        c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages, false, E2);
+        c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages, false, E2, kc.org);
         while (c->smem > smem_max && c->groups_per_cta > 1) {
             c->groups_per_cta >>= 1;
-            c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages, false, E2);
+            c->smem = exact_smem_bytes(A, E1, c->row_stride, seq_words, c->groups_per_cta, c->stages, false, E2, kc.org);
         }
         if (c->smem > smem_max) warp = false;
     }
@@ -580,26 +581,26 @@ static int choose_cfg(wfagpu_device *d, const Slot &s, const wfagpu_plan_t &plan
             const size_t budget = std::min(smem_max, smem_sm / k - 1024);
             for (int st = 2; st >= 1; --st) {
                 if (d->force_stages && st != d->force_stages) continue;
-                if (!fits(k, exact_smem_bytes(RA, RE, rs(n_min), seq_words, 1, st, sched, E2), budget)) continue;
+                if (!fits(k, exact_smem_bytes(RA, RE, rs(n_min), seq_words, 1, st, sched, E2, kc.org), budget)) continue;
                 int lo = n_min, hi = n_want;             /* widest rings that still fit k CTAs */
                 while (lo < hi) {
                     const int mid = (lo + hi + 1) / 2;
-                    if (fits(k, exact_smem_bytes(RA, RE, rs(mid), seq_words, 1, st, sched, E2), budget)) lo = mid; else hi = mid - 1;
+                    if (fits(k, exact_smem_bytes(RA, RE, rs(mid), seq_words, 1, st, sched, E2, kc.org), budget)) lo = mid; else hi = mid - 1;
                 }
                 best_k = k; stages = st; n_cap = lo;
-                smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, st, sched, E2);
+                smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, st, sched, E2, kc.org);
                 break;
             }
         }
         if (!best_k) {
             /* does not fit even alone: hold as many diagonals as one CTA can */
             stages = 1;
-            const size_t fixed = exact_smem_bytes(RA, RE, 0, seq_words, 1, stages, sched, E2);
-            const int rows_q = RA + 2 * RE + 2 * E2;
+            const size_t fixed = exact_smem_bytes(RA, RE, 0, seq_words, 1, stages, sched, E2, kc.org);
+            const int rows_q = (RA + 2 * RE + 2 * E2) * (kc.org ? 2 : 1);
             if (fixed + (size_t)rows_q * rs(1) * 2 > smem_max) return -2;   /* the sequences alone do not fit */
             n_cap = (int)((smem_max - fixed - 64) / ((size_t)rows_q * 4)) - 2 * G - (ck ? 16 : 2);
             if (n_cap < 1) return -2;
-            smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, stages, sched, E2);
+            smem = exact_smem_bytes(RA, RE, rs(n_cap), seq_words, 1, stages, sched, E2, kc.org);
             best_k = 1;
         }
         c->stages = stages;
@@ -1080,7 +1081,7 @@ static int size_arenas(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, con
         s.budget_cache = arena_budget;
     }
     const size_t groups = (size_t)c.ctas * c.groups_per_cta;
-    a.gring_elems = c.k.gring ? (uint64_t)(c.A + 2 * c.E1 + 2 * c.E2) * (uint64_t)c.row_stride : 0;
+    a.gring_elems = c.k.gring ? (uint64_t)(c.A + 2 * c.E1 + 2 * c.E2) * (c.k.org ? 2u : 1u) * (uint64_t)c.row_stride : 0;
     if (s.gring.ensure(groups * a.gring_elems + 1)) return -1;
     a.scratch_words = plan.with_cigar ? (uint32_t)((2 * (size_t)a.d_end + 31) / 16 + 2) : 1;
     a.arenas = per_pair ? a.items_per_launch : groups;
@@ -1583,6 +1584,7 @@ extern "C" int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n
     d->no_bound = true; d->no_quad = true; d->use_hint = false; d->force_warp = 0; d->independent = true;
     wfagpu_plan_t p2 = *plan;
     p2.with_cigar = 0;
+    p2.with_ends = 0;
     std::vector<wfagpu_pair_out_t> out(n);
     int rc = wfagpu_device_align_span(d, slot, n, &p2, 1, span);
     if (!rc) rc = wfagpu_device_download(d, slot, n, out.data(), nullptr, nullptr, nullptr);

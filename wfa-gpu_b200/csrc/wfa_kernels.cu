@@ -488,13 +488,21 @@ struct NoPiece2 {};
  * EF (ends-free, DESIGN.md §9): score 0 holds the extend of (max(0, -k), max(0, k)) on every diagonal of
  * [-pb, tb]; the pruning measures the distance to the target range [kt - te, kt + pe] instead of kt; an M cell on
  * a target diagonal finishes when its offset reaches min(tlen, plen + k), the lowest such k of the first finishing
- * score wins; the traceback starts there and stops at score 0.  k_begin / k_end go to p.ends[idx]. */
-template <bool WARP, bool ASCII, bool BT, typename R, bool CKPT, bool EF = false, bool P2 = false>
+ * score wins; the traceback starts there and stops at score 0.  k_begin / k_end go to p.ends[idx].
+ *
+ * ORG (score-only ends-free with coordinates, DESIGN.md §9): every M, I and D cell also stores the origin of its value,
+ * the score-0 diagonal its path started on, in an origin row at a fixed byte offset (the value rows' size) from its
+ * value row.  The origin follows the winner the decision byte of the CIGAR kernel records (I / D: extend beats open;
+ * M: D > X > I), so the origin of the finishing cell is the traceback's k_begin, ties included.  Only a winner's
+ * origin is read and a winner with a valid offset always has a written origin: origin rows need no prologue and no
+ * NULL stores (tests/endsfree_origin_model.py checks this with poisoned origin cells). */
+template <bool WARP, bool ASCII, bool BT, typename R, bool CKPT, bool EF = false, bool P2 = false, bool ORG = false>
 __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_kernel(const __grid_constant__ KernelParams p)
 {
     static_assert(!CKPT || (BT && !WARP && R::kElem == 2), "checkpointed traceback: CTA groups with shared-memory rings");
     static_assert(!(EF && CKPT), "ends-free: decision-byte traceback only");
     static_assert(!(P2 && (CKPT || EF)), "gap-affine 2-piece: global alignment, decision-byte traceback only");
+    static_assert(!ORG || (EF && !BT && !CKPT && !P2), "origins: score-only ends-free only");
     using G = Group<WARP>;
     using RA = typename R::addr_t;
     constexpr bool GR = (R::kElem == 4);          /* rings in global memory */
@@ -510,7 +518,8 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
     /* ---- carve shared memory: [rings][sequence stages][ctl] per group ---- */
     const int rows = p.A + 2 * p.E1 + (P2 ? 2 * p.E2 : 0);
     const uint32_t row_bytes = (uint32_t)p.row_stride * R::kElem;
-    const uint32_t ring_bytes = GR ? 0u : (((uint32_t)rows * row_bytes + 15u) & ~15u);
+    const uint32_t org_off = (uint32_t)rows * row_bytes;          /* ORG: origin row = value row + org_off */
+    const uint32_t ring_bytes = GR ? 0u : (((ORG ? 2u : 1u) * org_off + 15u) & ~15u);
     const uint32_t seq_bytes = (uint32_t)p.seq_words * 4u;          /* one sequence, one stage */
     const uint32_t seq_total = ASCII ? 0u : 2u * (uint32_t)p.stages * seq_bytes;
     const uint32_t group_bytes = (ring_bytes + seq_total + (uint32_t)sizeof(GroupCtl) + (SCHED ? kSchedBytes : 0u) + 15u) & ~15u;
@@ -634,6 +643,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
         int dist = 0;
         bool finished = false;
         int k_end = kt;                              /* ends-free: diagonal of the finishing cell */
+        int k_org = 0;                               /* ORG: origin of the finishing cell (score > 0) */
         /* ends-free end test: the lowest finishing diagonal of the group (kb = INT_MAX: none on this thread); also the
          * barrier after the score's cells */
         auto ef_lowest = [&](int kb) -> int {
@@ -703,6 +713,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                     for (int k = slo + tid; k <= shi; k += gsz) {
                         const int m = extend(k, max(0, k));
                         R::st(M0, k, m);
+                        if constexpr (ORG) R::st(R::add(M0, org_off), k, k);
                         if (k >= klo_t && k <= khi_t && m == min(tlen, plen + k)) kb = min(kb, k);
                     }
                 } else {
@@ -850,6 +861,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                                 m = R::ld(aMx, k) + 1;
                                 if (m >= 0) m = extend(k, m);
                                 if (EF && k >= klo_t && k <= khi_t && m == min(tlen, plen + k)) kb = min(kb, k);
+                                if constexpr (ORG) R::st(R::add(aMc, org_off), k, R::ld(R::add(aMx, org_off), k));
                             }
                             R::st(aMc, k, m);
                         }
@@ -912,6 +924,15 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                             R::st(aDc, k, D);
                             R::st(aMc, k, M);
                             if (BT && !CKPT) rowb[k] = (uint8_t)((bI ? 1u : 0u) | (bD ? 2u : 0u) | (bM0 ? 4u : 0u) | (bM1 ? 8u : 0u));
+                            if constexpr (ORG) {
+                                /* the origin of the winner the decision byte would record */
+                                const int oI = R::ld(R::add(bI ? aIe : aMo, org_off), k - 1);
+                                const int oD = R::ld(R::add(bD ? aDe : aMo, org_off), k + 1);
+                                const int oM = bM1 ? (bM0 ? oD : R::ld(R::add(aMx, org_off), k)) : oI;
+                                R::st(R::add(aIc, org_off), k, oI);
+                                R::st(R::add(aDc, org_off), k, oD);
+                                R::st(R::add(aMc, org_off), k, oM);
+                            }
                             if (EF && k >= klo_t && k <= khi_t && M == min(tlen, plen + k)) kb = min(kb, k);
                         }
                     }
@@ -921,6 +942,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                             finished = true;
                             dist = d;
                             k_end = kb;
+                            if constexpr (ORG) k_org = R::ld(R::add(aMc, org_off), kb);
                             break;
                         }
                     } else {
@@ -941,7 +963,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
         uint32_t n_ops = 0;
         if (tid == 0) {
             uint32_t ops_off = 0;
-            int k_begin = k_end;                     /* ends-free: diagonal of the path's score-0 cell */
+            int k_begin = (ORG && dist > 0) ? k_org : k_end;    /* ends-free: diagonal of the path's score-0 cell */
             if (BT && finished && dist > 0) {
               if constexpr (!CKPT) {
                 int cd = dist, ck = EF ? k_end : kt, comp = 0;
@@ -3213,9 +3235,10 @@ int max_ctas_per_sm(kernel_fn kfn, int threads, size_t smem)
     return n;
 }
 
-size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched, int E2)
+size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched, int E2,
+                        bool org)
 {
-    const int rows = A + 2 * E1 + 2 * E2;
+    const int rows = (A + 2 * E1 + 2 * E2) * (org ? 2 : 1);
     const size_t ring_bytes = ((size_t)rows * row_stride * sizeof(int16_t) + 15) & ~(size_t)15;
     const size_t seq_bytes = (size_t)seq_words * 4;
     const size_t group_bytes = (ring_bytes + 2 * (size_t)stages * seq_bytes + sizeof(GroupCtl) + (sched ? kSchedBytes : 0) + 15) & ~(size_t)15;
@@ -3261,10 +3284,17 @@ int traceback_max_ctas_per_sm(int A, int period, int warps, bool ascii)
     return max_ctas_per_sm(traceback_fn(ascii, period), 32 * warps, traceback_smem_bytes(A, period, warps));
 }
 
-/* wfa_exact_kernel of one tier (WARP, Ring) in the batch's mode: ends-free, 2-piece or single-piece global */
+/* wfa_exact_kernel of one tier (WARP, Ring) in the batch's mode: ends-free (score only: with or without origins),
+ * 2-piece or single-piece global */
 template <bool WARP, bool ASCII, bool BT, typename R>
 static kernel_fn exact_mode(const KernelChoice &k)
 {
+    if (k.org) {
+        if constexpr (!BT) {
+            if (k.ef && !k.p2) return wfa_exact_kernel<WARP, ASCII, false, R, false, true, false, true>;
+        }
+        return nullptr;
+    }
     if (k.ef) return wfa_exact_kernel<WARP, ASCII, BT, R, false, true>;
     if (k.p2) return wfa_exact_kernel<WARP, ASCII, BT, R, false, false, true>;
     return wfa_exact_kernel<WARP, ASCII, BT, R, false>;
@@ -3284,6 +3314,7 @@ static kernel_fn exact_fn(const KernelChoice &k)
 
 kernel_fn wavefront_kernel(const KernelChoice &k, bool count_cells)
 {
+    if (k.org && (k.family != Family::Exact || k.ckpt)) return nullptr;    /* origins: the exact kernel's ends-free rings */
     switch (k.family) {
     case Family::Exact:
         if (k.ascii) return k.bt ? exact_fn<true, true>(k) : exact_fn<true, false>(k);

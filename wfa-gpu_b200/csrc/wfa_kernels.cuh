@@ -142,6 +142,7 @@ struct KernelChoice {
     bool ckpt = false;    /* ring snapshots for wfa_traceback_kernel instead of decision bytes */
     bool ef = false;      /* exact: ends-free (decision-byte traceback on every tier) */
     bool p2 = false;      /* exact: gap-affine 2-piece (likewise) */
+    bool org = false;     /* exact, ends-free, score only: origin rows carry each alignment's start diagonal to p.ends */
     int threads = 0;      /* threads per CTA; QuadG picks its register budget (MAXT) from it */
     bool quad() const { return family == Family::Quad || family == Family::QuadG || family == Family::BandQ; }
 };
@@ -164,9 +165,9 @@ cudaError_t launch_traceback(const KernelParams &p, int ctas, int warps, bool as
 size_t traceback_smem_bytes(int A, int period, int warps);
 int traceback_max_ctas_per_sm(int A, int period, int warps, bool ascii_extend);
 /* sched: CTA-per-pair kernels with shared-memory rings keep per-score schedule records (3 KB; not the 2-piece kernels).
- * E2 > 0: the two extra I2 / D2 rings of a 2-piece launch */
+ * E2 > 0: the two extra I2 / D2 rings of a 2-piece launch.  org: every ring row has an origin row (KernelChoice::org) */
 size_t exact_smem_bytes(int A, int E1, int row_stride, int seq_words, int groups_per_cta, int stages, bool sched = false,
-                        int E2 = 0);
+                        int E2 = 0, bool org = false);
 size_t banded_smem_bytes(int A, int win, int seq_words, int stages);
 size_t bandq_smem_bytes(int A, int win, int seq_words, int stages);
 /* decision bytes of wfa_bandq_kernel -> 2-bit ops, one thread per pair of the launch */

@@ -245,6 +245,11 @@ bool wfagpu_align(wfagpu_aligner_t *aligner)
 
 bool wfagpu_align_span(wfagpu_aligner_t *aligner, const wfagpu_span_t *span)
 {
+    return wfagpu_align_span_coords(aligner, span, NULL);
+}
+
+bool wfagpu_align_span_coords(wfagpu_aligner_t *aligner, const wfagpu_span_t *span, wfagpu_coords_t *coords)
+{
     if (!aligner) { ERR("Invalid aligner."); return false; }
     if (!aligner->results || !aligner->sequences_metadata) { ERR("Aligner parameters are not initialized."); return false; }
     if (span && (span->pattern_begin_free < 0 || span->pattern_end_free < 0 || span->text_begin_free < 0 ||
@@ -258,9 +263,9 @@ bool wfagpu_align_span(wfagpu_aligner_t *aligner, const wfagpu_span_t *span)
         ERR("Ends-free alignment cannot be combined with the adaptive band.");
         return false;
     }
-    wfagpu_launch_alignments_span(aligner->sequences_buffer, aligner->sequences_buffer_len, aligner->sequences_metadata,
-                                  aligner->results, aligner->alignment_options,
-                                  aligner->alignment_options.compute_cigar, false, ef ? span : NULL);
+    wfagpu_launch_alignments_span_coords(aligner->sequences_buffer, aligner->sequences_buffer_len,
+                                         aligner->sequences_metadata, aligner->results, aligner->alignment_options,
+                                         aligner->alignment_options.compute_cigar, false, ef ? span : NULL, coords);
     return wfagpu_last_launch_ok();
 }
 

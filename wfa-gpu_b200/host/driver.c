@@ -115,6 +115,7 @@ typedef struct {
     wfagpu_span_t span;
     bool p2;                /* gap-affine 2-piece call: `pen2` replaces opt.penalties */
     wfagpu_affine2p_t pen2;
+    wfagpu_coords_t *coords;  /* the caller's, one per pair, or NULL */
     int decode_threads;
     /* accumulated */
     wfagpu_run_stats_t stats;
@@ -137,7 +138,7 @@ typedef struct {
     size_t pairs_cap;
     wfagpu_pair_out_t *out;
     size_t out_cap;
-    int32_t *ends;          /* ends-free, CIGAR text on the host: {k_begin, k_end} per pair */
+    int32_t *ends;          /* ends-free, CIGAR text on the host or coordinates: {k_begin, k_end} per pair */
 } inflight_t;
 
 static double now_s(void)
@@ -276,6 +277,17 @@ static void fill_plan(const job_t *j, bool cigar, wfagpu_plan_t *plan)
     plan->threads_hint = j->opt.threads_per_block;
     plan->workers_hint = j->opt.num_workers;
     if (j->p2) { plan->o2 = j->pen2.o2; plan->e2 = j->pen2.e2; }
+    plan->with_ends = j->ef && j->coords;
+}
+
+/* wfagpu_coords_t of a finished pair from its {k_begin, k_end} (NULL: a global alignment covers both sequences) */
+static wfagpu_coords_t coords_of(const sequence_pair_t *m, const int32_t *ends)
+{
+    const int plen = (int)m->pattern_len, tlen = (int)m->text_len;
+    if (!ends) return (wfagpu_coords_t){0, plen, 0, tlen};
+    const int kb = ends[0], ke = ends[1];
+    const int te = tlen < plen + ke ? tlen : plen + ke;
+    return (wfagpu_coords_t){kb < 0 ? -kb : 0, te - ke, kb > 0 ? kb : 0, te};
 }
 
 static int submit(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
@@ -384,8 +396,9 @@ static int collect(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f, wfagpu
     if (j->cigar && !j->host_cigar) {
         if (wfagpu_device_download_text(d, slot, f->n, &text, &text_bytes, &refs)) return -1;
         wfagpu_device_last_stats(d, slot, &bs);
-    } else if (j->cigar && j->ef) {
-        /* the host decoder needs the diagonal every alignment starts on */
+    }
+    if (j->ef && (j->coords || (j->cigar && j->host_cigar))) {
+        /* the coordinates and the host decoder need the diagonals every alignment starts and ends on */
         free(f->ends);
         f->ends = (int32_t *)malloc(2 * f->n * sizeof(int32_t));
         if (!f->ends || wfagpu_device_download_ends(d, slot, f->n, f->ends)) return -1;
@@ -409,6 +422,7 @@ static int collect(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f, wfagpu
         }
         if (!(o->status & WFAGPU_ST_FINISHED)) { bad++; continue; }
         res[i].error = (unsigned int)o->distance;
+        if (j->coords) j->coords[f->from + (size_t)i] = coords_of(&m[i], j->ef ? f->ends + 2 * i : NULL);
         if (j->cigar && refs) {
             /* text was printed on the GPU: append it to the caller's buffer */
             if (!wfagpu_cigar_append(&res[i].cigar, text + refs[i].off, refs[i].len)) bad++;
@@ -509,7 +523,7 @@ void wfagpu_plan_chunks(size_t n, size_t batch_size, int n_devices, size_t ascii
 
 static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_alignment_result_t *res,
                     wfa_alignment_options_t opt, bool cigar, bool check, const wfagpu_span_t *ends_free,
-                    const wfagpu_affine2p_t *affine2p)
+                    const wfagpu_affine2p_t *affine2p, wfagpu_coords_t *coords)
 {
     const double t0 = now_s();
     memset(&t_last_stats, 0, sizeof(t_last_stats));
@@ -560,6 +574,9 @@ static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_align
     if (ef) job.span = *sp;
     job.p2 = affine2p != NULL;
     if (affine2p) job.pen2 = *affine2p;
+    job.coords = coords;
+    if (coords)
+        for (size_t i = 0; i < opt.num_alignments; ++i) coords[i] = (wfagpu_coords_t){-1, -1, -1, -1};   /* until aligned */
     job.n = opt.num_alignments;
     job.pageable = !wfagpu_host_is_pinned(buf);
     const size_t span = meta[job.n - 1].text_offset + meta[job.n - 1].text_len + 1 - meta[0].pattern_offset;
@@ -652,7 +669,7 @@ void launch_alignments(char *sequences_buffer, const size_t sequences_buffer_siz
                        wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, true,
-            check_correctness, NULL, NULL);
+            check_correctness, NULL, NULL, NULL);
 }
 
 void launch_alignments_distance(char *sequences_buffer, const size_t sequences_buffer_size,
@@ -661,7 +678,7 @@ void launch_alignments_distance(char *sequences_buffer, const size_t sequences_b
                                 wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, false,
-            check_correctness, NULL, NULL);
+            check_correctness, NULL, NULL, NULL);
 }
 
 void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buffer_size,
@@ -670,7 +687,16 @@ void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buff
                                    const wfagpu_span_t *span)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
-            check_correctness, span, NULL);
+            check_correctness, span, NULL, NULL);
+}
+
+void wfagpu_launch_alignments_span_coords(char *sequences_buffer, size_t sequences_buffer_size,
+                                          sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                          wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                          const wfagpu_span_t *span, wfagpu_coords_t *coords)
+{
+    run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
+            check_correctness, span, NULL, coords);
 }
 
 void wfagpu_launch_alignments_affine2p(char *sequences_buffer, size_t sequences_buffer_size,
@@ -679,5 +705,5 @@ void wfagpu_launch_alignments_affine2p(char *sequences_buffer, size_t sequences_
                                        const wfagpu_affine2p_t *pen)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
-            check_correctness, NULL, pen);
+            check_correctness, NULL, pen, NULL);
 }

@@ -61,7 +61,8 @@ class Step(C.Structure):
 class Plan(C.Structure):
     _fields_ = [("x", C.c_int), ("o", C.c_int), ("e", C.c_int), ("max_steps", C.c_int), ("band", C.c_int),
                 ("band_width", C.c_int), ("with_cigar", C.c_int), ("threads_hint", C.c_int), ("workers_hint", C.c_int),
-                ("o2", C.c_int), ("e2", C.c_int)]      # gap-affine 2-piece: second piece; e2 = 0 (default): one piece
+                ("o2", C.c_int), ("e2", C.c_int),      # gap-affine 2-piece: second piece; e2 = 0 (default): one piece
+                ("with_ends", C.c_int)]                # ends-free score only: also find k_begin (default 0: no)
 
 
 class PairOut(C.Structure):
@@ -88,6 +89,11 @@ class Affine2p(C.Structure):
     _fields_ = [("x", C.c_int), ("o1", C.c_int), ("e1", C.c_int), ("o2", C.c_int), ("e2", C.c_int)]
 
 
+class Coords(C.Structure):
+    """wfagpu_coords_t: the aligned part, pattern[pattern_begin, pattern_end) against text[text_begin, text_end)."""
+    _fields_ = [("pattern_begin", C.c_int), ("pattern_end", C.c_int), ("text_begin", C.c_int), ("text_end", C.c_int)]
+
+
 class DevPair(C.Structure):
     _fields_ = [("p_ascii", C.c_uint32), ("t_ascii", C.c_uint32), ("p_word", C.c_uint32), ("t_word", C.c_uint32),
                 ("plen", C.c_uint32), ("tlen", C.c_uint32), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
@@ -112,6 +118,7 @@ EXPORTS = [
     "wfagpu_device_download_ends", "wfagpu_device_rescore_span", "wfagpu_ops_to_cigar_span",
     "wfagpu_check_result_span", "wfagpu_build_step_table_span", "wfagpu_align_affine2p",
     "wfagpu_launch_alignments_affine2p", "wfagpu_check_result_affine2p", "wfagpu_build_step_table_affine2p",
+    "wfagpu_align_span_coords", "wfagpu_launch_alignments_span_coords",
 ]
 
 _lib = None
@@ -224,6 +231,11 @@ def load():
                                                C.c_char_p]
     L.wfagpu_check_result_affine2p.restype = C.c_bool
     L.wfagpu_build_step_table_affine2p.argtypes = [C.c_int] * 7 + [P(Step), P(C.c_uint64)]
+    L.wfagpu_align_span_coords.argtypes = [P(AlignerStruct), P(Span), P(Coords)]
+    L.wfagpu_align_span_coords.restype = C.c_bool
+    L.wfagpu_launch_alignments_span_coords.argtypes = [C.c_void_p, C.c_size_t, P(SequencePair), P(AlignmentResult),
+                                                       AlignmentOptions, C.c_bool, C.c_bool, P(Span), P(Coords)]
+    L.wfagpu_launch_alignments_span_coords.restype = None
     _lib = L
     return L
 
@@ -261,6 +273,7 @@ class Aligner:
         if not self.L.wfagpu_initialize_aligner(C.byref(self.s)):
             raise RuntimeError("wfagpu_initialize_aligner failed")
         self._alive = True
+        self._coords = None
 
     # -- reference API -------------------------------------------------------
     def add_sequences(self, query, target):
@@ -276,18 +289,29 @@ class Aligner:
     def options(self):
         return self.s.alignment_options
 
-    def align(self, ends_free=None, affine2p=None):
+    def align(self, ends_free=None, affine2p=None, coords=False):
         """ends_free: None (global) or (pattern_begin_free, pattern_end_free, text_begin_free, text_end_free),
         WFA2-lib's order: that many leading / trailing bases of either sequence are free (wfagpu_align_span).
         affine2p: None or (x, o1, e1, o2, e2), gap-affine 2-piece penalties for this call in place of the aligner's
-        (wfagpu_align_affine2p); global alignment only."""
+        (wfagpu_align_affine2p); global alignment only.
+        coords: also record where every alignment lies, with or without a CIGAR (wfagpu_align_span_coords); read
+        them with coords().  Not with affine2p."""
         sp = span_of(ends_free)
         pen2 = affine2p_of(affine2p)
+        self._coords = None
         if pen2 is not None:
             if sp is not None:
                 raise ValueError("affine2p cannot be combined with ends_free")
+            if coords:
+                raise ValueError("affine2p cannot be combined with coords")
             if not self.L.wfagpu_align_affine2p(C.byref(self.s), C.byref(pen2)):
                 raise RuntimeError("wfagpu_align_affine2p failed (see stderr); there is no CPU fallback")
+            return True
+        if coords:
+            cs = (Coords * self.num_pairs)()
+            if not self.L.wfagpu_align_span_coords(C.byref(self.s), C.byref(sp) if sp is not None else None, cs):
+                raise RuntimeError("wfagpu_align_span_coords failed (see stderr); there is no CPU fallback")
+            self._coords = cs
             return True
         if sp is None:
             if not self.L.wfagpu_align(C.byref(self.s)):
@@ -325,6 +349,14 @@ class Aligner:
 
     def cigars(self):
         return [self.cigar(i) for i in range(self.num_pairs)]
+
+    def coords(self):
+        """(pattern_begin, pattern_end, text_begin, text_end) of every pair of the last align(coords=True): the
+        alignment covers pattern[pattern_begin:pattern_end] and text[text_begin:text_end]; all -1 for a pair that
+        was not aligned."""
+        if self._coords is None:
+            raise RuntimeError("no coordinates: call align(..., coords=True) first")
+        return [(c.pattern_begin, c.pattern_end, c.text_begin, c.text_end) for c in self._coords]
 
     def pair(self, i):
         m = self.s.sequences_metadata[i]

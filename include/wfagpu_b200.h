@@ -177,6 +177,11 @@ int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wfagpu_pair_o
  * provisioning hint of global batches.  -3 for negative values or band > 0 with a non-zero span. */
 int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident,
                              const wfagpu_span_t *span);
+/* The same with one span per pair of the batch (spans[i] for pair i; NULL: global).  The batch is ends-free when any
+ * pair's span is non-zero; every pair is aligned under its own span, and a pair with an all-zero span gets its global
+ * alignment.  -3 as above when any pair's span is rejected. */
+int wfagpu_device_align_spans(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident,
+                              const wfagpu_span_t *spans);
 /* After wfagpu_device_download of an ends-free batch: per pair {k_begin, k_end} (2 n ints), the diagonals of the
  * alignment's first and last cell: it starts at (max(0, -k_begin), max(0, k_begin)) and ends at offset
  * min(tlen, plen + k_end).  k_end is always valid; k_begin only when the batch was aligned with with_cigar or
@@ -285,6 +290,9 @@ int wfagpu_device_rescore(wfagpu_device_t *d, int slot, size_t n, const wfagpu_p
 /* The same for an ends-free span (NULL = global).  with_cigar and with_ends of the plan are ignored. */
 int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
                                const wfagpu_span_t *span, int32_t *scores);
+/* The same with one span per pair (spans[i] for pair i; NULL = global). */
+int wfagpu_device_rescore_spans(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
+                                const wfagpu_span_t *spans, int32_t *scores);
 
 /* Makes room for `bytes` more sequence bytes and `pairs` more pairs in one step (readers, generators). */
 bool wfagpu_reserve(wfagpu_aligner_t *aligner, size_t bytes, size_t pairs);
@@ -361,6 +369,17 @@ void wfagpu_launch_alignments_span_coords(char *sequences_buffer, size_t sequenc
                                           sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
                                           wfa_alignment_options_t options, bool cigar, bool check_correctness,
                                           const wfagpu_span_t *span, wfagpu_coords_t *coords);
+
+/* Per-pair spans: wfagpu_align_span_coords with spans[i] for pair i (num_sequence_pairs entries; honours compute_cigar;
+ * coords may be NULL).  Pairs with an all-zero span get their global alignment; all-zero spans or NULL: exactly
+ * wfagpu_align.  False, with a message, for a negative value, or for band > 0 with a non-zero span. */
+bool wfagpu_align_spans(wfagpu_aligner_t *aligner, const wfagpu_span_t *spans, wfagpu_coords_t *coords);
+/* wfagpu_launch_alignments_span_coords with spans[i] for pair i, indexed like sequences_metadata; check_correctness
+ * validates every CIGAR under its pair's span and re-computes every score with the same spans. */
+void wfagpu_launch_alignments_spans(char *sequences_buffer, size_t sequences_buffer_size,
+                                    sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                    wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                    const wfagpu_span_t *spans, wfagpu_coords_t *coords);
 
 /* The reference library's generic validators, same names, argument order (text first) and input format
  * (utils/verification.h:37-58): the op string may be UNROLLED ("MMXMMI", what the reference's recover_cigar

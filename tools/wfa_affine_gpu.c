@@ -18,6 +18,8 @@
  *   -c/--check                       validate every result: CIGAR on the host, score against an independent GPU pass
  *   -F/--ends-free P0,Pf,T0,Tf       ends-free alignment (WFA2-lib's order): that many leading / trailing pattern and
  *                                    text bases are free; not with -B
+ *   -E/--ends-free-file FILE         ends-free with a span per pair: one "P0,Pf,T0,Tf" line per pair, in input order
+ *                                    (as many lines as pairs read); not with -F, -B or -G
  *   -G/--affine2p-penalties x,o1,e1,o2,e2
  *                                    gap-affine 2-piece penalties (WFA2-lib's affine2p): a gap of L bases costs
  *                                    min(o1 + e1 L, o2 + e2 L); signs are stripped, e1, e2 >= 1; not with -g, -B or -F
@@ -39,7 +41,7 @@
 #include "wfagpu_b200.h"
 
 typedef struct {
-    const char *seq, *fq, *ft, *out, *pen, *devices, *ends_free, *pen2;
+    const char *seq, *fq, *ft, *out, *pen, *devices, *ends_free, *pen2, *span_file;
     long n, e, t, b, w, band, stream;
     int have_e, have_t, have_b, have_w, have_band, have_stream, cigar, check, print, verbose, coords;
 } args_t;
@@ -64,6 +66,7 @@ static void usage(void)
             "\t-B, --band L                    banded heuristic, re-centre every L scores (auto = 25)\n"
             "\t-c, --check                     check the alignments\n"
             "\t-F, --ends-free P0,Pf,T0,Tf     ends-free: free leading/trailing pattern (P) and text (T) bases\n"
+            "\t-E, --ends-free-file FILE       ends-free with one P0,Pf,T0,Tf line per pair, in input order\n"
             "\t-G, --affine2p-penalties x,o1,e1,o2,e2  gap-affine 2-piece: a gap of L costs min(o1+e1*L, o2+e2*L)\n"
             "[System]\n"
             "\t-t, --threads-per-block T       threads per alignment (band width with -B)\n"
@@ -82,6 +85,7 @@ static const struct { char s; const char *l; int has_val; } OPTS[] = {
     {'t', "threads-per-block", 1}, {'b', "batch-size", 1}, {'w', "workers", 1}, {'B', "band", 1},
     {'o', "output-file", 1}, {'p', "print-output", 0}, {'O', "output-verbose", 0}, {'D', "devices", 1},
     {'S', "stream", 1}, {'F', "ends-free", 1}, {'G', "affine2p-penalties", 1}, {'P', "print-coords", 0},
+    {'E', "ends-free-file", 1},
 };
 
 static int parse(int argc, char **argv, args_t *a)
@@ -109,6 +113,7 @@ static int parse(int argc, char **argv, args_t *a)
         case 'g': a->pen = val; break;
         case 'D': a->devices = val; break;
         case 'F': a->ends_free = val; break;
+        case 'E': a->span_file = val; break;
         case 'G': a->pen2 = val; break;
         case 'S': a->stream = atol(val); a->have_stream = 1; break;
         case 'n': a->n = atoll(val); break;
@@ -132,6 +137,42 @@ static double now_s(void)
     struct timespec ts;
     clock_gettime(CLOCK_MONOTONIC, &ts);
     return (double)ts.tv_sec + 1e-9 * (double)ts.tv_nsec;
+}
+
+/* -E: the spans of the next `n` pairs, one "P0,Pf,T0,Tf" line each (surrounding blanks allowed).  0, or -1 with a
+ * message for a missing, malformed or negative line. */
+static int read_spans(FILE *fp, const char *path, long first_pair, long n, wfagpu_span_t *spans)
+{
+    char line[256];
+    for (long i = 0; i < n; ++i) {
+        wfagpu_span_t *sp = &spans[i];
+        char tail = 0;
+        if (!fgets(line, sizeof(line), fp)) {
+            fprintf(stderr, "[!] ERROR: --ends-free-file %s has %ld line(s) but there are more pairs.\n", path, first_pair + i);
+            return -1;
+        }
+        if (sscanf(line, " %d , %d , %d , %d %c", &sp->pattern_begin_free, &sp->pattern_end_free, &sp->text_begin_free,
+                   &sp->text_end_free, &tail) != 4 ||
+            sp->pattern_begin_free < 0 || sp->pattern_end_free < 0 || sp->text_begin_free < 0 || sp->text_end_free < 0) {
+            line[strcspn(line, "\r\n")] = 0;
+            fprintf(stderr, "[!] ERROR: --ends-free-file %s line %ld: expected four values >= 0, P0,Pf,T0,Tf (got \"%s\").\n",
+                    path, first_pair + i + 1, line);
+            return -1;
+        }
+    }
+    return 0;
+}
+
+/* -E after the last pair: anything but blank lines left means the file does not match the input */
+static int spans_left_over(FILE *fp, const char *path, long pairs)
+{
+    char line[256];
+    while (fgets(line, sizeof(line), fp))
+        if (line[strspn(line, " \t\r\n")]) {
+            fprintf(stderr, "[!] ERROR: --ends-free-file %s has more lines than the %ld pairs read.\n", path, pairs);
+            return -1;
+        }
+    return 0;
 }
 
 /* ---- streaming: window w + 1 is read (into page-locked memory) by a helper thread while the GPU aligns window w ---- */
@@ -165,6 +206,15 @@ int main(int argc, char **argv)
 
     if (!parse(argc, argv, &a)) { usage(); return 1; }
     if (!a.seq && !(a.fq && a.ft)) { fprintf(stderr, "[!] ERROR: No input file provided.\n"); return 1; }
+    FILE *span_fp = NULL;
+    if (a.span_file) {
+        if (a.ends_free) { fprintf(stderr, "[!] ERROR: --ends-free-file cannot be combined with --ends-free (-F).\n"); return 1; }
+        if (a.have_band) { fprintf(stderr, "[!] ERROR: --ends-free-file cannot be combined with the band (-B).\n"); return 1; }
+        if (!a.pen2 && !(span_fp = fopen(a.span_file, "r"))) {
+            fprintf(stderr, "[!] ERROR: Could not open --ends-free-file %s\n", a.span_file);
+            return 1;
+        }
+    }
 
     /* -G: gap-affine 2-piece penalties instead of -g */
     wfagpu_affine2p_t pen2 = {0, 0, 0, 0, 0};
@@ -172,6 +222,7 @@ int main(int argc, char **argv)
         if (a.pen) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --affine-penalties (-g).\n"); return 1; }
         if (a.have_band) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with the band (-B).\n"); return 1; }
         if (a.ends_free) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --ends-free (-F).\n"); return 1; }
+        if (a.span_file) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --ends-free-file (-E).\n"); return 1; }
         if (a.coords) { fprintf(stderr, "[!] ERROR: --affine2p-penalties cannot be combined with --print-coords (-P).\n"); return 1; }
         if (sscanf(a.pen2, "%d,%d,%d,%d,%d", &pen2.x, &pen2.o1, &pen2.e1, &pen2.o2, &pen2.e2) != 5) {
             fprintf(stderr, "[!] ERROR: --affine2p-penalties takes five values: x,o1,e1,o2,e2 (got %s).\n", a.pen2);
@@ -297,6 +348,9 @@ int main(int argc, char **argv)
         }
         wfagpu_coords_t *coords = a.coords ? (wfagpu_coords_t *)malloc((size_t)pairs * sizeof(wfagpu_coords_t)) : NULL;
         if (a.coords && !coords) { fprintf(stderr, "[!] ERROR: Can not allocate the coordinates.\n"); return -1; }
+        wfagpu_span_t *spans = span_fp ? (wfagpu_span_t *)malloc((size_t)pairs * sizeof(wfagpu_span_t)) : NULL;
+        if (span_fp && (!spans || read_spans(span_fp, a.span_file, total, pairs, spans))) return -1;
+        if (span_fp && !more && spans_left_over(span_fp, a.span_file, total + pairs)) return -1;   /* the last window */
         wfa_alignment_options_t opt;
         memset(&opt, 0, sizeof(opt));
         opt.max_error = max_distance;
@@ -313,6 +367,9 @@ int main(int argc, char **argv)
         if (a.pen2)
             wfagpu_launch_alignments_affine2p(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results,
                                               opt, a.cigar, a.check, &pen2);
+        else if (spans)
+            wfagpu_launch_alignments_spans(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata, results,
+                                           opt, a.cigar, a.check, spans, coords);
         else if (a.ends_free || a.coords)
             wfagpu_launch_alignments_span_coords(A->sequences_buffer, A->sequences_buffer_len, A->sequences_metadata,
                                                  results, opt, a.cigar, a.check, a.ends_free ? &span : NULL, coords);
@@ -344,6 +401,7 @@ int main(int argc, char **argv)
             }
         }
         free(coords);
+        free(spans);
         destroy_wfa_results(results, (size_t)pairs);
         total += pairs;
         pairs = 0;
@@ -354,6 +412,8 @@ int main(int argc, char **argv)
             cur ^= 1;
         }
     }
+    if (span_fp && ok_run && spans_left_over(span_fp, a.span_file, total)) return -1;
+    if (span_fp) fclose(span_fp);
     printf("Alignment computed. Wall time: %.3fs (%.3f alignments per second)\n", t_align, (double)total / t_align);
     fprintf(stderr, "INFO: %d GPU(s), %llu kernel launches, %llu pairs re-dispatched on the GPU, %llu byte-compare pairs\n",
             sum.devices, (unsigned long long)sum.launches, (unsigned long long)sum.redispatched,

@@ -177,9 +177,10 @@ struct Slot {
     uint32_t max_len = 0;
     uint32_t kt_max = 0;               /* largest |tlen - plen| of the batch */
     uint32_t minlen_max = 0;           /* largest min(plen, tlen) of the batch */
-    /* ends-free batch (wfagpu_device_align_span with a non-zero span) */
+    /* ends-free batch (wfagpu_device_align_span(s) with a non-zero span for some pair) */
     bool ef = false;
-    wfagpu_span_t span{};
+    DevBuf<int4> spans;                /* per pair {pb, pe, tb, te}, each clamped to the sequence it applies to */
+    PinBuf<int4> h_spans;
     int ef_w = 0;                      /* half width of the start row: max(pb, tb), at most the longest sequence */
     int ef_ext = 0;                    /* widest end of the target range: max(pe, te), likewise */
     bool plain = true;                 /* global single-piece batch (neither ends-free nor 2-piece): it reads and learns the
@@ -364,6 +365,7 @@ extern "C" void wfagpu_device_close_all(void)
             s.h_text.release(); s.h_refs.release(); s.h_heads.release(); s.h_ascii.release();
             s.h_pairs.release(); s.h_order.release(); s.h_seed.release(); s.h_out.release(); s.h_pool.release();
             s.h_counters.release(); s.h_cells.release(); s.h_steps.release(); s.ends.release(); s.h_ends.release();
+            s.spans.release(); s.h_spans.release();
             for (auto &ev : s.ev) if (ev) cudaEventDestroy(ev);
             if (s.ev_tab) cudaEventDestroy(s.ev_tab);
             if (s.stream) cudaStreamDestroy(s.stream);
@@ -1168,8 +1170,7 @@ static int enqueue_pass(wfagpu_device *d, Slot &s, const wfagpu_plan_t &plan, co
     kp.ascii_count = s.counters.p + CTR_ASCII;
     kp.cells = d->count_cells ? s.cells.p : nullptr;
     if (s.ef) {
-        kp.ef_pb = s.span.pattern_begin_free; kp.ef_pe = s.span.pattern_end_free;
-        kp.ef_tb = s.span.text_begin_free; kp.ef_te = s.span.text_end_free;
+        kp.spans = s.spans.p;
         kp.ends = s.ends.p;
     }
     if (plan.e2 > 0) { kp.o2 = plan.o2; kp.e2 = plan.e2; kp.E2 = c.E2; }
@@ -1326,18 +1327,21 @@ extern "C" int wfagpu_device_align(wfagpu_device_t *d, int slot, size_t n, const
     return wfagpu_device_align_span(d, slot, n, plan, resident, nullptr);
 }
 
-extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident,
-                                        const wfagpu_span_t *span)
+/* The span of pair i is spans[i * stride] (stride 0: one span for the batch); spans = NULL: global. */
+static int align_spans(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, const wfagpu_span_t *spans,
+                       size_t stride)
 {
-    (void)resident;
     if (!d || slot < 0 || slot > 1 || !plan) return -1;
-    const wfagpu_span_t sp = span ? *span : wfagpu_span_t{0, 0, 0, 0};
-    if (sp.pattern_begin_free < 0 || sp.pattern_end_free < 0 || sp.text_begin_free < 0 || sp.text_end_free < 0) {
-        fprintf(stderr, "[wfagpu] ends-free span values must be >= 0 (got %d,%d,%d,%d)\n", sp.pattern_begin_free,
-                sp.pattern_end_free, sp.text_begin_free, sp.text_end_free);
-        return -3;
+    bool ef = false;
+    for (size_t i = 0; spans && i < (stride ? n : 1); ++i) {
+        const wfagpu_span_t &sp = spans[i * stride];
+        if (sp.pattern_begin_free < 0 || sp.pattern_end_free < 0 || sp.text_begin_free < 0 || sp.text_end_free < 0) {
+            fprintf(stderr, "[wfagpu] ends-free span values must be >= 0 (got %d,%d,%d,%d for pair %zu)\n",
+                    sp.pattern_begin_free, sp.pattern_end_free, sp.text_begin_free, sp.text_end_free, i);
+            return -3;
+        }
+        ef = ef || sp.pattern_begin_free || sp.pattern_end_free || sp.text_begin_free || sp.text_end_free;
     }
-    const bool ef = sp.pattern_begin_free || sp.pattern_end_free || sp.text_begin_free || sp.text_end_free;
     if (ef && plan->band > 0) {
         fprintf(stderr, "[wfagpu] ends-free alignment is exact only: it cannot be combined with the adaptive band\n");
         return -3;
@@ -1363,17 +1367,23 @@ extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, 
     s.plan = *plan;
     s.ef = ef;
     s.plain = !ef && !p2;
-    s.span = sp;
-    /* the span clamped to every pair, then the widest of the batch: the start row's half width and the reach of the
-     * target range beyond kt (the step table and the rings are shared by the pairs of a batch) */
+    /* the span of every pair clamped to that pair (the kernels read it by pair index, on every pass), then the widest of
+     * the batch: the start row's half width and the reach of the target range beyond kt (the step table and the rings
+     * are shared by the pairs of a batch) */
     s.ef_w = 0;
     s.ef_ext = 0;
-    if (ef) {
+    if (ef && n > 0) {
+        if (s.spans.ensure(n) || s.h_spans.ensure(n)) return -1;
         for (size_t i = 0; i < n; ++i) {
+            const wfagpu_span_t &sp = spans[i * stride];
             const int pl = (int)s.h_pairs.p[i].plen, tl = (int)s.h_pairs.p[i].tlen;
-            s.ef_w = std::max(s.ef_w, std::max(std::min(sp.pattern_begin_free, pl), std::min(sp.text_begin_free, tl)));
-            s.ef_ext = std::max(s.ef_ext, std::max(std::min(sp.pattern_end_free, pl), std::min(sp.text_end_free, tl)));
+            const int4 c = make_int4(std::min(sp.pattern_begin_free, pl), std::min(sp.pattern_end_free, pl),
+                                     std::min(sp.text_begin_free, tl), std::min(sp.text_end_free, tl));
+            s.h_spans.p[i] = c;
+            s.ef_w = std::max(s.ef_w, std::max(c.x, c.z));
+            s.ef_ext = std::max(s.ef_ext, std::max(c.y, c.w));
         }
+        CK(cudaMemcpyAsync(s.spans.p, s.h_spans.p, n * sizeof(int4), cudaMemcpyHostToDevice, s.stream));
     }
     if (n == 0) return 0;
     if (ef && (s.ends.ensure(n) || s.h_ends.ensure(n))) return -1;
@@ -1412,6 +1422,20 @@ extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, 
     if (plan->with_cigar && d->device_text && enqueue_text(d, s, n, s.last_d_end)) return -1;
     CK(cudaEventRecord(s.ev[4], s.stream));                  /* align time = bound + wavefronts + traceback + CIGAR text */
     return 0;
+}
+
+extern "C" int wfagpu_device_align_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident,
+                                        const wfagpu_span_t *span)
+{
+    (void)resident;
+    return align_spans(d, slot, n, plan, span, 0);
+}
+
+extern "C" int wfagpu_device_align_spans(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, int resident,
+                                         const wfagpu_span_t *spans)
+{
+    (void)resident;
+    return align_spans(d, slot, n, plan, spans, 1);
 }
 
 extern "C" int wfagpu_device_download(wfagpu_device_t *d, int slot, size_t n, wfagpu_pair_out_t *out, uint32_t **ops,
@@ -1572,8 +1596,8 @@ extern "C" int wfagpu_device_rescore(wfagpu_device_t *d, int slot, size_t n, con
     return wfagpu_device_rescore_span(d, slot, n, plan, nullptr, scores);
 }
 
-extern "C" int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
-                                          const wfagpu_span_t *span, int32_t *scores)
+static int rescore_spans(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan, const wfagpu_span_t *spans,
+                         size_t stride, int32_t *scores)
 {
     if (!d || !plan || !scores || slot < 0 || slot > 1) return -1;
     if (n != d->slots[slot].n) return -1;
@@ -1586,12 +1610,24 @@ extern "C" int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n
     p2.with_cigar = 0;
     p2.with_ends = 0;
     std::vector<wfagpu_pair_out_t> out(n);
-    int rc = wfagpu_device_align_span(d, slot, n, &p2, 1, span);
+    int rc = align_spans(d, slot, n, &p2, spans, stride);
     if (!rc) rc = wfagpu_device_download(d, slot, n, out.data(), nullptr, nullptr, nullptr);
     d->no_bound = nb; d->no_quad = nq; d->use_hint = uh; d->force_warp = fw; d->independent = false;
     if (rc) return rc;
     for (size_t i = 0; i < n; ++i) scores[i] = (out[i].status & WFAGPU_ST_FINISHED) ? out[i].distance : -1;
     return 0;
+}
+
+extern "C" int wfagpu_device_rescore_span(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
+                                          const wfagpu_span_t *span, int32_t *scores)
+{
+    return rescore_spans(d, slot, n, plan, span, 0, scores);
+}
+
+extern "C" int wfagpu_device_rescore_spans(wfagpu_device_t *d, int slot, size_t n, const wfagpu_plan_t *plan,
+                                           const wfagpu_span_t *spans, int32_t *scores)
+{
+    return rescore_spans(d, slot, n, plan, spans, 1, scores);
 }
 
 extern "C" int wfagpu_device_download_ends(wfagpu_device_t *d, int slot, size_t n, int32_t *ends)

@@ -433,13 +433,16 @@ __device__ __forceinline__ bool prune_window(int n, int kt, int q, int n_cap, in
     return live;
 }
 
-/* The same for an ends-free alignment: the diagonals within q of the target range [tlo, thi]. */
-__device__ __forceinline__ bool prune_window_range(int n, int tlo, int thi, int q, int n_cap, int &lo, int &hi)
+/* The same for an ends-free alignment: the diagonals within q of the target range [tlo, thi] that the pair's own start
+ * row reaches, [dp - n, n - dt].  The step table's n = W + r(d) is sized for the widest start row W of the batch, so
+ * dp = W - pb and dt = W - tb narrow it to [-pb - r(d), tb + r(d)]: a cell further from the pair's start row needs a gap
+ * longer than r(d) and is NULL (DESIGN.md §9).  An all-NULL step NULLs that reach, clamped to the rings. */
+__device__ __forceinline__ bool prune_window_range(int n, int tlo, int thi, int q, int n_cap, int dp, int dt, int &lo, int &hi)
 {
-    lo = max(-n, tlo - q);
-    hi = min(n, thi + q);
+    lo = max(dp - n, tlo - q);
+    hi = min(n - dt, thi + q);
     const bool live = lo <= hi;
-    if (!live) { hi = min(n, n_cap); lo = -hi; }
+    if (!live) { lo = max(dp - n, -n_cap); hi = min(n - dt, n_cap); }
     return live;
 }
 
@@ -599,9 +602,12 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
         const wfagpu_pair_t pr = p.pairs[idx];
         const int plen = (int)pr.plen, tlen = (int)pr.tlen;
         const int kt = tlen - plen;
-        /* ends-free: the span clamped to this pair, and its target diagonals */
-        const int ef_pb = EF ? min(p.ef_pb, plen) : 0, ef_tb = EF ? min(p.ef_tb, tlen) : 0;
-        const int klo_t = EF ? kt - min(p.ef_te, tlen) : kt, khi_t = EF ? kt + min(p.ef_pe, plen) : kt;
+        /* ends-free: this pair's span (clamped by the host), its target diagonals, and how much narrower than the batch's
+         * widest start row W = steps[0].n its own start row [-pb, tb] is on either side (prune_window_range) */
+        const int4 sp = EF ? p.spans[idx] : make_int4(0, 0, 0, 0);
+        const int ef_w = EF ? (int)p.steps[0].n : 0;
+        const int ef_dp = ef_w - sp.x, ef_dt = ef_w - sp.z;
+        const int klo_t = EF ? kt - sp.w : kt, khi_t = EF ? kt + sp.y : kt;
 
         const uint32_t Pa = seq_sa + (uint32_t)(2 * stage) * seq_bytes;
         const uint32_t Ta = Pa + seq_bytes;
@@ -617,8 +623,9 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
 
         /* ---- ring prologue: NULL over [-2G, 2G] on every row (no full re-init) ---- */
         if constexpr (EF) {
-            /* ... widened by the start row's half width (steps[0].n): the windows of the first A scores reach W + G */
-            const int wz = min((int)p.steps[0].n, p.n_cap);
+            /* ... widened by this pair's start row half width max(pb, tb): its windows of the first A scores reach that
+             * + A - 1 (own reach, prune_window_range) */
+            const int wz = min(max(sp.x, sp.z), p.n_cap);
             const int span = 4 * GW + 2 * wz + 1;
             const int total = rows * span;
             for (int i = tid; i < total; i += gsz) {
@@ -675,7 +682,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                     if (d <= Dmax) {
                         const wfagpu_step_t st = p.steps[d];
                         int lo, hi;
-                        const bool live = EF ? prune_window_range((int)st.n, klo_t, khi_t, (Dmax - d) / e, p.n_cap, lo, hi)
+                        const bool live = EF ? prune_window_range((int)st.n, klo_t, khi_t, (Dmax - d) / e, p.n_cap, ef_dp, ef_dt, lo, hi)
                                              : prune_window((int)st.n, kt, (Dmax - d) / e, p.n_cap, lo, hi);
                         const bool stop = live && (lo < -p.n_cap || hi > p.n_cap);     /* wider than the rings */
                         const bool work = live && st.kind != WFAGPU_STEP_NULL;
@@ -704,10 +711,10 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
             };
             bool stop0 = false;                      /* ends-free: finished (or too wide for the rings) at score 0 */
             if constexpr (EF) {
-                /* score 0: the start row [-pb, tb], within the pruning window of score 0 */
+                /* score 0: the start row [-pb, tb] (the own reach of score 0), within the pruning window of score 0 */
                 int lo0, hi0;
-                const bool live0 = prune_window_range((int)p.steps[0].n, klo_t, khi_t, Dmax / e, p.n_cap, lo0, hi0);
-                const int slo = live0 ? max(-ef_pb, lo0) : 1, shi = live0 ? min(ef_tb, hi0) : 0;
+                const bool live0 = prune_window_range(ef_w, klo_t, khi_t, Dmax / e, p.n_cap, ef_dp, ef_dt, lo0, hi0);
+                const int slo = live0 ? lo0 : 1, shi = live0 ? hi0 : 0;
                 int kb = INT_MAX;
                 if (slo >= -p.n_cap && shi <= p.n_cap) {
                     for (int k = slo + tid; k <= shi; k += gsz) {
@@ -816,7 +823,7 @@ __global__ void __launch_bounds__(WARP ? 256 : 1024, WARP ? 4 : 1) wfa_exact_ker
                         } else {
                             if (pr_r == 0) { pr_r = e - 1; --pr_q; } else --pr_r;
                         }
-                        live = EF ? prune_window_range(n, klo_t, khi_t, pr_q, p.n_cap, lo, hi)
+                        live = EF ? prune_window_range(n, klo_t, khi_t, pr_q, p.n_cap, ef_dp, ef_dt, lo, hi)
                                   : prune_window(n, kt, pr_q, p.n_cap, lo, hi);
                         if (live && (lo < -p.n_cap || hi > p.n_cap)) break;     /* wider than the rings of this launch */
                         if (live && kind != WFAGPU_STEP_NULL) n_cells += (unsigned)(hi - lo + 1);

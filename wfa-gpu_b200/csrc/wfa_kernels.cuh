@@ -87,9 +87,11 @@ struct KernelParams {
     uint32_t *ascii_list;         /* pairs the packer flagged (byte-compare launch)          */
     uint32_t *ascii_count;
     unsigned long long *cells;    /* optional work counter (may be null)                     */
-    /* ends-free alignment (wfa_exact_kernel<..., EF = true>): free leading / trailing bases of the pattern and the
-     * text, clamped per pair; the step table's half widths include the start row's max(pb, tb) */
-    int ef_pb, ef_pe, ef_tb, ef_te;
+    /* ends-free alignment (wfa_exact_kernel<..., EF = true>): per pair its free leading / trailing bases of the pattern
+     * and the text {pb, pe, tb, te}, already clamped to that pair; the step table's half widths include the widest start
+     * row of the batch, max(pb, tb) over its pairs */
+    const int4 *spans;
+    int spans_pad[2];             /* keeps the offsets of the fields below, and with them the code of the kernels that read them */
     int2 *ends;                   /* ends-free: per pair {k_begin, k_end}; null in global mode */
     /* gap-affine 2-piece (wfa_exact_kernel<..., P2 = true>): second gap piece and the depth of its I2 / D2 rings (e2 + 1);
      * e2 == 0: one piece.  With P2, A = max(x, o + e, o2 + e2) + 1 */

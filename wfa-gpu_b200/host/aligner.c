@@ -174,6 +174,9 @@ bool wfagpu_add_sequences(wfagpu_aligner_t *aligner, const char *query, const ch
     }
     memcpy(aligner->sequences_buffer + p_off, query, plen);
     memcpy(aligner->sequences_buffer + t_off, target, tlen);
+    /* NUL padding up to the next sequence: a buffer reused after wfagpu_clear_sequences still holds the old bytes */
+    memset(aligner->sequences_buffer + p_off + plen, 0, t_off - (p_off + plen));
+    memset(aligner->sequences_buffer + t_off + tlen, 0, WFA_ALIGN_32_BITS(t_off + tlen + 1) - (t_off + tlen));
     sequence_pair_t *m = &aligner->sequences_metadata[slot];
     memset(m, 0, sizeof(*m));
     m->pattern_offset = p_off;
@@ -266,6 +269,17 @@ bool wfagpu_align_span_coords(wfagpu_aligner_t *aligner, const wfagpu_span_t *sp
     wfagpu_launch_alignments_span_coords(aligner->sequences_buffer, aligner->sequences_buffer_len,
                                          aligner->sequences_metadata, aligner->results, aligner->alignment_options,
                                          aligner->alignment_options.compute_cigar, false, ef ? span : NULL, coords);
+    return wfagpu_last_launch_ok();
+}
+
+bool wfagpu_align_spans(wfagpu_aligner_t *aligner, const wfagpu_span_t *spans, wfagpu_coords_t *coords)
+{
+    if (!aligner) { ERR("Invalid aligner."); return false; }
+    if (!aligner->results || !aligner->sequences_metadata) { ERR("Aligner parameters are not initialized."); return false; }
+    /* the spans are validated by the driver, before anything is aligned */
+    wfagpu_launch_alignments_spans(aligner->sequences_buffer, aligner->sequences_buffer_len, aligner->sequences_metadata,
+                                   aligner->results, aligner->alignment_options, aligner->alignment_options.compute_cigar,
+                                   false, spans, coords);
     return wfagpu_last_launch_ok();
 }
 

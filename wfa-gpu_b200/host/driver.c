@@ -111,8 +111,9 @@ typedef struct {
     bool failed;
     bool verbose;
     bool host_cigar;        /* WFAGPU_HOST_CIGAR=1: print the CIGAR text on the host instead of the GPU */
-    bool ef;                /* ends-free call: `span` is not all zero */
-    wfagpu_span_t span;
+    bool ef;                /* ends-free call: some pair's span is not all zero */
+    const wfagpu_span_t *spans;   /* the caller's: pair i has spans[i * span_stride] (stride 0: one span for the call) */
+    size_t span_stride;
     bool p2;                /* gap-affine 2-piece call: `pen2` replaces opt.penalties */
     wfagpu_affine2p_t pen2;
     wfagpu_coords_t *coords;  /* the caller's, one per pair, or NULL */
@@ -139,6 +140,7 @@ typedef struct {
     wfagpu_pair_out_t *out;
     size_t out_cap;
     int32_t *ends;          /* ends-free, CIGAR text on the host or coordinates: {k_begin, k_end} per pair */
+    bool ef;                /* the chunk was aligned as an ends-free batch: some pair of it has a non-zero span */
 } inflight_t;
 
 static double now_s(void)
@@ -290,6 +292,17 @@ static wfagpu_coords_t coords_of(const sequence_pair_t *m, const int32_t *ends)
     return (wfagpu_coords_t){kb < 0 ? -kb : 0, te - ke, kb > 0 ? kb : 0, te};
 }
 
+static bool span_is_free(const wfagpu_span_t *sp)
+{
+    return sp->pattern_begin_free || sp->pattern_end_free || sp->text_begin_free || sp->text_end_free;
+}
+
+/* the span of pair i of the job (NULL: a global call) */
+static const wfagpu_span_t *span_of(const job_t *j, size_t i)
+{
+    return j->ef ? j->spans + i * j->span_stride : NULL;
+}
+
 static int submit(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
 {
     if (f->pairs_cap < f->n) {
@@ -324,7 +337,11 @@ static int submit(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
         src = stage;
     }
     if (wfagpu_device_upload(d, slot, src, bytes, f->pairs, f->n)) return -1;
-    if (wfagpu_device_align_span(d, slot, f->n, &plan, 0, j->ef ? &j->span : NULL)) return -1;
+    f->ef = false;
+    for (size_t i = 0; j->ef && !f->ef && i < (j->span_stride ? f->n : 1); ++i) f->ef = span_is_free(span_of(j, f->from + i));
+    if (j->span_stride ? wfagpu_device_align_spans(d, slot, f->n, &plan, 0, span_of(j, f->from))
+                       : wfagpu_device_align_span(d, slot, f->n, &plan, 0, span_of(j, f->from)))
+        return -1;
     f->active = true;
     return 0;
 }
@@ -343,7 +360,8 @@ static void check_chunk(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
     wfagpu_plan_t plan;
     fill_plan(j, false, &plan);
     plan.band = 0;                                            /* the exact optimum, also for banded runs */
-    const bool have_ref = ref && wfagpu_device_rescore_span(d, slot, f->n, &plan, j->ef ? &j->span : NULL, ref) == 0;
+    const bool have_ref = ref && (j->span_stride ? wfagpu_device_rescore_spans(d, slot, f->n, &plan, span_of(j, f->from), ref)
+                                                 : wfagpu_device_rescore_span(d, slot, f->n, &plan, span_of(j, f->from), ref)) == 0;
     long bad = 0, sum = 0;
     #pragma omp parallel for schedule(dynamic, 64) num_threads(j->decode_threads) reduction(+:bad,sum) if (f->n > 256)
     for (long i = 0; i < (long)f->n; ++i) {
@@ -354,7 +372,7 @@ static void check_chunk(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f)
                                               m[i].text_len, &j->pen2, res[i].error, res[i].cigar.buffer);
         else if (j->cigar)
             ok = wfagpu_check_result_span(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
-                                          m[i].text_len, j->opt.penalties, j->ef ? &j->span : NULL, res[i].error,
+                                          m[i].text_len, j->opt.penalties, span_of(j, f->from + (size_t)i), res[i].error,
                                           res[i].cigar.buffer);
         /* a banded score may legitimately exceed the optimum; an exact one must equal it */
         if (have_ref && ref[i] >= 0 && (j->opt.band > 0 ? (long)res[i].error < ref[i] : (long)res[i].error != ref[i])) {
@@ -397,7 +415,7 @@ static int collect(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f, wfagpu
         if (wfagpu_device_download_text(d, slot, f->n, &text, &text_bytes, &refs)) return -1;
         wfagpu_device_last_stats(d, slot, &bs);
     }
-    if (j->ef && (j->coords || (j->cigar && j->host_cigar))) {
+    if (f->ef && (j->coords || (j->cigar && j->host_cigar))) {
         /* the coordinates and the host decoder need the diagonals every alignment starts and ends on */
         free(f->ends);
         f->ends = (int32_t *)malloc(2 * f->n * sizeof(int32_t));
@@ -422,11 +440,11 @@ static int collect(job_t *j, wfagpu_device_t *d, int slot, inflight_t *f, wfagpu
         }
         if (!(o->status & WFAGPU_ST_FINISHED)) { bad++; continue; }
         res[i].error = (unsigned int)o->distance;
-        if (j->coords) j->coords[f->from + (size_t)i] = coords_of(&m[i], j->ef ? f->ends + 2 * i : NULL);
+        if (j->coords) j->coords[f->from + (size_t)i] = coords_of(&m[i], f->ef ? f->ends + 2 * i : NULL);
         if (j->cigar && refs) {
             /* text was printed on the GPU: append it to the caller's buffer */
             if (!wfagpu_cigar_append(&res[i].cigar, text + refs[i].off, refs[i].len)) bad++;
-        } else if (j->cigar && j->ef) {
+        } else if (j->cigar && f->ef) {
             if (!wfagpu_ops_to_cigar_span(j->buf + m[i].pattern_offset, m[i].pattern_len, j->buf + m[i].text_offset,
                                           m[i].text_len, f->ends[2 * i], ops + o->ops_off, o->n_ops, &res[i].cigar))
                 bad++;
@@ -523,7 +541,7 @@ void wfagpu_plan_chunks(size_t n, size_t batch_size, int n_devices, size_t ascii
 
 static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_alignment_result_t *res,
                     wfa_alignment_options_t opt, bool cigar, bool check, const wfagpu_span_t *ends_free,
-                    const wfagpu_affine2p_t *affine2p, wfagpu_coords_t *coords)
+                    size_t span_stride, const wfagpu_affine2p_t *affine2p, wfagpu_coords_t *coords)
 {
     const double t0 = now_s();
     memset(&t_last_stats, 0, sizeof(t_last_stats));
@@ -548,11 +566,16 @@ static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_align
         fprintf(stderr, "[!] ERROR: penalties must satisfy x >= 1, e >= 1, o >= 0.\n");
         return;
     }
-    const wfagpu_span_t *sp = ends_free;
-    const bool ef = sp && (sp->pattern_begin_free || sp->pattern_end_free || sp->text_begin_free || sp->text_end_free);
-    if (sp && (sp->pattern_begin_free < 0 || sp->pattern_end_free < 0 || sp->text_begin_free < 0 || sp->text_end_free < 0)) {
-        fprintf(stderr, "[!] ERROR: ends-free span values must be >= 0.\n");
-        return;
+    /* every span is checked before anything is aligned */
+    bool ef = false;
+    for (size_t i = 0; ends_free && i < (span_stride ? opt.num_alignments : 1); ++i) {
+        const wfagpu_span_t *sp = ends_free + i * span_stride;
+        if (sp->pattern_begin_free < 0 || sp->pattern_end_free < 0 || sp->text_begin_free < 0 || sp->text_end_free < 0) {
+            fprintf(stderr, "[!] ERROR: ends-free span values must be >= 0 (pair %zu: %d,%d,%d,%d).\n", i,
+                    sp->pattern_begin_free, sp->pattern_end_free, sp->text_begin_free, sp->text_end_free);
+            return;
+        }
+        ef = ef || span_is_free(sp);
     }
     if (ef && opt.band > 0) {
         fprintf(stderr, "[!] ERROR: ends-free alignment cannot be combined with the adaptive band (-B).\n");
@@ -571,7 +594,8 @@ static void run_job(char *buf, size_t buf_size, sequence_pair_t *meta, wfa_align
     job.buf = buf; job.buf_size = buf_size; job.meta = meta; job.res = res; job.opt = opt; job.cigar = cigar;
     job.check = check;
     job.ef = ef;
-    if (ef) job.span = *sp;
+    job.spans = ends_free;
+    job.span_stride = span_stride;
     job.p2 = affine2p != NULL;
     if (affine2p) job.pen2 = *affine2p;
     job.coords = coords;
@@ -669,7 +693,7 @@ void launch_alignments(char *sequences_buffer, const size_t sequences_buffer_siz
                        wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, true,
-            check_correctness, NULL, NULL, NULL);
+            check_correctness, NULL, 0, NULL, NULL);
 }
 
 void launch_alignments_distance(char *sequences_buffer, const size_t sequences_buffer_size,
@@ -678,7 +702,7 @@ void launch_alignments_distance(char *sequences_buffer, const size_t sequences_b
                                 wfa_alignment_options_t options, bool check_correctness)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, false,
-            check_correctness, NULL, NULL, NULL);
+            check_correctness, NULL, 0, NULL, NULL);
 }
 
 void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buffer_size,
@@ -687,7 +711,7 @@ void wfagpu_launch_alignments_span(char *sequences_buffer, size_t sequences_buff
                                    const wfagpu_span_t *span)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
-            check_correctness, span, NULL, NULL);
+            check_correctness, span, 0, NULL, NULL);
 }
 
 void wfagpu_launch_alignments_span_coords(char *sequences_buffer, size_t sequences_buffer_size,
@@ -696,7 +720,16 @@ void wfagpu_launch_alignments_span_coords(char *sequences_buffer, size_t sequenc
                                           const wfagpu_span_t *span, wfagpu_coords_t *coords)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
-            check_correctness, span, NULL, coords);
+            check_correctness, span, 0, NULL, coords);
+}
+
+void wfagpu_launch_alignments_spans(char *sequences_buffer, size_t sequences_buffer_size,
+                                    sequence_pair_t *sequences_metadata, wfa_alignment_result_t *alignment_results,
+                                    wfa_alignment_options_t options, bool cigar, bool check_correctness,
+                                    const wfagpu_span_t *spans, wfagpu_coords_t *coords)
+{
+    run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
+            check_correctness, spans, 1, NULL, coords);
 }
 
 void wfagpu_launch_alignments_affine2p(char *sequences_buffer, size_t sequences_buffer_size,
@@ -705,5 +738,5 @@ void wfagpu_launch_alignments_affine2p(char *sequences_buffer, size_t sequences_
                                        const wfagpu_affine2p_t *pen)
 {
     run_job(sequences_buffer, sequences_buffer_size, sequences_metadata, alignment_results, options, cigar,
-            check_correctness, NULL, pen, NULL);
+            check_correctness, NULL, 0, pen, NULL);
 }

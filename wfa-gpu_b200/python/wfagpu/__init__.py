@@ -8,6 +8,7 @@ runs on the GPU.  There is no CPU path: without the CUDA library or a GPU the
 calls fail loudly.
 """
 import ctypes as C
+import operator
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -118,7 +119,8 @@ EXPORTS = [
     "wfagpu_device_download_ends", "wfagpu_device_rescore_span", "wfagpu_ops_to_cigar_span",
     "wfagpu_check_result_span", "wfagpu_build_step_table_span", "wfagpu_align_affine2p",
     "wfagpu_launch_alignments_affine2p", "wfagpu_check_result_affine2p", "wfagpu_build_step_table_affine2p",
-    "wfagpu_align_span_coords", "wfagpu_launch_alignments_span_coords",
+    "wfagpu_align_span_coords", "wfagpu_launch_alignments_span_coords", "wfagpu_align_spans",
+    "wfagpu_launch_alignments_spans", "wfagpu_device_align_spans", "wfagpu_device_rescore_spans",
 ]
 
 _lib = None
@@ -236,6 +238,13 @@ def load():
     L.wfagpu_launch_alignments_span_coords.argtypes = [C.c_void_p, C.c_size_t, P(SequencePair), P(AlignmentResult),
                                                        AlignmentOptions, C.c_bool, C.c_bool, P(Span), P(Coords)]
     L.wfagpu_launch_alignments_span_coords.restype = None
+    L.wfagpu_align_spans.argtypes = [P(AlignerStruct), P(Span), P(Coords)]
+    L.wfagpu_align_spans.restype = C.c_bool
+    L.wfagpu_launch_alignments_spans.argtypes = [C.c_void_p, C.c_size_t, P(SequencePair), P(AlignmentResult),
+                                                 AlignmentOptions, C.c_bool, C.c_bool, P(Span), P(Coords)]
+    L.wfagpu_launch_alignments_spans.restype = None
+    L.wfagpu_device_align_spans.argtypes = [C.c_void_p, C.c_int, C.c_size_t, P(Plan), C.c_int, P(Span)]
+    L.wfagpu_device_rescore_spans.argtypes = [C.c_void_p, C.c_int, C.c_size_t, P(Plan), P(Span), P(C.c_int32)]
     _lib = L
     return L
 
@@ -248,6 +257,32 @@ def span_of(ends_free):
     if len(vals) != 4:
         raise ValueError("ends_free takes four values: pattern_begin_free, pattern_end_free, text_begin_free, text_end_free")
     return Span(*vals)
+
+
+def spans_of(ends_free, num_pairs):
+    """Per-pair ends-free spans: a sequence of `num_pairs` 4-tuples, or an (num_pairs, 4) array -> a Span array.
+    ValueError for another count or shape."""
+    try:
+        rows = [tuple(operator.index(v) for v in r) for r in ends_free]
+    except TypeError:
+        raise ValueError("ends_free: give one span of four integers per pair, or a single 4-tuple") from None
+    if len(rows) != num_pairs:
+        raise ValueError(f"ends_free has {len(rows)} spans for {num_pairs} pairs: give one per pair, or a single 4-tuple")
+    if any(len(r) != 4 for r in rows):
+        raise ValueError("every per-pair span takes four values: pattern_begin_free, pattern_end_free, "
+                         "text_begin_free, text_end_free")
+    return (Span * num_pairs)(*(Span(*r) for r in rows))
+
+
+def _per_pair(ends_free):
+    """True when ends_free holds one span per pair (its entries are sequences), False for a single 4-tuple."""
+    if ends_free is None or len(ends_free) == 0:
+        return ends_free is not None
+    try:
+        iter(ends_free[0])
+    except TypeError:
+        return False
+    return True
 
 
 def affine2p_of(pen):
@@ -291,12 +326,15 @@ class Aligner:
 
     def align(self, ends_free=None, affine2p=None, coords=False):
         """ends_free: None (global) or (pattern_begin_free, pattern_end_free, text_begin_free, text_end_free),
-        WFA2-lib's order: that many leading / trailing bases of either sequence are free (wfagpu_align_span).
+        WFA2-lib's order: that many leading / trailing bases of either sequence are free (wfagpu_align_span).  Or one
+        such span per pair: a sequence of num_pairs 4-tuples or an (num_pairs, 4) array (wfagpu_align_spans); a pair
+        whose span is all zero gets its global alignment.
         affine2p: None or (x, o1, e1, o2, e2), gap-affine 2-piece penalties for this call in place of the aligner's
         (wfagpu_align_affine2p); global alignment only.
         coords: also record where every alignment lies, with or without a CIGAR (wfagpu_align_span_coords); read
         them with coords().  Not with affine2p."""
-        sp = span_of(ends_free)
+        per_pair = _per_pair(ends_free)
+        sp = spans_of(ends_free, self.num_pairs) if per_pair else span_of(ends_free)
         pen2 = affine2p_of(affine2p)
         self._coords = None
         if pen2 is not None:
@@ -306,6 +344,12 @@ class Aligner:
                 raise ValueError("affine2p cannot be combined with coords")
             if not self.L.wfagpu_align_affine2p(C.byref(self.s), C.byref(pen2)):
                 raise RuntimeError("wfagpu_align_affine2p failed (see stderr); there is no CPU fallback")
+            return True
+        if per_pair:
+            cs = (Coords * self.num_pairs)() if coords else None
+            if not self.L.wfagpu_align_spans(C.byref(self.s), sp, cs):
+                raise RuntimeError("wfagpu_align_spans failed (see stderr); there is no CPU fallback")
+            self._coords = cs
             return True
         if coords:
             cs = (Coords * self.num_pairs)()
